@@ -2,7 +2,7 @@
 """bench.py — camera x point visibility tests/s on a synthetic city grid (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3|cfg4|cfg5]
-                    [--cull-mode grid|exhaustive] [--impl reference]
+                    [--cull-mode grid|exhaustive] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (c2b_visibility_graph: point grid -> plan -> fused cull + occlusion ->
 sort + write) over the whole workload; cameras are sharded across GPUs (contiguous ranges, the mesh, BVH and
@@ -26,6 +26,8 @@ ONE JSON line on rank 0.
   --impl reference : the reference's algorithm on the box's host cores (the oracle's OpenMP + CPU-BVH arm,
           built -O3 -march=native on the box; the Rust/Embree reference cannot be built in this image), on a
           bounded camera sample of the same workload.
+  --dump-outputs DIR : after the run, the CSR the e2e call returned in its last timed step as float64 .npy files
+          (see dump_outputs), so that two builds can be compared output for output on the same inputs.
 """
 from __future__ import annotations
 
@@ -41,6 +43,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the checkout may be read-only: the bench writes nothing into it
 
 WORKLOADS = {
     # name: (blocks, cameras_per_block, points_per_block)  — BASELINE.md section 4
@@ -236,6 +239,22 @@ def expected_hash(workload):
         return None
 
 
+DUMP_MAX_OBS = 2_000_000  # 48 MB of (point index, u, v) in float64; with the offsets under 64 MB at every workload
+
+
+def dump_outputs(out_dir, offsets, idx, uv, seed=0):
+    """Writes a CSR (offsets, idx, uv) as float64 arrays (exact: indices and offsets are below 2**53):
+    offsets.npy, all C + 1 entries; point_idx.npy (O,) and uv.npy (O, 2), every observation, or, when there are
+    more than DUMP_MAX_OBS (cfg4: 53 M), the observations at a seeded sample of positions, ascending, which is
+    the same sample for two results with the same number of observations."""
+    O = len(idx)
+    sel = slice(None) if O <= DUMP_MAX_OBS else np.unique(np.random.default_rng(seed).integers(0, O, DUMP_MAX_OBS))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "offsets.npy"), np.asarray(offsets, np.float64))
+    np.save(os.path.join(out_dir, "point_idx.npy"), np.asarray(idx)[sel].astype(np.float64))
+    np.save(os.path.join(out_dir, "uv.npy"), np.asarray(uv, np.float64).reshape(-1, 2)[sel])
+
+
 def parity_against(sample_idx, vis, offsets, idx, uv):
     """rows `sample_idx` of the CSR (offsets, idx, uv) against the oracle graph `vis` of those cameras"""
     off = np.asarray(offsets, np.int64)
@@ -327,7 +346,13 @@ def main():
     ap.add_argument("--no-noise", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the cfg3 / cfg5 lines of the default run")
     ap.add_argument("--no-extras", action="store_true", help="skip e2e_pageable / e2e_cold")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the CSR of the last timed e2e step to DIR/{offsets,point_idx,uv}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU result; --impl reference computes a camera sample only")
     default_run = args.workload is None
     if args.workload is None:
         # the metric's target is quoted on the 64x64-block city (cfg4); it fits one GPU
@@ -793,6 +818,8 @@ def main():
             p2.scene.close()
             del p2
         line["secondary"] = sec
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *csr)
     real_stdout.write(json.dumps(line) + "\n")
     real_stdout.flush()
     if world > 1:

@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -49,30 +50,11 @@ class _Vis(C.Structure):
 _lib = None
 
 
-def _cpu_id() -> str:
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("flags"):
-                import hashlib
-                return hashlib.sha1(line.encode()).hexdigest()
-    except OSError:
-        pass
-    return "unknown"
-
-
-def build_native() -> str:
-    """-O3 -march=native build of the same sources for the TIMED CPU arm, made on the machine that runs it
-    (rebuilt when it was made on a CPU with other ISA flags: the repo snapshot travels between machines)."""
-    so, tag = os.path.join(_HERE, "liboracle_native.so"), os.path.join(_HERE, "liboracle_native.cpu")
-    srcs = [os.path.join(_HERE, f) for f in ("cpu_ref.c", "c2b_oracle.c", "c2b_oracle.h")]
-    cpu = _cpu_id()
-    fresh = (os.path.exists(so) and os.path.exists(tag) and open(tag).read() == cpu
-             and all(os.path.getmtime(s) <= os.path.getmtime(so) for s in srcs))
-    if not fresh:
-        if os.path.exists(so):
-            os.unlink(so)
-        subprocess.check_call(["make", "-C", _HERE, "-s", "native"])
-        open(tag, "w").write(cpu)
+def build_native(out_dir: str) -> str:
+    """-O3 -march=native build of the same sources for the TIMED CPU arm, made by the process that runs it (a
+    build made on another CPU may not run here) into `out_dir`, outside the checkout, which may be read-only."""
+    so = os.path.join(out_dir, "liboracle_native.so")
+    subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"NATIVE_OUT={so}"])
     return so
 
 
@@ -81,7 +63,8 @@ def lib():
     global _lib
     if _lib is None:
         if os.environ.get("C2B_ORACLE_NATIVE") == "1":
-            _lib = C.CDLL(build_native())
+            with tempfile.TemporaryDirectory(prefix="c2b_oracle_native_") as d:
+                _lib = C.CDLL(build_native(d))   # stays mapped after the directory is removed
         else:
             build()
             _lib = C.CDLL(_SO)

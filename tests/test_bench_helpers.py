@@ -4,6 +4,7 @@ exactly the cameras whose rows differ from the oracle's."""
 import numpy as np
 
 import bench
+from conftest import bits_equal
 
 
 def _graph(orc):
@@ -57,6 +58,35 @@ def test_parity_against_counts_differing_cameras(orc):
     assert bench.parity_against(sample, ref, v.offsets, v.point_idx, uv)["mismatches"] == 1
     # what the bench hands over: the flat (2 * O,) view of the library's uv array
     assert bench.parity_against(sample, ref, v.offsets, v.point_idx, v.uv.reshape(-1))["mismatches"] == 0
+
+
+def test_dump_outputs_whole_and_sampled(orc, tmp_path, monkeypatch):
+    _, _, _, _, v = _graph(orc)
+    bench.dump_outputs(tmp_path / "all", v.offsets, v.point_idx, v.uv.reshape(-1))
+    load = lambda d, n: np.load(tmp_path / d / f"{n}.npy")  # noqa: E731
+    assert all(load("all", n).dtype == np.float64 for n in ("offsets", "point_idx", "uv"))
+    assert np.array_equal(load("all", "offsets"), v.offsets) and np.array_equal(load("all", "point_idx"), v.point_idx)
+    assert bits_equal(load("all", "uv"), v.uv) and load("all", "uv").shape == v.uv.shape
+    monkeypatch.setattr(bench, "DUMP_MAX_OBS", 1000)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(tmp_path / d, v.offsets, v.point_idx, v.uv)
+    assert np.array_equal(load("s1", "point_idx"), load("s2", "point_idx"))   # the same seeded sample
+    n = len(load("s1", "point_idx"))
+    assert 900 < n <= 1000 and load("s1", "uv").shape == (n, 2)
+    assert np.isin(load("s1", "point_idx"), v.point_idx.astype(np.float64)).all()
+
+
+def test_native_oracle_builds_outside_the_checkout():
+    """the bench's CPU arm builds the oracle -march=native where it runs; the checkout may be read-only"""
+    import os
+    import subprocess
+    import sys
+    from conftest import ROOT
+    here = os.path.join(ROOT, "oracle")
+    before = sorted(os.listdir(here))
+    subprocess.check_call([sys.executable, "-c", "from oracle import oracle as o; assert o.lib().orc_deg_to_rad(180.0) > 3"],
+                          cwd=ROOT, env={**os.environ, "C2B_ORACLE_NATIVE": "1", "PYTHONDONTWRITEBYTECODE": "1"})
+    assert sorted(os.listdir(here)) == before
 
 
 def test_workload_generators_agree():

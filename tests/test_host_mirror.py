@@ -98,9 +98,22 @@ def _dump(models):
     return out
 
 
+def _write_golden_mesh_obj(path, name):
+    """the reference's own meshes (test_scene.obj, tests/box.obj) as tests/golden stores them, after tobj's
+    triangulation, written back as OBJ text: one object, one `f` record per stored index triple (the triples
+    the `l` records left are degenerate ones); returns the stored (xyz, tri)"""
+    import os
+    from conftest import GOLDEN
+    g = np.load(os.path.join(GOLDEN, name))
+    lines = ["o Mesh"] + ["v %r %r %r" % tuple(float(x) for x in v) for v in g["xyz"]]
+    lines += ["f %d %d %d" % tuple(int(k) + 1 for k in t) for t in g["tri"]]
+    open(path, "w").write("\n".join(lines) + "\n")
+    return g["xyz"], g["tri"]
+
+
 def test_obj_loader_python_equals_cpp(c2b, tmp_path):
-    """the two host mirrors read OBJ files identically (tobj 0.1.12's rules): the hand-written scene everywhere,
-    the reference's own fixtures where /root/reference exists (build container only)"""
+    """the two host mirrors read OBJ files identically (tobj 0.1.12's rules): the hand-written scene and the
+    reference's own meshes from tests/golden, which both must read back to the stored triangles"""
     import os
     import subprocess
     from conftest import ROOT
@@ -112,7 +125,13 @@ def test_obj_loader_python_equals_cpp(c2b, tmp_path):
                            "-lcity2ba_cuda", f"-Wl,-rpath,{so_dir}"])
     mine = str(tmp_path / "scene.obj")
     _write_obj(mine)
-    files = [mine] + [f for f in ("/root/reference/tests/box.obj", "/root/reference/test_scene.obj") if os.path.exists(f)]
+    files = [mine]
+    for name in ("box_obj.npz", "cfg1_test_scene.npz"):
+        f = str(tmp_path / name.replace(".npz", ".obj"))
+        xyz, tri = _write_golden_mesh_obj(f, name)
+        lx, lt = generate.concat_models(generate.load_obj(f))
+        assert np.array_equal(lx[lt], xyz[tri]), name     # the same triangles, corner for corner
+        files.append(f)
     for f in files:
         cpp = []
         for line in subprocess.check_output([exe, "obj", f], text=True).splitlines():
