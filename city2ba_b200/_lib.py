@@ -80,6 +80,18 @@ class MultiStats(C.Structure):
     ]
 
 
+class CullStats(C.Structure):
+    """c2b_cull_stats: sizes after LCC + remove_singletons to a fixed point, and device times"""
+    _fields_ = [
+        ("n_cameras", C.c_uint64), ("n_points", C.c_uint64), ("n_obs", C.c_uint64),
+        ("iterations", C.c_uint32), ("reserved", C.c_uint32),
+        ("ms_h2d", C.c_float), ("ms_compute", C.c_float), ("ms_d2h", C.c_float),
+    ]
+
+    def to_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
 CULL_GRID, CULL_EXHAUSTIVE = 0, 1
 OCC_MESH, OCC_NONE, OCC_ANALYTIC = 0, 1, 2
 PRED_WATERTIGHT, PRED_MT = 0, 1
@@ -96,7 +108,7 @@ EXPORTS = [
     "c2b_visibility_graph_resident", "c2b_download_obs", "c2b_reprojection_error_resident",
     "c2b_add_drift", "c2b_add_drift_normalized", "c2b_add_noise", "c2b_add_sin_noise", "c2b_noise_timing",
     "c2b_add_drift_resident", "c2b_add_noise_resident", "c2b_add_sin_noise_resident", "c2b_download_problem",
-    "c2b_mean_std", "c2b_generate_world_points_uniform",
+    "c2b_mean_std", "c2b_cull_problem", "c2b_cull_problem_resident", "c2b_generate_world_points_uniform",
     "c2b_grid_num_cameras", "c2b_grid_num_points", "c2b_grid_cameras", "c2b_grid_points",
     "c2b_line_cameras", "c2b_line_points", "c2b_city_mesh", "c2b_camera_center",
     "c2b_camera_project_world", "c2b_camera_project", "c2b_camera_from_position_direction",
@@ -174,6 +186,8 @@ def lib():
     L.c2b_add_sin_noise_resident.argtypes = [vp, pd, pd, dbl, dbl]
     L.c2b_download_problem.argtypes = [vp, pd, pd]
     L.c2b_mean_std.argtypes = [vp, pd, u64, pd, u64, pd, pd]
+    L.c2b_cull_problem.argtypes = [vp, pd, u64, pd, u64, C.POINTER(u64), pu32, pd, C.POINTER(CullStats)]
+    L.c2b_cull_problem_resident.argtypes = [vp, C.POINTER(CullStats)]
     L.c2b_probe_fp64.argtypes = [vp, pd]
     L.c2b_generate_world_points_uniform.argtypes = [vp, pf, u64, pu32, u64, pd, u64, u64, dbl, u64, pd,
                                                     C.POINTER(u64)]

@@ -408,6 +408,32 @@ class BAProblem:
             return filtered.subset(ci, pi)
         return self.subset(ci, pi)
 
+    def cull_gpu(self, ctx=None, stats=None):
+        """cull() on the GPU (c2b_cull_problem): the same problem, bit for bit.  Works on copies; `stats`, a dict
+        if given, receives the call's c2b_cull_stats (iterations, device times)."""
+        from ._lib import CullStats
+        ctx = ctx or context()
+        g = self.vis_graph
+        cams = np.array(self.cameras, np.float64, order="C").reshape(-1, CAM_STRIDE)
+        pts = np.array(self.points, np.float64, order="C").reshape(-1, 3)
+        off = np.array(g.offsets, np.uint64, order="C")
+        if len(off) != len(cams) + 1:
+            raise ValueError("cameras and CSR offsets disagree")
+        idx = g.point_idx
+        if len(idx) and int(idx.max()) > 0xffffffff:
+            raise ValueError("point index does not fit 32 bits")
+        idx = np.array(idx, np.uint32, order="C")
+        uv = np.array(g.uv, np.float64, order="C").reshape(-1, 2)
+        st = CullStats()
+        check(lib().c2b_cull_problem(ctx.handle, _p(cams), len(cams), _p(pts), len(pts),
+                                     off.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                     idx.ctypes.data_as(C.POINTER(C.c_uint32)), _p(uv), C.byref(st)))
+        if stats is not None:
+            stats.update(st.to_dict())
+        nc, npt, no = int(st.n_cameras), int(st.n_points), int(st.n_obs)
+        return BAProblem(cams[:nc].copy(), pts[:npt].copy(),
+                         VisGraph(off[:nc + 1].copy(), idx[:no].astype(np.uint64), uv[:no].copy()))
+
     def cull(self):
         """src/baproblem.rs:538-549: iterate LCC then remove_singletons to a fixed point."""
         nc, npt = self.num_cameras(), self.num_points()

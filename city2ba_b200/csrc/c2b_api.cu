@@ -22,6 +22,7 @@
 #include "c2b_compact.cuh"
 #include "c2b_cull.cuh"
 #include "c2b_fused.cuh"
+#include "c2b_graph_cull.cuh"
 #include "c2b_internal.h"
 #include "c2b_math.cuh"
 #include "c2b_noise.cuh"
@@ -285,6 +286,9 @@ struct CtxExtra {
   uint64_t points_version = 0;
   double pts_bounds[6] = {0, 0, 0, 0, 0, 0};
   bool have_points = false, have_cameras = false, have_result = false;
+  // the last pass was the host-buffer c2b_visibility_graph (only its last batch stays).  have_result is already false
+  // then; this only picks the message with which c2b_cull_problem_resident refuses
+  bool host_call_last = false;
   uint64_t res_candidates = 0;
 };
 
@@ -431,8 +435,11 @@ void c2b_shutdown(c2b_ctx *ctx) {
                     &ctx->misc, &ctx->tri_list, &ctx->tri_count, &ctx->pts_aos, &ctx->ev_off,
                     &ctx->vis_count, &ctx->seg_off, &ctx->scratch_idx, &ctx->plan_rows, &ctx->plan_row_count,
                     &ctx->nz_cams, &ctx->nz_centers, &ctx->nz_pts, &ctx->nz_uv, &ctx->nz_scratch,
-                    &ctx->epi_status, &ctx->epi_prefix, &ctx->cams_all};
+                    &ctx->epi_status, &ctx->epi_prefix, &ctx->cams_all, &ctx->pr_parent, &ctx->pr_size,
+                    &ctx->pr_cam_cnt, &ctx->pr_pt_cnt, &ctx->pr_words, &ctx->pr_prefix, &ctx->pr_small};
   for (auto *b : bufs) b->release();
+  for (int i = 0; i < 2; ++i)
+    for (DevBuf *b : {&ctx->pr_cams[i], &ctx->pr_pts[i], &ctx->pr_off[i], &ctx->pr_idx[i], &ctx->pr_uv[i]}) b->release();
   PinBuf *pins[] = {&ctx->pin_in, &ctx->h_offsets, &ctx->h_idx, &ctx->h_uv, &ctx->h_small};
   for (auto *p : pins) p->release();
   for (int i = 0; i < EV_COUNT; ++i)
@@ -676,6 +683,7 @@ int c2b_points_commit(c2b_ctx *ctx, uint64_t P) {
   x->grid.valid = false;
   x->have_points = true;
   x->have_result = false;
+  x->host_call_last = false;
   if (P == 0) return C2B_OK;
   C2B_TRY(ctx->pts.ensure(P * 24));
   double *px = ctx->pts.as<double>(), *py = px + P, *pz = py + P;
@@ -724,6 +732,7 @@ int c2b_upload_cameras(c2b_ctx *ctx, const double *cams, uint64_t C) {
   ctx->C = C;
   x->have_cameras = true;
   x->have_result = false;
+  x->host_call_last = false;
   if (C == 0) return C2B_OK;
   C2B_TRY(ctx->cams.ensure(C * 120));
   C2B_TRY(ctx->cam_center.ensure(C * 24));
@@ -1259,6 +1268,7 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
 int c2b_visibility_graph_resident(c2b_ctx *ctx, const c2b_scene *scene, double max_dist,
                                   const c2b_vis_options *opt_in, c2b_obs *stats) {
   const int rc = visibility_resident_impl(ctx, scene, max_dist, opt_in, stats);
+  if (ctx) extra_of(ctx)->host_call_last = false;
   return rc == ERR_TOO_LARGE ? C2B_ERR_INVALID : rc;
 }
 
@@ -1734,6 +1744,7 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
   cudaEventDestroy(d1);
   ctx->out_sel = 0;
   x->have_result = false;  // the resident state now holds the last batch only
+  x->host_call_last = true;
   if (rc != C2B_OK) {
     cudaStreamSynchronize(cs);
     return rc;
@@ -2381,6 +2392,169 @@ int c2b_mean_std(c2b_ctx *ctx, const double *cams, uint64_t C, const double *pts
   NoiseView v;
   C2B_TRY(noise_upload(ctx, v, cams, C, pts, P));
   return device_stats(ctx, v, mean, sd, false);
+}
+
+// ---- BAProblem::cull: LCC + remove_singletons to a fixed point (c2b_graph_cull.cuh) -------------------------
+namespace {
+struct CullEvents {  // timing events of one cull call
+  cudaEvent_t e[4] = {};
+  int create() {
+    for (auto &x : e) C2B_CUDA(cudaEventCreate(&x));
+    return C2B_OK;
+  }
+  ~CullEvents() {
+    for (auto x : e)
+      if (x) cudaEventDestroy(x);
+  }
+};
+}  // namespace
+
+static int cull_limits(uint64_t C, uint64_t P, uint64_t O, const char *who) {
+  if (C + P >= 0xffffffffull)
+    return set_error(C2B_ERR_INVALID, "%s: %llu cameras + %llu points exceed the 32-bit entity ids (C + P < 2^32 - 1)",
+                     who, (unsigned long long)C, (unsigned long long)P);
+  if (O >= 0xffffffffull)
+    return set_error(C2B_ERR_INVALID, "%s: %llu observations exceed the 32-bit compaction (O < 2^32 - 1)", who,
+                     (unsigned long long)O);
+  return C2B_OK;
+}
+
+int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64_t P, uint64_t *offsets,
+                     uint32_t *point_idx, double *uv, c2b_cull_stats *out) {
+  if (!ctx || !offsets || (C && !cams) || (P && !pts)) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: null argument");
+  const uint64_t O = offsets[C];
+  if (O && (!point_idx || !uv)) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: null observation array");
+  C2B_TRY(cull_limits(C, P, O, "c2b_cull_problem"));
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  PruneSet sets[2];
+  for (int i = 0; i < 2; ++i) sets[i] = PruneSet{&ctx->pr_cams[i], &ctx->pr_pts[i], &ctx->pr_off[i], &ctx->pr_idx[i], &ctx->pr_uv[i]};
+  C2B_TRY(ctx->pr_cams[0].ensure(std::max<uint64_t>(C, 1) * 120));
+  C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
+  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
+  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
+  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
+  C2B_TRY(ctx->pr_small.ensure(64));
+  C2B_TRY(ctx->h_small.ensure(256));
+  CullEvents events;
+  C2B_TRY(events.create());
+  cudaEvent_t *ev = events.e;
+  int rc = [&]() -> int {
+    C2B_CUDA(cudaEventRecord(ev[0], st));
+    if (C) C2B_TRY(copy_in(ctx, ctx->pr_cams[0].p, cams, C * 120, cudaMemcpyHostToDevice));
+    if (P) C2B_TRY(copy_in(ctx, ctx->pr_pts[0].p, pts, P * 24, cudaMemcpyHostToDevice));
+    C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
+    if (O) {
+      C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
+      C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
+    }
+    // from_visibility's asserts, on the device: offsets start at 0 and do not decrease, indices < P
+    uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
+    C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+    const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
+    k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
+        ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, P, flag);
+    C2B_KERNEL_CHECK();
+    C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaEventRecord(ev[1], st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    const uint32_t bad = *ctx->h_small.as<uint32_t>();
+    if (bad & 1u) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: offsets[0] != 0 or the CSR offsets decrease");
+    if (bad & 2u) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: an observation references a point >= %llu",
+                                   (unsigned long long)P);
+    int cur = 0;
+    uint64_t c = C, p = P, o = O;
+    uint32_t it = 0;
+    C2B_TRY(prune_fixed_point(ctx, sets, &cur, &c, &p, &o, &it));
+    C2B_CUDA(cudaEventRecord(ev[2], st));
+    const PruneSet &r = sets[cur];
+    if (c) C2B_CUDA(cudaMemcpyAsync(cams, r.cams->p, c * 120, cudaMemcpyDeviceToHost, st));
+    if (p) C2B_CUDA(cudaMemcpyAsync(pts, r.pts->p, p * 24, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaMemcpyAsync(offsets, r.off->p, (c + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (o) {
+      C2B_CUDA(cudaMemcpyAsync(point_idx, r.idx->p, o * 4, cudaMemcpyDeviceToHost, st));
+      C2B_CUDA(cudaMemcpyAsync(uv, r.uv->p, o * 16, cudaMemcpyDeviceToHost, st));
+    }
+    C2B_CUDA(cudaEventRecord(ev[3], st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    if (out) {
+      memset(out, 0, sizeof *out);
+      out->n_cameras = c;
+      out->n_points = p;
+      out->n_obs = o;
+      out->iterations = it;
+      cudaEventElapsedTime(&out->ms_h2d, ev[0], ev[1]);
+      cudaEventElapsedTime(&out->ms_compute, ev[1], ev[2]);
+      cudaEventElapsedTime(&out->ms_d2h, ev[2], ev[3]);
+    }
+    return C2B_OK;
+  }();
+  if (rc != C2B_OK) cudaStreamSynchronize(st);
+  return rc;
+}
+
+int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
+  if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: null ctx");
+  CtxExtra *x = extra_of(ctx);
+  if (x->host_call_last)
+    return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: the resident CSR is the last camera batch of the "
+                                      "host-buffer c2b_visibility_graph, not the graph of an uploaded problem; run "
+                                      "c2b_visibility_graph_resident first");
+  if (!x->have_result || !x->have_points || !x->have_cameras)
+    return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: no resident result (upload cameras and points, "
+                                      "then c2b_visibility_graph_resident)");
+  uint64_t C = ctx->out_C, P = ctx->P, O = ctx->out_O;
+  C2B_TRY(cull_limits(C, P, O, "c2b_cull_problem_resident"));
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const int sel = ctx->out_sel;
+  // set 0: the resident problem; set 1: the other half of the double-buffered CSR and spare camera / point arrays
+  PruneSet sets[2] = {{&ctx->cams, &ctx->pts_aos, &ctx->out_offsets[sel], &ctx->out_idx[sel], &ctx->out_uv[sel]},
+                      {&ctx->pr_cams[1], &ctx->pr_pts[1], &ctx->out_offsets[sel ^ 1], &ctx->out_idx[sel ^ 1],
+                       &ctx->out_uv[sel ^ 1]}};
+  CullEvents events;
+  C2B_TRY(events.create());
+  cudaEvent_t *ev = events.e;
+  int cur = 0;
+  uint32_t it = 0;
+  int rc = [&]() -> int {
+    C2B_CUDA(cudaEventRecord(ev[0], st));
+    C2B_TRY(prune_fixed_point(ctx, sets, &cur, &C, &P, &O, &it));
+    C2B_CUDA(cudaEventRecord(ev[1], st));
+    return C2B_OK;
+  }();
+  if (rc == C2B_OK && cur == 1) {
+    std::swap(ctx->cams, ctx->pr_cams[1]);
+    std::swap(ctx->pts_aos, ctx->pr_pts[1]);
+    ctx->out_sel = sel ^ 1;
+  }
+  if (rc != C2B_OK) {
+    // the resident arrays may be half rewritten: nothing of the resident problem is usable any more
+    cudaStreamSynchronize(st);
+    x->have_result = x->have_cameras = x->have_points = false;
+    return rc;
+  }
+  // the culled problem becomes the resident one: camera centres, SoA points, bounds; the point grid is stale
+  ctx->C = C;
+  ctx->out_C = C;
+  ctx->out_O = O;
+  if (C) {
+    double *cx = ctx->cam_center.as<double>();
+    k_cam_prep<<<blocks_for(C, 128), 128, 0, st>>>(ctx->cams.as<double>(), C, cx, cx + C, cx + 2 * C);
+    C2B_KERNEL_CHECK();
+  }
+  C2B_TRY(c2b_points_commit(ctx, P));
+  x->have_result = true;  // the CSR is the graph of the culled problem
+  C2B_CUDA(cudaStreamSynchronize(st));
+  if (out) {
+    memset(out, 0, sizeof *out);
+    out->n_cameras = C;
+    out->n_points = P;
+    out->n_obs = O;
+    out->iterations = it;
+    cudaEventElapsedTime(&out->ms_compute, ev[0], ev[1]);
+  }
+  return C2B_OK;
 }
 
 }  // extern "C"

@@ -228,6 +228,11 @@ struct c2b_ctx {
   c2b::DevBuf nz_cams, nz_centers, nz_pts, nz_uv, nz_scratch;
   float noise_ms[3] = {0, 0, 0};  // last noise call: upload, statistics + kernels, download
 
+  // LCC + remove_singletons (c2b_graph_cull.cuh): the host entry's two problem sets (the resident entry uses set 1
+  // of cameras / points beside the resident arrays), union-find labels, component sizes, counts, ballot words
+  c2b::DevBuf pr_cams[2], pr_pts[2], pr_off[2], pr_idx[2], pr_uv[2];
+  c2b::DevBuf pr_parent, pr_size, pr_cam_cnt, pr_pt_cnt, pr_words, pr_prefix, pr_small;
+
   // host results
   c2b::PinBuf h_offsets, h_idx, h_uv, h_small;
 };

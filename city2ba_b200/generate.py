@@ -321,6 +321,14 @@ class ResidentProblem:
         check(lib().c2b_reprojection_error_resident(self.ctx.handle, float(norm), C.byref(v)))
         return v.value
 
+    def cull(self) -> dict:
+        """BAProblem::cull (LCC + remove_singletons to a fixed point) on the resident problem, in HBM.  Afterwards
+        download / download_problem / reprojection_error / add_* and a new run see the culled problem.  Returns
+        the stats: n_cameras, n_points, n_obs after the cull, iterations, ms_compute (device time)."""
+        st = _lib.CullStats()
+        check(lib().c2b_cull_problem_resident(self.ctx.handle, C.byref(st)))
+        return st.to_dict()
+
 
 def generate_world_points_uniform(xyz, tri, cameras, num_points, max_dist, seed=None, ctx=None) -> np.ndarray:
     """src/generate.rs:356-420 on the GPU: `num_points` points on the mesh (area-weighted triangle,

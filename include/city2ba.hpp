@@ -957,6 +957,42 @@ struct BAProblem {
     }
     return culled;
   }
+  // the same on the GPU (c2b_cull_problem): identical result, bit for bit.  stats (optional) receives the
+  // call's sizes, iteration count and device times.
+  BAProblem cull(const Context &ctx, c2b_cull_stats *stats = nullptr) const {
+    const size_t nc = num_cameras();
+    std::vector<double> cams(nc * C2B_CAM_STRIDE);
+    for (size_t i = 0; i < nc; ++i) std::memcpy(&cams[i * C2B_CAM_STRIDE], cameras[i].rec, sizeof cameras[i].rec);
+    std::vector<double> pts(points.size() * 3);
+    for (size_t i = 0; i < points.size(); ++i) std::memcpy(&pts[3 * i], points[i].data(), 3 * sizeof(double));
+    std::vector<uint64_t> offsets(nc + 1, 0);
+    for (size_t i = 0; i < nc; ++i) offsets[i + 1] = offsets[i] + vis_graph[i].size();
+    std::vector<uint32_t> idx(offsets[nc]);
+    std::vector<double> uv(2 * offsets[nc]);
+    for (size_t i = 0, k = 0; i < nc; ++i)
+      for (const auto &e : vis_graph[i]) {
+        detail::require(e.first <= 0xffffffffull, "point index does not fit 32 bits");
+        idx[k] = (uint32_t)e.first;
+        uv[2 * k] = e.second.first;
+        uv[2 * k + 1] = e.second.second;
+        ++k;
+      }
+    c2b_cull_stats st;
+    detail::check(c2b_cull_problem(ctx.handle(), cams.data(), nc, pts.data(), points.size(), offsets.data(), idx.data(),
+                                   uv.data(), &st));
+    if (stats) *stats = st;
+    BAProblem out;
+    out.cameras.resize(st.n_cameras);
+    for (size_t i = 0; i < st.n_cameras; ++i) std::memcpy(out.cameras[i].rec, &cams[i * C2B_CAM_STRIDE], sizeof out.cameras[i].rec);
+    out.points.resize(st.n_points);
+    for (size_t i = 0; i < st.n_points; ++i) std::memcpy(out.points[i].data(), &pts[3 * i], 3 * sizeof(double));
+    out.vis_graph.resize(st.n_cameras);
+    for (size_t i = 0; i < st.n_cameras; ++i) {
+      out.vis_graph[i].reserve(offsets[i + 1] - offsets[i]);
+      for (uint64_t k = offsets[i]; k < offsets[i + 1]; ++k) out.vis_graph[i].push_back({(size_t)idx[k], {uv[2 * k], uv[2 * k + 1]}});
+    }
+    return out;
+  }
 
   // ---- BAL I/O, src/baproblem.rs:580-785 ----
   // Rust's `{}` for f64: shortest digits that round-trip, positional (never an exponent)

@@ -288,6 +288,36 @@ int c2b_noise_timing(c2b_ctx *ctx, float ms[3]);
 int c2b_mean_std(c2b_ctx *ctx, const double *cams, uint64_t C, const double *pts, uint64_t P,
                  double mean[3], double std[3]);
 
+/* ---- graph post-processing -------------------------------------------------------------------------
+ * replaces BAProblem::cull (src/baproblem.rs:538-549) = largest_connected_component (:456-534, with its
+ * observation filter at :523 as written: the point index looked up as an entity index without the camera offset)
+ * then remove_singletons (:426-453), to a fixed point.  Components are labelled by their smallest entity
+ * (cameras 0..C-1, then points C..C+P-1); the largest wins, the lowest label on a tie (the reference's HashMap
+ * order is unspecified).  Records, points and (u, v) are copied, never recomputed: the result equals the host
+ * mirrors' bit for bit.  Bounds: C + P < 2^32 - 1 and O < 2^32 - 1 (C2B_ERR_INVALID otherwise).
+ * After c2b_visibility_graph_multi the graph is spread over the GPUs: cull its host CSR with c2b_cull_problem on
+ * c2b_multi_ctx(m, 0). */
+typedef struct {
+  uint64_t n_cameras, n_points, n_obs; /* after the cull */
+  uint32_t iterations;                 /* applications of LCC + remove_singletons, as the reference's loop */
+  uint32_t reserved;
+  float ms_h2d, ms_compute, ms_d2h;    /* device time (CUDA events on the ctx stream); h2d/d2h 0 when resident;
+                                          ms_h2d includes the input check */
+} c2b_cull_stats;
+/* in place on host arrays: the culled problem is written into the prefixes of cams / pts / offsets /
+ * point_idx / uv.  O = offsets[C], and point_idx / uv must hold O entries: they are read up to that length before
+ * anything is checked, so offsets[C] has to be the arrays' length even when other offsets are wrong.  Rejects offsets[0] != 0, decreasing offsets and point_idx >= P
+ * (from_visibility's asserts) with C2B_ERR_INVALID and leaves the arrays untouched.  Does not touch the
+ * ctx's resident problem.  out may be NULL. */
+int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64_t P, uint64_t *offsets,
+                     uint32_t *point_idx, double *uv, c2b_cull_stats *out);
+/* the same on the resident problem: the cameras / points of the last c2b_upload_* calls and the CSR of the last
+ * c2b_visibility_graph_resident.  Afterwards c2b_download_obs / c2b_download_problem /
+ * c2b_reprojection_error_resident / c2b_add_*_resident see the culled problem, and a new
+ * c2b_visibility_graph_resident computes the culled problem's graph.  C2B_ERR_INVALID without a resident result,
+ * and after the host-buffer c2b_visibility_graph (which leaves only its last camera batch resident). */
+int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out);
+
 /* ---- input generation on the GPU -------------------------------------------------------------------
  * replaces generate_world_points_uniform (src/generate.rs:356-420): num_points world points, each
  * on an area-weighted random triangle (all index triples of all models, concatenated), uniform

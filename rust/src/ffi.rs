@@ -40,6 +40,14 @@ pub struct c2b_multi_stats {
     pub ms_wall: c_float,
 }
 
+// BAProblem::cull on the GPU (c2b_cull_problem / c2b_cull_problem_resident)
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct c2b_cull_stats {
+    pub n_cameras: u64, pub n_points: u64, pub n_obs: u64,
+    pub iterations: u32, pub reserved: u32,
+    pub ms_h2d: c_float, pub ms_compute: c_float, pub ms_d2h: c_float,
+}
+
 // Embree's RTCRay layout (48 bytes): what embree_rs::Ray wraps (src/generate.rs:253-262, :457-464)
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct c2b_ray48 {
@@ -123,6 +131,11 @@ extern "C" {
     pub fn c2b_noise_timing(ctx: *mut c2b_ctx, ms: *mut c_float) -> c_int;
     pub fn c2b_mean_std(ctx: *mut c2b_ctx, cams: *const c_double, c: u64, pts: *const c_double, p: u64,
                         mean: *mut c_double, std: *mut c_double) -> c_int;
+    // ---- graph post-processing: a Rust BAProblem::cull would call c2b_cull_problem (INTEGRATION.md) ----
+    pub fn c2b_cull_problem(ctx: *mut c2b_ctx, cams: *mut c_double, c: u64, pts: *mut c_double, p: u64,
+                            offsets: *mut u64, point_idx: *mut u32, uv: *mut c_double,
+                            out: *mut c2b_cull_stats) -> c_int;
+    pub fn c2b_cull_problem_resident(ctx: *mut c2b_ctx, out: *mut c2b_cull_stats) -> c_int;
     // ---- input generation ----
     pub fn c2b_generate_world_points_uniform(ctx: *mut c2b_ctx, xyz: *const c_float, nv: u64, tri: *const u32,
                                              nt: u64, cams: *const c_double, c: u64, num_points: u64,
