@@ -310,6 +310,14 @@ class ResidentProblem:
         check(lib().c2b_add_noise_resident(self.ctx.handle, float(translation_std), float(rotation_std),
                                            float(point_std), float(observations_std), int(seed)))
 
+    def add_sin_noise(self, direction, noise_direction, strength, frequency):
+        """noise::add_sin_noise on the resident cameras / points (dimensions from their extent)"""
+        pd = C.POINTER(C.c_double)
+        d = np.ascontiguousarray(direction, np.float64)
+        nd = np.ascontiguousarray(noise_direction, np.float64)
+        check(lib().c2b_add_sin_noise_resident(self.ctx.handle, d.ctypes.data_as(pd), nd.ctypes.data_as(pd),
+                                               float(strength), float(frequency)))
+
     def download_problem(self, num_cameras: int, num_points: int):
         cams, pts = np.empty((num_cameras, CAM_STRIDE)), np.empty((num_points, 3))
         pd = C.POINTER(C.c_double)
