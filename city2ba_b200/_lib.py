@@ -92,7 +92,20 @@ class CullStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
 
 
+class BalStats(C.Structure):
+    """c2b_bal_stats: bytes and chunks of one BAL file, device ms of encode / D2H, host ms of write(2)"""
+    _fields_ = [
+        ("bytes", C.c_uint64), ("chunks", C.c_uint64),
+        ("ms_encode", C.c_float), ("ms_d2h", C.c_float), ("ms_write", C.c_float),
+    ]
+
+    def to_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 CULL_GRID, CULL_EXHAUSTIVE = 0, 1
+BAL_TEXT, BAL_BINARY = 0, 1
+ERR_INVALID, ERR_IO = -1, -7
 OCC_MESH, OCC_NONE, OCC_ANALYTIC = 0, 1, 2
 PRED_WATERTIGHT, PRED_MT = 0, 1
 
@@ -108,11 +121,12 @@ EXPORTS = [
     "c2b_visibility_graph_resident", "c2b_download_obs", "c2b_reprojection_error_resident",
     "c2b_add_drift", "c2b_add_drift_normalized", "c2b_add_noise", "c2b_add_sin_noise", "c2b_noise_timing",
     "c2b_add_drift_resident", "c2b_add_noise_resident", "c2b_add_sin_noise_resident", "c2b_download_problem",
-    "c2b_mean_std", "c2b_cull_problem", "c2b_cull_problem_resident", "c2b_generate_world_points_uniform",
+    "c2b_mean_std", "c2b_cull_problem", "c2b_cull_problem_resident", "c2b_write_bal", "c2b_write_bal_resident",
+    "c2b_generate_world_points_uniform",
     "c2b_grid_num_cameras", "c2b_grid_num_points", "c2b_grid_cameras", "c2b_grid_points",
     "c2b_line_cameras", "c2b_line_points", "c2b_city_mesh", "c2b_camera_center",
     "c2b_camera_project_world", "c2b_camera_project", "c2b_camera_from_position_direction",
-    "c2b_camera_transform",
+    "c2b_camera_transform", "c2b_camera_to_vec",
 ]
 
 _lib = None
@@ -188,6 +202,8 @@ def lib():
     L.c2b_mean_std.argtypes = [vp, pd, u64, pd, u64, pd, pd]
     L.c2b_cull_problem.argtypes = [vp, pd, u64, pd, u64, C.POINTER(u64), pu32, pd, C.POINTER(CullStats)]
     L.c2b_cull_problem_resident.argtypes = [vp, C.POINTER(CullStats)]
+    L.c2b_write_bal.argtypes = [vp, C.c_char_p, i32, pd, u64, pd, u64, C.POINTER(u64), pu32, pd, C.POINTER(BalStats)]
+    L.c2b_write_bal_resident.argtypes = [vp, C.c_char_p, i32, C.POINTER(BalStats)]
     L.c2b_probe_fp64.argtypes = [vp, pd]
     L.c2b_generate_world_points_uniform.argtypes = [vp, pf, u64, pu32, u64, pd, u64, u64, dbl, u64, pd,
                                                     C.POINTER(u64)]
@@ -210,6 +226,8 @@ def lib():
     L.c2b_camera_from_position_direction.restype = None
     L.c2b_camera_transform.argtypes = [pd, pd, pd, pd]
     L.c2b_camera_transform.restype = None
+    L.c2b_camera_to_vec.argtypes = [pd, pd]
+    L.c2b_camera_to_vec.restype = None
     _lib = L
     return L
 

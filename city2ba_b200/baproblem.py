@@ -478,17 +478,51 @@ class BAProblem:
             for p in self.points:
                 f.write(f"{fmt(p[0])} {fmt(p[1])} {fmt(p[2])}\n")
 
-    def write(self, path):
-        """src/baproblem.rs:768-785"""
+    @staticmethod
+    def _bal_binary(path):
+        """src/baproblem.rs:768-785: the extension picks the format (True: .bbal, False: .bal)"""
         path = str(path)
         if "." not in path.rsplit("/", 1)[-1]:
             raise IOError_("file does not have an extension")
         ext = path.rsplit(".", 1)[-1]
-        if ext == "bal":
-            return self.write_text(path)
-        if ext == "bbal":
-            return self.write_binary(path)
-        raise IOError_(f"unknown file extension {ext}")
+        if ext not in ("bal", "bbal"):
+            raise IOError_(f"unknown file extension {ext}")
+        return ext == "bbal"
+
+    def write(self, path):
+        """src/baproblem.rs:768-785"""
+        return self.write_binary(path) if self._bal_binary(path) else self.write_text(path)
+
+    def write_gpu(self, path, ctx=None, stats=None):
+        """write() with the file encoded on the GPU (c2b_write_bal) and streamed to disk in chunks.  The bytes are
+        the reference's: the shortest round-trip digits of every value, positional, camera vectors from the host's
+        to_vec (c2b_camera_to_vec).  `stats`, a dict if given, receives bytes, chunks and the encode / D2H / write
+        times."""
+        from ._lib import C2BError, BalStats, BAL_BINARY, BAL_TEXT, ERR_IO
+        fmt = BAL_BINARY if self._bal_binary(path) else BAL_TEXT
+        ctx = ctx or context()
+        g = self.vis_graph
+        cams = np.ascontiguousarray(self.cameras, np.float64).reshape(-1, CAM_STRIDE)
+        pts = np.ascontiguousarray(self.points, np.float64).reshape(-1, 3)
+        off = np.ascontiguousarray(g.offsets, np.uint64)
+        if len(off) != len(cams) + 1:
+            raise ValueError("cameras and CSR offsets disagree")
+        idx = g.point_idx
+        if len(idx) and int(idx.max()) > 0xffffffff:
+            raise ValueError("point index does not fit 32 bits")
+        idx = np.ascontiguousarray(idx, np.uint32)
+        uv = np.ascontiguousarray(g.uv, np.float64).reshape(-1, 2)
+        st = BalStats()
+        try:
+            check(lib().c2b_write_bal(ctx.handle, str(path).encode(), fmt, _p(cams), len(cams), _p(pts), len(pts),
+                                      off.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                      idx.ctypes.data_as(C.POINTER(C.c_uint32)), _p(uv), C.byref(st)))
+        except C2BError as e:
+            if e.code == ERR_IO:
+                raise IOError_(str(e)) from e
+            raise
+        if stats is not None:
+            stats.update(st.to_dict())
 
     @classmethod
     def from_file_binary(cls, path):

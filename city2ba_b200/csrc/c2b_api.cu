@@ -14,9 +14,13 @@
 #include <vector>
 
 #if defined(__linux__)
+#include <cerrno>
+#include <fcntl.h>
 #include <sys/mman.h>
+#include <sys/stat.h>
 #endif
 
+#include "c2b_bal.cuh"
 #include "c2b_bvh.cuh"
 #include "c2b_common.cuh"
 #include "c2b_compact.cuh"
@@ -113,6 +117,7 @@ struct Tunables {
                                    // same 32 warps per SM a warp's epilogue is just appended to its serial
                                    // chain, and warps parked in its latency-bound loops leave fewer warps to
                                    // fill the issue slots (64.6 % issue-active against 77 %; profiles/r02f)
+  uint64_t bal_chunk_bytes = 1ull << 25;  // BAL writer: bytes per chunk (device buffer, pinned ring slot)
 };
 
 // Pageable host memory backed by transparent huge pages (mmap + MADV_HUGEPAGE): what the FIRST host-buffer call
@@ -277,10 +282,15 @@ struct CtxExtra {
   bool grid_locked = false;  // inside c2b_visibility_graph: the grid was built for all of the call's cameras
   PageBuf pg_idx, pg_uv;     // first host-buffer call: unpinned result arrays (see PageBuf)
   PinBuf pin_out;            // and the ring they are filled through
+  // BAL writer (c2b_bal.cuh): window lengths / offsets, two chunk buffers, camera 9-vectors, pinned chunk ring
+  DevBuf bal_scan, bal_out[2], bal_vecs;
+  PinBuf bal_ring;
   ~CtxExtra() {
     pg_idx.release();
     pg_uv.release();
     pin_out.release();
+    for (DevBuf *b : {&bal_scan, &bal_out[0], &bal_out[1], &bal_vecs}) b->release();
+    bal_ring.release();
   }
   GridCache grid;
   uint64_t points_version = 0;
@@ -320,6 +330,7 @@ static bool tune(Tunables &t, const char *name, double v) {
   else if (n == "epilogue") t.epilogue = v != 0;
   else if (n == "optimistic") t.optimistic = v != 0;
   else if (n == "cold_staged") t.cold_staged = v != 0;
+  else if (n == "bal_chunk_bytes") t.bal_chunk_bytes = (uint64_t)(v >= 4096.0 ? std::min(v, 1073741824.0) : 4096.0) & ~7ull;
   else return false;
   return true;
 }
@@ -400,7 +411,8 @@ int c2b_init(int device, c2b_ctx **out) {
         {"C2B_PARTS_LOG2", "parts_log2"}, {"C2B_TRILIST_CAP", "trilist_cap"}, {"C2B_MAX_PAIRS", "max_pairs"},
         {"C2B_HOIST_MAX", "hoist_max"}, {"C2B_PACKET_BVH", "packet_bvh"}, {"C2B_TRILIST_WARP", "trilist_warp"},
         {"C2B_BATCHES", "batches"}, {"C2B_FU_OCC3", "fu_occ3"}, {"C2B_GRID_CELL_FACTOR", "grid_cell_factor"},
-        {"C2B_STAGE_THREADS", "stage_threads"}, {"C2B_EPILOGUE", "epilogue"}, {"C2B_OPTIMISTIC", "optimistic"}, {"C2B_COLD_STAGED", "cold_staged"}};
+        {"C2B_STAGE_THREADS", "stage_threads"}, {"C2B_EPILOGUE", "epilogue"}, {"C2B_OPTIMISTIC", "optimistic"}, {"C2B_COLD_STAGED", "cold_staged"},
+        {"C2B_BAL_CHUNK_BYTES", "bal_chunk_bytes"}};
     for (auto &h : hooks)
       if (const char *e = getenv(h.env)) (void)tune(x->tun, h.name, atof(e));
   }
@@ -2555,6 +2567,275 @@ int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
     cudaEventElapsedTime(&out->ms_compute, ev[0], ev[1]);
   }
   return C2B_OK;
+}
+
+
+// ---- BAL files (c2b_bal.cuh) ----------------------------------------------------------------------------------
+namespace {
+constexpr int BAL_RING = 3;                 // pinned chunk slots: D2H of chunk k while chunk k-1 is written
+constexpr uint32_t BAL_WINDOW = 1u << 20;   // lines per length pass: 2^20 lines of <= 2952 bytes keep the u32 scan exact
+
+struct BalEvents {  // per ring slot: encode start / end (ctx stream), copy start / end (copy stream)
+  cudaEvent_t e[BAL_RING][4] = {};
+  int create() {
+    for (auto &s : e)
+      for (auto &x : s) C2B_CUDA(cudaEventCreate(&x));
+    return C2B_OK;
+  }
+  ~BalEvents() {
+    for (auto &s : e)
+      for (auto x : s)
+        if (x) cudaEventDestroy(x);
+  }
+};
+
+// the camera 9-vectors of C records (host memory) -> x->bal_vecs
+int bal_upload_vecs(c2b_ctx *ctx, CtxExtra *x, const double *cams, uint64_t C) {
+  C2B_TRY(x->bal_vecs.ensure(std::max<uint64_t>(C, 1) * 72));
+  if (!C) return C2B_OK;
+  std::vector<double> vecs(9 * C);
+  for (uint64_t c = 0; c < C; ++c) c2b_camera_to_vec(cams + 15 * c, &vecs[9 * c]);
+  C2B_CUDA(cudaMemcpyAsync(x->bal_vecs.p, vecs.data(), C * 72, cudaMemcpyHostToDevice, ctx->stream));
+  C2B_CUDA(cudaStreamSynchronize(ctx->stream));  // vecs is freed on return
+  return C2B_OK;
+}
+
+// Encodes the problem `v` (device arrays) chunk by chunk and writes it to `path`.  Chunk k: the encoding kernels on
+// the ctx stream into device buffer k % 2, its copy on the copy stream into ring slot k % 3, then write(2) on a
+// writer thread; the host waits only for the chunk's line count (text) and for a free ring slot.
+int bal_stream(c2b_ctx *ctx, const char *path, int format, const BalView &v, c2b_bal_stats *out) {
+  CtxExtra *x = extra_of(ctx);
+  const uint64_t B = x->tun.bal_chunk_bytes;
+  const bool text = format == C2B_BAL_TEXT;
+  cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+  C2B_TRY(x->bal_out[0].ensure(B));
+  C2B_TRY(x->bal_out[1].ensure(B));
+  x->bal_ring.node = ctx->numa_node;
+  C2B_TRY(x->bal_ring.ensure(BAL_RING * B));
+  if (text) {
+    C2B_TRY(x->bal_scan.ensure((size_t)(BAL_WINDOW + 1) * 4));
+    C2B_TRY(ctx->h_small.ensure(256));
+  }
+  BalEvents events;
+  C2B_TRY(events.create());
+  auto &ev = events.e;
+  const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC | O_CLOEXEC, 0666);
+  if (fd < 0) return set_error(C2B_ERR_IO, "cannot create %s: %s", path, strerror(errno));
+  struct stat sb;
+  const bool regular = fstat(fd, &sb) == 0 && S_ISREG(sb.st_mode);  // /dev/null and pipes are never removed
+
+  struct Job {
+    int slot;
+    uint64_t bytes;
+  };
+  std::mutex mu;
+  std::condition_variable cv;
+  std::deque<Job> jobs;
+  bool quit = false;
+  uint64_t chunks_done = 0;
+  int io_errno = 0;
+  cudaError_t cuda_err = cudaSuccess;
+  float ms_encode = 0, ms_d2h = 0;
+  double ms_write = 0;
+  char *ring = x->bal_ring.as<char>();
+  const int device = ctx->device;
+  std::thread writer([&]() {
+    cudaError_t e = cudaSetDevice(device);
+    for (;;) {
+      Job j;
+      {
+        std::unique_lock<std::mutex> lk(mu);
+        cv.wait(lk, [&] { return !jobs.empty() || quit; });
+        if (jobs.empty()) break;
+        j = jobs.front();
+        jobs.pop_front();
+      }
+      if (e == cudaSuccess) e = cudaEventSynchronize(ev[j.slot][3]);
+      float a = 0, b = 0;
+      int err = 0;
+      double ms = 0;
+      if (e == cudaSuccess) {
+        cudaEventElapsedTime(&a, ev[j.slot][0], ev[j.slot][1]);
+        cudaEventElapsedTime(&b, ev[j.slot][2], ev[j.slot][3]);
+        const auto t0 = std::chrono::steady_clock::now();
+        const char *p = ring + (size_t)j.slot * B;
+        for (uint64_t left = j.bytes; left && !io_errno;) {
+          const ssize_t r = ::write(fd, p, left);
+          if (r < 0 && errno == EINTR) continue;
+          if (r <= 0) {
+            err = r < 0 ? errno : EIO;
+            break;
+          }
+          p += r;
+          left -= (uint64_t)r;
+        }
+        ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+      }
+      {
+        std::lock_guard<std::mutex> lk(mu);
+        ms_encode += a;
+        ms_d2h += b;
+        ms_write += ms;
+        if (err && !io_errno) io_errno = err;
+        if (e != cudaSuccess) cuda_err = e;
+        ++chunks_done;
+      }
+      cv.notify_all();
+    }
+  });
+
+  uint64_t chunks = 0, bytes = 0;
+  int rc = [&]() -> int {
+    const uint64_t units = text ? 1 + v.O + v.C + v.P : 3 + v.C + 3 * v.O + 9 * v.C + 3 * v.P;  // lines or words
+    uint32_t window = (uint32_t)std::min<uint64_t>(BAL_WINDOW, std::max<uint64_t>(1024, B / 64));
+    uint32_t *scan = x->bal_scan.as<uint32_t>();
+    const uint32_t *res = ctx->h_small.as<uint32_t>();
+    for (uint64_t pos = 0; pos < units; ++chunks) {
+      const int slot = (int)(chunks % BAL_RING);
+      char *dbuf = x->bal_out[chunks % 2].as<char>();
+      {
+        std::unique_lock<std::mutex> lk(mu);
+        cv.wait(lk, [&] { return chunks_done + BAL_RING > chunks; });  // the slot's previous chunk is on disk
+        if (io_errno) return set_error(C2B_ERR_IO, "write to %s failed: %s", path, strerror(io_errno));
+        if (cuda_err != cudaSuccess) return set_error(C2B_ERR_CUDA, "BAL chunk copy: %s", cudaGetErrorString(cuda_err));
+      }
+      // the device buffer's previous chunk (k - 2) has been copied out
+      if (chunks >= 2) C2B_CUDA(cudaStreamWaitEvent(st, ev[(chunks - 2) % BAL_RING][3], 0));
+      C2B_CUDA(cudaEventRecord(ev[slot][0], st));
+      uint64_t n_bytes;
+      if (text) {
+        const uint32_t n = (uint32_t)std::min<uint64_t>(window, units - pos);
+        k_bal_text_len<<<blocks_for(n, BAL_THREADS), BAL_THREADS, 0, st>>>(v, pos, n, scan);
+        C2B_KERNEL_CHECK();
+        C2B_TRY(exclusive_scan_u32(st, scan, scan, n, scan + BAL_WINDOW, ctx->scan_tmp));
+        k_bal_text_cut<<<1, 1, 0, st>>>(scan, scan + BAL_WINDOW, n, (uint32_t)B, ctx->h_small.as<uint32_t>());
+        C2B_KERNEL_CHECK();
+        C2B_CUDA(cudaStreamSynchronize(st));
+        const uint32_t k = res[0];
+        n_bytes = res[1];
+        k_bal_text_write<<<blocks_for(k, BAL_THREADS), BAL_THREADS, 0, st>>>(v, pos, k, scan, dbuf);
+        C2B_KERNEL_CHECK();
+        pos += k;
+        // next window: the lines that fitted, and some more; twice as many when all of them fitted
+        window = (uint32_t)std::min<uint64_t>(BAL_WINDOW, k == n ? 2ull * n : k + k / 8 + 64);
+      } else {
+        const uint64_t n = std::min<uint64_t>(B / 8, units - pos);
+        k_bal_binary<<<(unsigned)((n + BAL_THREADS - 1) / BAL_THREADS), BAL_THREADS, 0, st>>>(
+            v, pos, n, reinterpret_cast<uint64_t *>(dbuf));
+        C2B_KERNEL_CHECK();
+        n_bytes = 8 * n;
+        pos += n;
+      }
+      C2B_CUDA(cudaEventRecord(ev[slot][1], st));
+      C2B_CUDA(cudaStreamWaitEvent(cp, ev[slot][1], 0));
+      C2B_CUDA(cudaEventRecord(ev[slot][2], cp));
+      C2B_CUDA(cudaMemcpyAsync(ring + (size_t)slot * B, dbuf, n_bytes, cudaMemcpyDeviceToHost, cp));
+      C2B_CUDA(cudaEventRecord(ev[slot][3], cp));
+      {
+        std::lock_guard<std::mutex> lk(mu);
+        jobs.push_back(Job{slot, n_bytes});
+      }
+      cv.notify_all();
+      bytes += n_bytes;
+    }
+    return C2B_OK;
+  }();
+  {
+    std::lock_guard<std::mutex> lk(mu);
+    quit = true;
+  }
+  cv.notify_all();
+  writer.join();
+  if (rc == C2B_OK && io_errno) rc = set_error(C2B_ERR_IO, "write to %s failed: %s", path, strerror(io_errno));
+  if (rc == C2B_OK && cuda_err != cudaSuccess)
+    rc = set_error(C2B_ERR_CUDA, "BAL chunk copy: %s", cudaGetErrorString(cuda_err));
+  if (close(fd) != 0 && rc == C2B_OK) rc = set_error(C2B_ERR_IO, "closing %s failed: %s", path, strerror(errno));
+  if (rc != C2B_OK) {
+    cudaStreamSynchronize(st);
+    cudaStreamSynchronize(cp);
+    if (regular) unlink(path);  // no truncated file behind a failed call
+    return rc;
+  }
+  if (out) {
+    memset(out, 0, sizeof *out);
+    out->bytes = bytes;
+    out->chunks = chunks;
+    out->ms_encode = ms_encode;
+    out->ms_d2h = ms_d2h;
+    out->ms_write = (float)ms_write;
+  }
+  return C2B_OK;
+}
+}  // namespace
+
+int c2b_write_bal(c2b_ctx *ctx, const char *path, int format, const double *cams, uint64_t C, const double *pts,
+                  uint64_t P, const uint64_t *offsets, const uint32_t *point_idx, const double *uv,
+                  c2b_bal_stats *out) {
+  if (!ctx || !path || !offsets || (C && !cams) || (P && !pts)) return set_error(C2B_ERR_INVALID, "c2b_write_bal: null argument");
+  if (format != C2B_BAL_TEXT && format != C2B_BAL_BINARY) return set_error(C2B_ERR_INVALID, "c2b_write_bal: unknown format %d", format);
+  const uint64_t O = offsets[C];
+  if (O && (!point_idx || !uv)) return set_error(C2B_ERR_INVALID, "c2b_write_bal: null observation array");
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  CtxExtra *x = extra_of(ctx);
+  // the cull's host-entry buffers (set 0): never the resident problem
+  C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
+  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
+  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
+  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
+  C2B_TRY(ctx->pr_small.ensure(64));
+  C2B_TRY(ctx->h_small.ensure(256));
+  int rc = [&]() -> int {
+    if (P) C2B_TRY(copy_in(ctx, ctx->pr_pts[0].p, pts, P * 24, cudaMemcpyHostToDevice));
+    C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
+    if (O) {
+      C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
+      C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
+    }
+    // the checks of c2b_cull_problem (from_visibility's asserts), before the file exists
+    uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
+    C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+    const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
+    k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
+        ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, P, flag);
+    C2B_KERNEL_CHECK();
+    C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    const uint32_t bad = *ctx->h_small.as<uint32_t>();
+    if (bad & 1u) return set_error(C2B_ERR_INVALID, "c2b_write_bal: offsets[0] != 0 or the CSR offsets decrease");
+    if (bad & 2u) return set_error(C2B_ERR_INVALID, "c2b_write_bal: an observation references a point >= %llu",
+                                   (unsigned long long)P);
+    C2B_TRY(bal_upload_vecs(ctx, x, cams, C));
+    const BalView v{x->bal_vecs.as<double>(), ctx->pr_pts[0].as<double>(), ctx->pr_off[0].as<uint64_t>(),
+                    ctx->pr_idx[0].as<uint32_t>(), ctx->pr_uv[0].as<double>(), C, P, O};
+    return bal_stream(ctx, path, format, v, out);
+  }();
+  if (rc != C2B_OK) cudaStreamSynchronize(st);
+  return rc;
+}
+
+int c2b_write_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_stats *out) {
+  if (!ctx || !path) return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: null argument");
+  if (format != C2B_BAL_TEXT && format != C2B_BAL_BINARY)
+    return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: unknown format %d", format);
+  CtxExtra *x = extra_of(ctx);
+  if (x->host_call_last)
+    return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: the resident CSR is the last camera batch of the "
+                                      "host-buffer c2b_visibility_graph, not the graph of an uploaded problem; run "
+                                      "c2b_visibility_graph_resident first");
+  if (!x->have_result || !x->have_points || !x->have_cameras)
+    return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: no resident result (upload cameras and points, "
+                                      "then c2b_visibility_graph_resident)");
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  const uint64_t C = ctx->out_C, P = ctx->P, O = ctx->out_O;
+  const int sel = ctx->out_sel;
+  std::vector<double> cams(15 * C);
+  if (C) C2B_CUDA(cudaMemcpyAsync(cams.data(), ctx->cams.p, C * 120, cudaMemcpyDeviceToHost, ctx->stream));
+  C2B_CUDA(cudaStreamSynchronize(ctx->stream));
+  C2B_TRY(bal_upload_vecs(ctx, x, cams.data(), C));
+  const BalView v{x->bal_vecs.as<double>(), ctx->pts_aos.as<double>(), ctx->out_offsets[sel].as<uint64_t>(),
+                  ctx->out_idx[sel].as<uint32_t>(), ctx->out_uv[sel].as<double>(), C, P, O};
+  return bal_stream(ctx, path, format, v, out);
 }
 
 }  // extern "C"

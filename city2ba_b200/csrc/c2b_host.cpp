@@ -3,6 +3,7 @@
 // src/synthetic.rs:178-258, 323-344), the city-block box mesh that stands in for the OBJ scene
 // on synthetic cities, and SnavelyCamera helpers for the host mirror.  No GPU work here.
 // Compiled with -ffp-contract=off (c2b_math.cuh's host path relies on it).
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 
@@ -173,6 +174,47 @@ void c2b_camera_transform(const double *cam, const double dR[9], const double dl
   memcpy(c, cam, sizeof c);
   camera_transform(c, dR, V3{dloc[0], dloc[1], dloc[2]}, out);
   memcpy(cam_out, out, sizeof out);
+}
+
+// SnavelyCamera::to_vec (src/baproblem.rs:192-202, to_rodrigues :93-102): the same operations in the same order as
+// include/city2ba.hpp's to_vec / to_rodrigues / detail::quat_from_mat, so that the BAL writer's camera lines equal
+// the C++ mirror's bit for bit (acos is the host libm's; the device's differs)
+void c2b_camera_to_vec(const double *cam, double out[9]) {
+  auto M = [&](int c, int r) { return cam[c * 3 + r]; };
+  double q[4];
+  const double trace = (M(0, 0) + M(1, 1)) + M(2, 2);
+  if (trace >= 0.0) {
+    double s = std::sqrt(1.0 + trace);
+    const double w = 0.5 * s;
+    s = 0.5 / s;
+    q[0] = w, q[1] = (M(1, 2) - M(2, 1)) * s, q[2] = (M(2, 0) - M(0, 2)) * s, q[3] = (M(0, 1) - M(1, 0)) * s;
+  } else if (M(0, 0) > M(1, 1) && M(0, 0) > M(2, 2)) {
+    double s = std::sqrt(((M(0, 0) - M(1, 1)) - M(2, 2)) + 1.0);
+    const double x = 0.5 * s;
+    s = 0.5 / s;
+    q[0] = (M(1, 2) - M(2, 1)) * s, q[1] = x, q[2] = (M(1, 0) + M(0, 1)) * s, q[3] = (M(0, 2) + M(2, 0)) * s;
+  } else if (M(1, 1) > M(2, 2)) {
+    double s = std::sqrt(((M(1, 1) - M(0, 0)) - M(2, 2)) + 1.0);
+    const double y = 0.5 * s;
+    s = 0.5 / s;
+    q[0] = (M(2, 0) - M(0, 2)) * s, q[1] = (M(1, 0) + M(0, 1)) * s, q[2] = y, q[3] = (M(2, 1) + M(1, 2)) * s;
+  } else {
+    double s = std::sqrt(((M(2, 2) - M(0, 0)) - M(1, 1)) + 1.0);
+    const double z = 0.5 * s;
+    s = 0.5 / s;
+    q[0] = (M(0, 1) - M(1, 0)) * s, q[1] = (M(0, 2) + M(2, 0)) * s, q[2] = (M(2, 1) + M(1, 2)) * s, q[3] = z;
+  }
+  const double angle = 2.0 * std::acos(std::max(-1.0, std::min(1.0, q[0])));
+  const double d = 1.0 - q[0] * q[0];
+  if (d < 2.220446049250313e-16) {
+    out[0] = out[1] = out[2] = 0.0;
+  } else {
+    const double sd = std::sqrt(d);
+    const double a[3] = {q[1] / sd, q[2] / sd, q[3] / sd};
+    const double inv = 1.0 / std::sqrt((a[0] * a[0] + a[1] * a[1]) + a[2] * a[2]);
+    for (int k = 0; k < 3; ++k) out[k] = a[k] * inv * angle;
+  }
+  for (int k = 0; k < 6; ++k) out[3 + k] = cam[9 + k];
 }
 
 }  // extern "C"

@@ -337,6 +337,21 @@ class ResidentProblem:
         check(lib().c2b_cull_problem_resident(self.ctx.handle, C.byref(st)))
         return st.to_dict()
 
+    def write(self, path) -> dict:
+        """BAProblem::write of the resident problem (c2b_write_bal_resident): .bal text or .bbal binary by the
+        extension, encoded on the GPU and streamed to disk.  Returns the stats: bytes, chunks, ms_encode, ms_d2h
+        (device time), ms_write (host time in write(2))."""
+        from .baproblem import BAProblem, IOError_
+        fmt = _lib.BAL_BINARY if BAProblem._bal_binary(path) else _lib.BAL_TEXT
+        st = _lib.BalStats()
+        try:
+            check(lib().c2b_write_bal_resident(self.ctx.handle, str(path).encode(), fmt, C.byref(st)))
+        except _lib.C2BError as e:
+            if e.code == _lib.ERR_IO:
+                raise IOError_(str(e)) from e
+            raise
+        return st.to_dict()
+
 
 def generate_world_points_uniform(xyz, tri, cameras, num_points, max_dist, seed=None, ctx=None) -> np.ndarray:
     """src/generate.rs:356-420 on the GPU: `num_points` points on the mesh (area-weighted triangle,

@@ -55,7 +55,8 @@ struct Error : std::runtime_error {
 namespace detail {
 inline void check(int rc) {
   if (rc == C2B_OK) return;
-  throw Error(rc == C2B_ERR_EMPTY ? Error::EmptyProblem : Error::Gpu, c2b_last_error());
+  throw Error(rc == C2B_ERR_EMPTY ? Error::EmptyProblem : rc == C2B_ERR_IO ? Error::IOError : Error::Gpu,
+              c2b_last_error());
 }
 inline void require(bool ok, const char *what) {
   if (!ok) throw std::logic_error(what);  // the reference's assert! / panic!
@@ -1048,15 +1049,45 @@ struct BAProblem {
     if (!f) throw Error(Error::IOError, "write failed: " + path);
   }
   // src/baproblem.rs:768-785: the extension picks the format
-  void write(const std::string &path) const {
+  static c2b_bal_format bal_format(const std::string &path) {
     const auto dot = path.rfind('.');
     const std::string ext = dot == std::string::npos ? "" : path.substr(dot + 1);
-    if (ext == "bal")
+    if (ext == "bal") return C2B_BAL_TEXT;
+    if (ext == "bbal") return C2B_BAL_BINARY;
+    throw Error(Error::IOError, "unknown file extension: " + path);
+  }
+  void write(const std::string &path) const {
+    if (bal_format(path) == C2B_BAL_TEXT)
       write_text(path);
-    else if (ext == "bbal")
-      write_binary(path);
     else
-      throw Error(Error::IOError, "unknown file extension: " + path);
+      write_binary(path);
+  }
+  // the same file encoded on the GPU and streamed to disk (c2b_write_bal).  The bytes are the reference's, which
+  // write_text's std::to_chars does not give for |values| >= 2^53 and NaN (DESIGN.md, BAL files); the camera vectors
+  // are to_vec's, bit for bit.  stats (optional) receives bytes, chunks and the encode / D2H / write times.
+  void write(const Context &ctx, const std::string &path, c2b_bal_stats *stats = nullptr) const {
+    const c2b_bal_format format = bal_format(path);
+    const size_t nc = num_cameras();
+    std::vector<double> cams(nc * C2B_CAM_STRIDE);
+    for (size_t i = 0; i < nc; ++i) std::memcpy(&cams[i * C2B_CAM_STRIDE], cameras[i].rec, sizeof cameras[i].rec);
+    std::vector<double> pts(points.size() * 3);
+    for (size_t i = 0; i < points.size(); ++i) std::memcpy(&pts[3 * i], points[i].data(), 3 * sizeof(double));
+    std::vector<uint64_t> offsets(nc + 1, 0);
+    for (size_t i = 0; i < nc; ++i) offsets[i + 1] = offsets[i] + vis_graph[i].size();
+    std::vector<uint32_t> idx(offsets[nc]);
+    std::vector<double> uv(2 * offsets[nc]);
+    for (size_t i = 0, k = 0; i < nc; ++i)
+      for (const auto &e : vis_graph[i]) {
+        detail::require(e.first <= 0xffffffffull, "point index does not fit 32 bits");
+        idx[k] = (uint32_t)e.first;
+        uv[2 * k] = e.second.first;
+        uv[2 * k + 1] = e.second.second;
+        ++k;
+      }
+    c2b_bal_stats st;
+    detail::check(c2b_write_bal(ctx.handle(), path.c_str(), format, cams.data(), nc, pts.data(), points.size(),
+                                offsets.data(), idx.data(), uv.data(), &st));
+    if (stats) *stats = st;
   }
   // src/baproblem.rs:580-706
   static BAProblem from_file(const std::string &path) {

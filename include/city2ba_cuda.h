@@ -31,7 +31,8 @@ typedef enum {
   C2B_ERR_CUDA = -3,      /* a CUDA runtime call or kernel failed; message has the detail */
   C2B_ERR_OOM = -4,       /* device or pinned-host allocation failed                      */
   C2B_ERR_EMPTY = -5,     /* empty problem (reference: Error::EmptyProblem, src/baproblem.rs:36) */
-  C2B_ERR_NCCL = -6       /* libnccl.so.2 could not be loaded, or an NCCL call failed (multi-GPU entries only) */
+  C2B_ERR_NCCL = -6,      /* libnccl.so.2 could not be loaded, or an NCCL call failed (multi-GPU entries only) */
+  C2B_ERR_IO = -7         /* a file could not be created, or a write was short (reference: Error::IOError) */
 } c2b_status;
 
 typedef struct c2b_ctx c2b_ctx;
@@ -68,6 +69,8 @@ uint64_t c2b_kernel_launches(void);
  *                                epilogue) instead of the count scan + k_sort_write; measured slower, kept for study
  *   stage_threads (4)            host threads staging a PAGEABLE input array through the pinned ring (0: leave
  *                                the pageable copy to the driver)
+ *   bal_chunk_bytes (2^25)       byte budget of one chunk of c2b_write_bal* (device buffer and pinned ring slot);
+ *                                at least 4096, rounded down to a multiple of 8
  * Unknown names are C2B_ERR_INVALID. */
 int c2b_tune(c2b_ctx *ctx, const char *name, double value);
 /* measurement aid (SURVEY 8d): sustained rate of independent f64 FMAs on this device, in DFMA/s
@@ -318,6 +321,35 @@ int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64
  * and after the host-buffer c2b_visibility_graph (which leaves only its last camera batch resident). */
 int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out);
 
+/* ---- BAL files (BAProblem::write, src/baproblem.rs:709-764) ----------------------------------------------------
+ * The file is encoded on the device and streamed to disk in chunks of at most bal_chunk_bytes: the D2H copy and
+ * the host write of one chunk overlap the encoding of the next, and the device and pinned memory of the encoder
+ * do not grow with the problem.  The bytes are the reference's:
+ *   C2B_BAL_TEXT    header "C P O", then "c p u v" per observation, the 9-vector (to_vec) of every camera and the
+ *                   3 coordinates of every point, one line each; every f64 as Rust's `{}` prints it: the shortest
+ *                   digits that round-trip, positional (1e21 -> 1000000000000000000000, 5e-324 -> 0.000...005),
+ *                   "NaN", "inf", "-inf", "-0"
+ *   C2B_BAL_BINARY  big-endian u64 C P O, per camera its observation count then (u64 point, f64 u, f64 v) records,
+ *                   the camera 9-vectors, the points
+ * The camera 9-vectors are computed on the host by c2b_camera_to_vec. */
+typedef enum { C2B_BAL_TEXT = 0, C2B_BAL_BINARY = 1 } c2b_bal_format;
+typedef struct {
+  uint64_t bytes;      /* size of the file written */
+  uint64_t chunks;
+  float ms_encode;     /* device time of the encoding kernels, summed over chunks (CUDA events) */
+  float ms_d2h;        /* device time of the chunk copies to pinned memory, summed */
+  float ms_write;      /* host wall time spent in write(2), summed */
+} c2b_bal_stats;
+/* host arrays in the layout of c2b_cull_problem (cams C x 15, pts P x 3, offsets C + 1, point_idx / uv
+ * offsets[C] entries); offsets[0] != 0, decreasing offsets and point_idx >= P are C2B_ERR_INVALID and no file
+ * is created.  Does not touch the ctx's resident problem.  out may be NULL. */
+int c2b_write_bal(c2b_ctx *ctx, const char *path, int format, const double *cams, uint64_t C, const double *pts,
+                  uint64_t P, const uint64_t *offsets, const uint32_t *point_idx, const double *uv,
+                  c2b_bal_stats *out);
+/* the resident problem (after c2b_visibility_graph_resident, and after a resident cull or noise pass); refuses
+ * in the cases c2b_cull_problem_resident refuses */
+int c2b_write_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_stats *out);
+
 /* ---- input generation on the GPU -------------------------------------------------------------------
  * replaces generate_world_points_uniform (src/generate.rs:356-420): num_points world points, each
  * on an area-weighted random triangle (all index triples of all models, concatenated), uniform
@@ -353,6 +385,9 @@ void c2b_camera_project(const double *cam, const double pc[3], double out[2]);
 void c2b_camera_from_position_direction(const double pos[3], const double R[9], double *cam_out);
 void c2b_camera_transform(const double *cam, const double dR[9], const double dloc[3],
                           double *cam_out);
+/* SnavelyCamera::to_vec (src/baproblem.rs:192-202): [rodrigues 3, translation 3, f, k1, k2], the same operations
+ * as include/city2ba.hpp's to_vec, bit for bit */
+void c2b_camera_to_vec(const double *cam, double out[9]);
 
 #ifdef __cplusplus
 }

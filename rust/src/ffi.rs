@@ -48,6 +48,15 @@ pub struct c2b_cull_stats {
     pub ms_h2d: c_float, pub ms_compute: c_float, pub ms_d2h: c_float,
 }
 
+// BAL files on the GPU (c2b_write_bal / c2b_write_bal_resident)
+pub const C2B_BAL_TEXT: c_int = 0;
+pub const C2B_BAL_BINARY: c_int = 1;
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct c2b_bal_stats {
+    pub bytes: u64, pub chunks: u64,
+    pub ms_encode: c_float, pub ms_d2h: c_float, pub ms_write: c_float,
+}
+
 // Embree's RTCRay layout (48 bytes): what embree_rs::Ray wraps (src/generate.rs:253-262, :457-464)
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct c2b_ray48 {
@@ -136,6 +145,12 @@ extern "C" {
                             offsets: *mut u64, point_idx: *mut u32, uv: *mut c_double,
                             out: *mut c2b_cull_stats) -> c_int;
     pub fn c2b_cull_problem_resident(ctx: *mut c2b_ctx, out: *mut c2b_cull_stats) -> c_int;
+    // ---- BAL files: a Rust BAProblem::write would call c2b_write_bal with the format of its extension ----
+    pub fn c2b_write_bal(ctx: *mut c2b_ctx, path: *const c_char, format: c_int, cams: *const c_double, c: u64,
+                         pts: *const c_double, p: u64, offsets: *const u64, point_idx: *const u32,
+                         uv: *const c_double, out: *mut c2b_bal_stats) -> c_int;
+    pub fn c2b_write_bal_resident(ctx: *mut c2b_ctx, path: *const c_char, format: c_int,
+                                  out: *mut c2b_bal_stats) -> c_int;
     // ---- input generation ----
     pub fn c2b_generate_world_points_uniform(ctx: *mut c2b_ctx, xyz: *const c_float, nv: u64, tri: *const u32,
                                              nt: u64, cams: *const c_double, c: u64, num_points: u64,
@@ -159,4 +174,5 @@ extern "C" {
     pub fn c2b_camera_from_position_direction(pos: *const c_double, r: *const c_double, cam_out: *mut c_double);
     pub fn c2b_camera_transform(cam: *const c_double, d_r: *const c_double, dloc: *const c_double,
                                 cam_out: *mut c_double);
+    pub fn c2b_camera_to_vec(cam: *const c_double, out: *mut c_double);
 }
