@@ -104,7 +104,6 @@ struct Tunables {
   int packet_bvh = 1;              // list overflow: 1 = lane = node packet traversal, 0 = per-ray stackless walk
   int trilist_warp = -1;           // leaf lists by one warp per camera (1) / one thread (0); -1 = by camera count
   int batches = 0;                 // camera batches of the host-buffer call; 0 = automatic
-  int fu_occ3 = 0;                 // fused kernel at 3 CTAs/SM (80 registers) instead of 4 (64)
   double grid_cell_factor = 0.25;  // point-grid cell side / max_dist
   int stage_threads = 4;           // host threads staging a pageable input through the pinned ring; 0 = let the
                                    // driver copy from pageable memory itself
@@ -112,11 +111,6 @@ struct Tunables {
                                    // through a pinned ring (0: pin the result arrays at once, as later calls do)
   int optimistic = 1;              // launch a pass's kernels without waiting for the plan's totals when the
                                    // previous pass on this ctx left sizes to go by (one host sync instead of three)
-  int epilogue = 0;                // 1: sort + CSR write inside the fused kernel instead of the count scan +
-                                   // k_sort_write.  Measured slower (cfg4: 4.04 ms against 2.69 + 0.80): at the
-                                   // same 32 warps per SM a warp's epilogue is just appended to its serial
-                                   // chain, and warps parked in its latency-bound loops leave fewer warps to
-                                   // fill the issue slots (64.6 % issue-active against 77 %; profiles/r02f)
   uint64_t bal_chunk_bytes = 1ull << 25;  // BAL writer: bytes per chunk (device buffer, pinned ring slot)
 };
 
@@ -324,10 +318,8 @@ static bool tune(Tunables &t, const char *name, double v) {
   else if (n == "packet_bvh") t.packet_bvh = v != 0;
   else if (n == "trilist_warp") t.trilist_warp = v < 0 ? -1 : (v != 0);
   else if (n == "batches") t.batches = std::max(0, (int)v);
-  else if (n == "fu_occ3") t.fu_occ3 = v != 0;
   else if (n == "grid_cell_factor") t.grid_cell_factor = v > 0 ? v : 0.25;
   else if (n == "stage_threads") t.stage_threads = std::min(std::max(0, (int)v), 16);
-  else if (n == "epilogue") t.epilogue = v != 0;
   else if (n == "optimistic") t.optimistic = v != 0;
   else if (n == "cold_staged") t.cold_staged = v != 0;
   else if (n == "bal_chunk_bytes") t.bal_chunk_bytes = (uint64_t)(v >= 4096.0 ? std::min(v, 1073741824.0) : 4096.0) & ~7ull;
@@ -410,8 +402,8 @@ int c2b_init(int device, c2b_ctx **out) {
     struct { const char *env, *name; } hooks[] = {
         {"C2B_PARTS_LOG2", "parts_log2"}, {"C2B_TRILIST_CAP", "trilist_cap"}, {"C2B_MAX_PAIRS", "max_pairs"},
         {"C2B_HOIST_MAX", "hoist_max"}, {"C2B_PACKET_BVH", "packet_bvh"}, {"C2B_TRILIST_WARP", "trilist_warp"},
-        {"C2B_BATCHES", "batches"}, {"C2B_FU_OCC3", "fu_occ3"}, {"C2B_GRID_CELL_FACTOR", "grid_cell_factor"},
-        {"C2B_STAGE_THREADS", "stage_threads"}, {"C2B_EPILOGUE", "epilogue"}, {"C2B_OPTIMISTIC", "optimistic"}, {"C2B_COLD_STAGED", "cold_staged"},
+        {"C2B_BATCHES", "batches"}, {"C2B_GRID_CELL_FACTOR", "grid_cell_factor"},
+        {"C2B_STAGE_THREADS", "stage_threads"}, {"C2B_OPTIMISTIC", "optimistic"}, {"C2B_COLD_STAGED", "cold_staged"},
         {"C2B_BAL_CHUNK_BYTES", "bal_chunk_bytes"}};
     for (auto &h : hooks)
       if (const char *e = getenv(h.env)) (void)tune(x->tun, h.name, atof(e));
@@ -447,7 +439,7 @@ void c2b_shutdown(c2b_ctx *ctx) {
                     &ctx->misc, &ctx->tri_list, &ctx->tri_count, &ctx->pts_aos, &ctx->ev_off,
                     &ctx->vis_count, &ctx->seg_off, &ctx->scratch_idx, &ctx->plan_rows, &ctx->plan_row_count,
                     &ctx->nz_cams, &ctx->nz_centers, &ctx->nz_pts, &ctx->nz_uv, &ctx->nz_scratch,
-                    &ctx->epi_status, &ctx->epi_prefix, &ctx->cams_all, &ctx->pr_parent, &ctx->pr_size,
+                    &ctx->cams_all, &ctx->pr_parent, &ctx->pr_size,
                     &ctx->pr_cam_cnt, &ctx->pr_pt_cnt, &ctx->pr_words, &ctx->pr_prefix, &ctx->pr_small};
   for (auto *b : bufs) b->release();
   for (int i = 0; i < 2; ++i)
@@ -1072,8 +1064,7 @@ int visibility_grid_fused(c2b_ctx *ctx, CtxExtra *x, const c2b_scene *scene, dou
   // launch everything back to back, and check at the one final sync that it all fitted.
   const uint64_t max_pairs = x->tun.max_pairs;  // 32-bit scratch offsets (lower: test hook)
   const bool mt = mesh && opt.predicate == C2B_PRED_MT;
-  const bool epi = x->tun.epilogue && parts_log2 == 0 && !opt.count_traversal && !mt && !(mesh && x->tun.fu_occ3);
-  const bool optimistic = x->tun.optimistic && x->memo.valid && !epi && !opt.count_traversal && ctx->scratch_idx.cap >= 4 &&
+  const bool optimistic = x->tun.optimistic && x->memo.valid && !opt.count_traversal && ctx->scratch_idx.cap >= 4 &&
                           ctx->out_idx[sel].cap >= 4 && ctx->out_uv[sel].cap >= 16;
   bool any_overflow = x->memo.any_overflow;
   if (!optimistic) {
@@ -1089,60 +1080,29 @@ int visibility_grid_fused(c2b_ctx *ctx, CtxExtra *x, const c2b_scene *scene, dou
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_CULL], st));
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_SORT], st));
 
-  // fused cull + occlusion (+ the in-kernel sort / CSR write: see epilogue_sort_write)
+  // fused cull + occlusion
   C2B_CUDA(cudaMemsetAsync(ctx->vis_count.p, 0, (slots + 1) * 4, st));
-  if (epi) {
-    // the visible count is at most the planned row points: output arrays of that size can never overflow
-    C2B_TRY(ctx->out_idx[sel].ensure(std::max<uint64_t>(pairs_eval, 1) * 4));
-    C2B_TRY(ctx->out_uv[sel].ensure(std::max<uint64_t>(pairs_eval, 1) * 16));
-    const uint64_t c_pad = (C + 127) & ~127ull;  // the scanner reads and writes whole 128-camera steps
-    C2B_TRY(ctx->epi_status.ensure(c_pad * 4));
-    C2B_TRY(ctx->epi_prefix.ensure(c_pad * 8));
-    C2B_CUDA(cudaMemsetAsync(ctx->epi_status.p, 0, c_pad * 4, st));
-    C2B_CUDA(cudaMemsetAsync(ctx->epi_prefix.p, 0, c_pad * 8, st));
-    fa.status = ctx->epi_status.as<uint32_t>();
-    fa.prefix = ctx->epi_prefix.as<unsigned long long>();
-    fa.p_aos = ctx->pts_aos.as<double>();
-    fa.out_offsets = ctx->out_offsets[sel].as<uint64_t>();
-    fa.out_idx = ctx->out_idx[sel].as<uint32_t>();
-    fa.out_uv = ctx->out_uv[sel].as<double2>();
-    fa.out_cap = std::min<uint64_t>(ctx->out_idx[sel].cap / 4, ctx->out_uv[sel].cap / 16);
-    fa.key_bits = std::max(pbits, 1);
-  }
   {
     // persistent warps draw cameras from a ticket; more CTAs than can be resident is harmless
     const unsigned nb = (unsigned)std::min<uint64_t>(blocks_for(slots, FU_WARPS), (uint64_t)ctx->sm_count * 8), nt = FU_WARPS * 32;
     const bool cnt = opt.count_traversal != 0;
     // The template's third argument counts CTAs of EIGHT warps per SM (fu_min_ctas translates for four-warp CTAs).
-    // Eight-warp CTAs, r01m kernels at cfg4: 4 CTAs/SM at 64 registers 2.68 ms; 3 at 80 (C2B_FU_OCC3) 2.69 ms; 5 at 48
-    // 2.74 ms.  Four-warp CTAs, r02y kernels: 7 CTAs/SM at 72 registers 2.31 ms against 2.38 ms for 4 x 8 warps at 64.
-    const bool occ4 = !x->tun.fu_occ3;
+    // Eight-warp CTAs, r01m kernels at cfg4: 4 CTAs/SM at 64 registers 2.68 ms; 3 at 80 2.69 ms; 5 at 48 2.74 ms.
+    // Four-warp CTAs, r02y kernels: 7 CTAs/SM at 72 registers 2.31 ms against 2.38 ms for 4 x 8 warps at 64.
     if (mt) {
       // candidates only; k_filter_candidates_mt decides occlusion below
       k_visibility_fused<FU_OCC_NONE, false, 3, false><<<nb, nt, 0, st>>>(fa);
     } else if (mesh) {
       if (cnt)
         k_visibility_fused<FU_OCC_MESH, true, 3, true><<<nb, nt, 0, st>>>(fa);
-      else if (any_overflow && epi)
-        k_visibility_fused<FU_OCC_MESH, false, 4, true, true><<<nb + 1, nt, 0, st>>>(fa);
       else if (any_overflow)
         k_visibility_fused<FU_OCC_MESH, false, 4, true><<<nb, nt, 0, st>>>(fa);
-      else if (epi)
-        k_visibility_fused<FU_OCC_MESH, false, 4, false, true><<<nb + 1, nt, 0, st>>>(fa);
-      else if (occ4)
+      else
         k_visibility_fused<FU_OCC_MESH, false, 4, false><<<nb, nt, 0, st>>>(fa);
-      else
-        k_visibility_fused<FU_OCC_MESH, false, 3, false><<<nb, nt, 0, st>>>(fa);
     } else if (opt.occlusion == C2B_OCC_ANALYTIC) {
-      if (epi)
-        k_visibility_fused<FU_OCC_ANALYTIC, false, 2, false, true><<<nb + 1, nt, 0, st>>>(fa);
-      else
-        k_visibility_fused<FU_OCC_ANALYTIC, false, 2, false><<<nb, nt, 0, st>>>(fa);
+      k_visibility_fused<FU_OCC_ANALYTIC, false, 2, false><<<nb, nt, 0, st>>>(fa);
     } else {
-      if (epi)
-        k_visibility_fused<FU_OCC_NONE, false, 3, false, true><<<nb + 1, nt, 0, st>>>(fa);
-      else
-        k_visibility_fused<FU_OCC_NONE, false, 3, false><<<nb, nt, 0, st>>>(fa);
+      k_visibility_fused<FU_OCC_NONE, false, 3, false><<<nb, nt, 0, st>>>(fa);
     }
     C2B_KERNEL_CHECK();
     if (mt) {
@@ -1154,20 +1114,6 @@ int visibility_grid_fused(c2b_ctx *ctx, CtxExtra *x, const c2b_scene *scene, dou
   }
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_TRAVERSE], st));
 
-  bool epi_done = false;
-  if (epi) {
-    // the kernel has written the CSR; the counters say whether every camera took part
-    C2B_TRY(read_counters(ctx, h_cnt));
-    if (h_cnt[5]) return set_error(C2B_ERR_CUDA, "internal: a camera's scratch slice overflowed");
-    if (h_cnt[11]) return set_error(C2B_ERR_CUDA, "internal: the fused kernel's epilogue gave up waiting for a camera's count");
-    n_cand = h_cnt[4];
-    if (h_cnt[9] <= SW_WARP_MAX && h_cnt[10] == 0) {
-      total_obs = h_cnt[8];
-      epi_done = true;
-    }
-    // else: a camera sees more points than the warp sort holds — the two-kernel path below redoes the tail
-  }
-  if (!epi_done) {
   // visible counts -> CSR offsets
   C2B_TRY(exclusive_scan_u32(st, fa.vis_count, ctx->seg_off.as<uint32_t>(), slots + 1, d_total, ctx->scan_tmp));
   k_max_cam<<<(unsigned)std::min<uint64_t>(blocks_for(C, 256), 1024), 256, 0, st>>>(ctx->seg_off.as<uint32_t>(), C, parts_log2, d_max);
@@ -1217,50 +1163,49 @@ int visibility_grid_fused(c2b_ctx *ctx, CtxExtra *x, const c2b_scene *scene, dou
     x->memo.any_overflow = h_cnt[0] != 0;
     x->memo.big = max32 > SW_WARP_MAX;
   } else {
-  C2B_TRY(read_totals());
-  x->memo.valid = true;
-  x->memo.any_overflow = any_overflow;
-  x->memo.big = max32 > SW_WARP_MAX;
-  if (total_obs) {
-    C2B_TRY(ctx->out_idx[sel].ensure(total_obs * 4));
-    C2B_TRY(ctx->out_uv[sel].ensure(total_obs * 16));
-    const SortWriteArgs sw = sort_write_args();
-    if (max32 <= SW_BLOCK_MAX) {
-      // registers capped for 8 CTAs/SM (measured at cfg4: 0.81 ms; 6 CTAs/SM 0.91 ms, 4 CTAs/SM 1.12 ms)
-      if (parts_log2 > 0)
-        k_sort_write<6, true><<<swb, swt, 0, st>>>(sw);
-      else
-        k_sort_write<8, false><<<swb, swt, 0, st>>>(sw);
-      C2B_KERNEL_CHECK();
-      if (max32 > SW_WARP_MAX) {
-        k_sort_write_block<<<(unsigned)C, 256, 0, st>>>(sw);
+    C2B_TRY(read_totals());
+    x->memo.valid = true;
+    x->memo.any_overflow = any_overflow;
+    x->memo.big = max32 > SW_WARP_MAX;
+    if (total_obs) {
+      C2B_TRY(ctx->out_idx[sel].ensure(total_obs * 4));
+      C2B_TRY(ctx->out_uv[sel].ensure(total_obs * 16));
+      const SortWriteArgs sw = sort_write_args();
+      if (max32 <= SW_BLOCK_MAX) {
+        // registers capped for 8 CTAs/SM (measured at cfg4: 0.81 ms; 6 CTAs/SM 0.91 ms, 4 CTAs/SM 1.12 ms)
+        if (parts_log2 > 0)
+          k_sort_write<6, true><<<swb, swt, 0, st>>>(sw);
+        else
+          k_sort_write<8, false><<<swb, swt, 0, st>>>(sw);
+        C2B_KERNEL_CHECK();
+        if (max32 > SW_WARP_MAX) {
+          k_sort_write_block<<<(unsigned)C, 256, 0, st>>>(sw);
+          C2B_KERNEL_CHECK();
+        }
+      } else {
+        // a camera sees more points than the shared-memory sort holds: radix-sort all visible keys
+        C2B_TRY(ctx->sort_keys[0].ensure(total_obs * 8));
+        C2B_TRY(ctx->sort_keys[1].ensure(total_obs * 8));
+        C2B_TRY(ctx->sort_vals[0].ensure(total_obs * 4));
+        C2B_TRY(ctx->sort_vals[1].ensure(total_obs * 4));
+        k_expand_keys<<<blocks_for(C, 8), 256, 0, st>>>(sw, pbits, ctx->sort_keys[0].as<uint64_t>());
+        C2B_KERNEL_CHECK();
+        uint64_t *keys[2] = {ctx->sort_keys[0].as<uint64_t>(), ctx->sort_keys[1].as<uint64_t>()};
+        uint32_t *vals[2] = {ctx->sort_vals[0].as<uint32_t>(), ctx->sort_vals[1].as<uint32_t>()};
+        int res = 0;
+        C2B_TRY(radix_sort_pairs(st, keys, vals, total_obs, pbits + cbits, ctx->sort_hist, ctx->scan_tmp, &res));
+        k_write_sorted<<<blocks_for(total_obs, 256), 256, 0, st>>>(
+            keys[res], total_obs, pbits, fa.cams, ctx->pts_aos.as<double>(), ctx->out_idx[sel].as<uint32_t>(),
+            ctx->out_uv[sel].as<double2>());
+        C2B_KERNEL_CHECK();
+        k_widen_cam_offsets<<<blocks_for(C + 1, 256), 256, 0, st>>>(ctx->seg_off.as<uint32_t>(), C + 1, parts_log2,
+                                                                   ctx->out_offsets[sel].as<uint64_t>());
         C2B_KERNEL_CHECK();
       }
     } else {
-      // a camera sees more points than the shared-memory sort holds: radix-sort all visible keys
-      C2B_TRY(ctx->sort_keys[0].ensure(total_obs * 8));
-      C2B_TRY(ctx->sort_keys[1].ensure(total_obs * 8));
-      C2B_TRY(ctx->sort_vals[0].ensure(total_obs * 4));
-      C2B_TRY(ctx->sort_vals[1].ensure(total_obs * 4));
-      k_expand_keys<<<blocks_for(C, 8), 256, 0, st>>>(sw, pbits, ctx->sort_keys[0].as<uint64_t>());
-      C2B_KERNEL_CHECK();
-      uint64_t *keys[2] = {ctx->sort_keys[0].as<uint64_t>(), ctx->sort_keys[1].as<uint64_t>()};
-      uint32_t *vals[2] = {ctx->sort_vals[0].as<uint32_t>(), ctx->sort_vals[1].as<uint32_t>()};
-      int res = 0;
-      C2B_TRY(radix_sort_pairs(st, keys, vals, total_obs, pbits + cbits, ctx->sort_hist, ctx->scan_tmp, &res));
-      k_write_sorted<<<blocks_for(total_obs, 256), 256, 0, st>>>(keys[res], total_obs, pbits, fa.cams,
-                                                                ctx->pts_aos.as<double>(), ctx->out_idx[sel].as<uint32_t>(),
-                                                                ctx->out_uv[sel].as<double2>());
-      C2B_KERNEL_CHECK();
-      k_widen_cam_offsets<<<blocks_for(C + 1, 256), 256, 0, st>>>(ctx->seg_off.as<uint32_t>(), C + 1, parts_log2,
-                                                                 ctx->out_offsets[sel].as<uint64_t>());
-      C2B_KERNEL_CHECK();
+      C2B_CUDA(cudaMemsetAsync(ctx->out_offsets[sel].p, 0, (C + 1) * 8, st));
     }
-  } else {
-    C2B_CUDA(cudaMemsetAsync(ctx->out_offsets[sel].p, 0, (C + 1) * 8, st));
   }
-  }  // !optimistic
-  }  // !epi_done
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_COMPACT], st));
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_D2H], st));
   C2B_CUDA(cudaStreamSynchronize(st));

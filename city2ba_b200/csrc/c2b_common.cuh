@@ -221,7 +221,6 @@ struct c2b_ctx {
   c2b::DevBuf tri_list, tri_count;  // per-camera leaf lists for list-driven traversal
   // fused grid schedule: per-camera plan (row points -> scratch slice), visible counts, CSR offsets
   c2b::DevBuf ev_off, vis_count, seg_off, scratch_idx, plan_rows, plan_row_count;
-  c2b::DevBuf epi_status, epi_prefix;  // in-kernel epilogue: per-camera count flags and CSR offsets
   int numa_node = -1;  // of the device, from sysfs (-1: unknown)
 
   // noise passes on host arrays: grow-only device copies kept between calls

@@ -68,27 +68,11 @@ struct FusedArgs {
   uint32_t *vis_count;        // [slots+1]
   unsigned long long *counters;  // [1] pairs evaluated, [2] list entries / nodes, [3] warp triangle tests,
                                  // [4] candidates (rays), [5] scratch slice overflow flag, [7] camera ticket,
-                                 // EPI: [8] total observations, [9] largest per-camera count, [10] flags;
+                                 // [8]-[11] unused;
                                  // [12] optimistic-launch flags (FU_FLAG_*): the host sized a buffer or chose a
                                  // kernel variant from the previous pass and this pass does not fit
-  // ---- in-kernel epilogue (template EPI, parts_log2 == 0): a camera's visible list is sorted and its CSR
-  // records are written by the warp that produced it, one camera later (see k_visibility_fused) ----
-  uint32_t *status;            // [C] EPI_READY | visible count, published after the camera's fused phase
-  unsigned long long *prefix;  // [C] EPI_FLAG | exclusive prefix of the counts = CSR offset, by the scanner warp
-  const double *p_aos;         // xyz records, original point order
-  uint64_t *out_offsets;       // [C + 1]
-  uint32_t *out_idx;
-  double2 *out_uv;
-  uint64_t out_cap;            // observations the output arrays hold
-  int key_bits;                // bits of the largest point index
 };
 enum { FU_FLAG_SCRATCH = 1, FU_FLAG_NEED_WALK = 2, FU_FLAG_OUT = 4 };
-constexpr uint32_t EPI_READY = 0x80000000u;
-constexpr unsigned long long EPI_FLAG = 1ull << 63;
-enum { EPI_OUT_OVERFLOW = 1, EPI_TIMED_OUT = 2 };
-// A wait that does not end within ~2 s (it cannot, short of a bug or a fault on another warp) gives up and
-// raises counters[11]; every other wait sees that and gives up too, so the launch ends and the host reports it.
-constexpr unsigned EPI_SPIN_LIMIT = 8u << 20;
 
 // camera_cell_range / camera_row run in BOTH k_cam_plan (which sizes each camera's scratch slice) and
 // k_visibility_fused (which scans the rows), so they must round identically in both inlined copies:
@@ -330,8 +314,7 @@ __global__ void __launch_bounds__(128, 5) k_cam_plan(FusedArgs a) {
   if ((threadIdx.x & 31) == 0 && n) atomicAdd(&a.counters[1], n);
 }
 
-// ---- warp-private radix sort of a camera's visible point indices (used by k_sort_write and by the
-// fused kernel's in-kernel epilogue) --------------------------------------------------------------------
+// ---- warp-private radix sort of a camera's visible point indices (k_sort_write) -----------------------
 struct SortWriteArgs {
   const uint32_t *ev_off;     // [C+1] scratch slice starts
   const uint32_t *seg_off;    // [C+1] exclusive scan of vis_count = CSR offsets
@@ -510,75 +493,6 @@ __device__ __forceinline__ void sort_warp_to_smem(const SortWriteArgs &s, const 
       if (t < n) sorted[sw_pad(t)] = a[r];
     }
   }
-}
-
-
-// Warp-private LSD radix sort of a camera's n <= SW_WARP_MAX visible indices, 8-bit digits, as ROLLED loops over
-// 32-key chunks that ping-pong between the camera's scratch slice (global, L2-resident) and a shared-memory
-// buffer.  Returns where the sorted keys ended up (the slice or `buf`).  About 30 registers and ~1.4 k SASS
-// lines; sort_warp_to_smem keeps the keys in up to 32 unrolled registers instead (64 registers, five
-// instantiations) and is the faster of the two as a kernel of its own: k_sort_write with this sort at 11 CTAs
-// per SM measured 1.35 ms against 0.82 ms at cfg4 (the ping-pong's global round trips cost more than the extra
-// warps hide; r02n) — so it serves the in-kernel epilogue only, where code size decides.
-__device__ __forceinline__ const uint32_t *rolled_warp_sort(uint32_t *slice, uint32_t n, int key_bits, uint32_t *buf,
-                                                            uint32_t *hist, int lane) {
-  const uint32_t *src = slice;
-  uint32_t *dst = buf;
-  const unsigned lt = (1u << lane) - 1u;
-#pragma unroll 1
-  for (int shift = 0; shift < key_bits; shift += SW_RADIX_BITS) {
-#pragma unroll
-    for (int k = 0; k < SW_BINS / 32; ++k) hist[k * 32 + lane] = 0u;
-    __syncwarp();
-#pragma unroll 1
-    for (uint32_t t = lane; t < n; t += 32) atomicAdd(&hist[(src[t] >> shift) & (SW_BINS - 1)], 1u);
-    __syncwarp();
-    uint32_t cnt[SW_BINS / 32];
-    uint32_t sum = 0;
-    bool one_bin = false;
-#pragma unroll
-    for (int k = 0; k < SW_BINS / 32; ++k) {
-      cnt[k] = hist[lane * (SW_BINS / 32) + k];
-      one_bin |= cnt[k] == n;
-      sum += cnt[k];
-    }
-    if (__any_sync(0xffffffffu, one_bin)) {  // every key has the same digit: order unchanged
-      __syncwarp();
-      continue;
-    }
-    uint32_t pre = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, pre, o);
-      if (lane >= o) pre += v;
-    }
-    pre -= sum;
-    __syncwarp();
-#pragma unroll
-    for (int k = 0; k < SW_BINS / 32; ++k) {
-      hist[lane * (SW_BINS / 32) + k] = pre;
-      pre += cnt[k];
-    }
-    __syncwarp();
-#pragma unroll 1
-    for (uint32_t first = 0; first < n; first += 32) {
-      const uint32_t t = first + lane;
-      const bool valid = t < n;
-      const uint32_t key = valid ? src[t] : 0u;
-      const uint32_t d = valid ? (key >> shift) & (SW_BINS - 1) : (uint32_t)SW_BINS;  // padding keeps to itself
-      const unsigned peers = __match_any_sync(0xffffffffu, d);
-      const int leader = __ffs(peers) - 1;
-      uint32_t old = 0;
-      if (valid && lane == leader) old = atomicAdd(&hist[d], (uint32_t)__popc(peers));  // warp-aggregated
-      const uint32_t pos = __shfl_sync(0xffffffffu, old, leader) + __popc(peers & lt);
-      if (valid) dst[pos] = key;
-    }
-    __syncwarp();
-    const uint32_t *filled = dst;
-    dst = dst == buf ? slice : buf;
-    src = filled;
-  }
-  return src;
 }
 
 // ---- the fused pass ---------------------------------------------------------------------------------
@@ -918,176 +832,37 @@ __device__ __forceinline__ int packet_bvh_hit(const FusedArgs &a, const Ray &ray
   return alive && !((am >> lane) & 1u) ? 1 : 0;
 }
 
-// ---- in-kernel epilogue -----------------------------------------------------------------------------
-// Sorting a camera's visible indices and writing its CSR records needs the camera's offset in the CSR = the
-// sum of the visible counts of ALL cameras before it.  Instead of ending the kernel there (count scan on the
-// host's clock, then a second kernel that re-reads the scratch lists: 0.79 ms of the 3.6 ms pass at cfg4,
-// latency-bound at 52 % issue-active) the persistent kernel finishes the job itself:
-//   * a worker warp publishes status[cam] = READY | count when its camera's fused phase ends;
-//   * ONE scanner warp (block 0, warp 0; it takes no tickets) walks the cameras in order, 32 per step, waits
-//     for their counts, and publishes prefix[cam] (and the CSR offsets, the total and the largest count);
-//   * a worker handles the epilogue of a camera only AFTER the fused phase of its NEXT camera (tickets are
-//     handed out in camera order, so by then every earlier camera has long been counted and the wait for
-//     prefix[cam] is over before it starts): sort (the same warp-private radix sort as k_sort_write, in the
-//     warp's shared-memory region), gather the points, recompute (u, v) bit-identically, write coalesced.
-// The epilogue's loads and shared-memory round trips interleave with other warps' fused phases, which is what
-// hides its latency.  Deadlock-free: publishing a count never waits, the scanner only waits for counts, and
-// every ticket holder is resident (block 0 is dispatched first).  Cameras that see more than SW_WARP_MAX points
-// or an output array that is too small are left to the host's fallback (the two-kernel path).
-__device__ __noinline__ void epilogue_sort_write(const FusedArgs &a, uint64_t cam, uint32_t n, uint32_t ev0,
-                                                 const double *c, uint32_t *region, int lane) {
-  n = __reduce_max_sync(0xffffffffu, n);  // uniform register (see k_sort_write)
-  if (n == 0u || n > SW_WARP_MAX) return;
-  unsigned long long w = 0ull;
-  if (lane == 0) {
-    const volatile unsigned long long *p = a.prefix + cam;
-    const volatile unsigned long long *abort_flag = a.counters + 11;
-    unsigned spins = 0;
-    while (!((w = *p) & EPI_FLAG)) {
-      __nanosleep(200);
-      if ((++spins & 1023u) == 0u && (*abort_flag || spins > EPI_SPIN_LIMIT)) {
-        atomicOr(&a.counters[11], 1ull);
-        break;
-      }
-    }
-  }
-  w = __shfl_sync(0xffffffffu, w, 0);
-  if (!(w & EPI_FLAG)) return;  // gave up: the host reports the failure
-  const uint64_t base = w & ~EPI_FLAG;
-  if (base + n > a.out_cap) {
-    if (lane == 0) atomicOr(&a.counters[10], (unsigned long long)EPI_OUT_OVERFLOW);
-    return;
-  }
-  // the rolled sort: the register version's five instantiations tripled this kernel's code (14.0 k SASS lines
-  // against 4.7 k) and the instruction cache thrashed — 8 of 16 stall cycles no_instruction, 6.0 ms against
-  // 2.7 + 0.8 (profiles/r02e)
-  const uint32_t *src = rolled_warp_sort(a.scratch_idx + ev0, n, a.key_bits, region, region + SW_WARP_MAX, lane);
-#pragma unroll 2
-  for (uint32_t i = lane; i < n; i += 32) {
-    const uint32_t pt = src[i];
-    const double *p = a.p_aos + 3 * (uint64_t)pt;
-    a.out_idx[base + i] = pt;
-    a.out_uv[base + i] = observe(c, p[0], p[1], p[2]);
-  }
-  __syncwarp();
-}
-
-__device__ __noinline__ void epilogue_scanner(const FusedArgs &a, int lane) {
-  const volatile unsigned long long *abort_flag = a.counters + 11;
-  unsigned long long running = 0ull;
-  uint32_t mx = 0u;
-  const uint64_t C = a.C;
-  // status[] and prefix[] are allocated in multiples of 128 entries, so the vector accesses stay in bounds;
-  // entries at or beyond C are never published and are treated as ready zeros
-  auto load4 = [&](uint64_t first) {
-    uint4 v;
-    asm volatile("ld.volatile.global.v4.u32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-                 : "l"(a.status + first)
-                 : "memory");
-    if (first + 0 >= C) v.x = EPI_READY;
-    if (first + 1 >= C) v.y = EPI_READY;
-    if (first + 2 >= C) v.z = EPI_READY;
-    if (first + 3 >= C) v.w = EPI_READY;
-    return v;
-  };
-  uint4 nxt = load4((uint64_t)lane * 4);
-  for (uint64_t base = 0; base < C; base += 128) {
-    const uint64_t first = base + (uint64_t)lane * 4;
-    uint4 cur = nxt;
-    if (base + 128 < C) nxt = load4(first + 128);  // in flight during this step
-    unsigned spins = 0;
-    bool gave_up = false;
-    while (!(cur.x & cur.y & cur.z & cur.w & EPI_READY)) {
-      __nanosleep(64);
-      cur = load4(first);
-      if ((++spins & 1023u) == 0u && (*abort_flag || spins > 2 * EPI_SPIN_LIMIT)) {
-        atomicOr(&a.counters[11], 1ull);
-        gave_up = true;
-        break;
-      }
-    }
-    if (__any_sync(0xffffffffu, gave_up)) return;
-    const uint32_t n0 = cur.x & ~EPI_READY, n1 = cur.y & ~EPI_READY, n2 = cur.z & ~EPI_READY, n3 = cur.w & ~EPI_READY;
-    const uint32_t mine = n0 + n1 + n2 + n3;
-    uint32_t incl = mine;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    const unsigned long long e0 = running + (unsigned long long)(incl - mine);
-    const unsigned long long e1 = e0 + n0, e2 = e1 + n1, e3 = e2 + n2;
-    if (first < C) {
-      // out_offsets has room for the closing entry only: vector stores while all four are real cameras
-      if (first + 3 < C) {
-        *reinterpret_cast<ulonglong2 *>(a.out_offsets + first) = make_ulonglong2(e0, e1);
-        *reinterpret_cast<ulonglong2 *>(a.out_offsets + first + 2) = make_ulonglong2(e2, e3);
-      } else {
-        a.out_offsets[first] = e0;
-        if (first + 1 < C) a.out_offsets[first + 1] = e1;
-        if (first + 2 < C) a.out_offsets[first + 2] = e2;
-      }
-      volatile ulonglong2 *pf = reinterpret_cast<volatile ulonglong2 *>(a.prefix + first);
-      pf[0].x = e0 | EPI_FLAG;
-      pf[0].y = e1 | EPI_FLAG;
-      pf[1].x = e2 | EPI_FLAG;
-      pf[1].y = e3 | EPI_FLAG;
-    }
-    running += (unsigned long long)__shfl_sync(0xffffffffu, incl, 31);
-    mx = max(max(mx, max(n0, n1)), max(n2, n3));
-  }
-  mx = __reduce_max_sync(0xffffffffu, mx);
-  if (lane == 0) {
-    a.out_offsets[a.C] = running;
-    a.counters[8] = running;
-    a.counters[9] = mx;
-  }
-}
-
 // Persistent warps: every warp draws the next camera from a global ticket (counters[7]), so a warp
 // that drew a cheap camera (city edge, few points in range) immediately gets another one and no
 // warp idles waiting for the slowest camera of its block.
 // WALK = the BVH traversals for cameras whose leaf list overflowed are compiled in; the host picks
 // the variant without them when k_cam_trilist reported no overflow (coarse meshes), which keeps
 // their registers out of the list-driven fast path.
-// EPI = the in-kernel epilogue above (parts_log2 must be 0): two camera-record slots per warp (the pending
-// camera's record stays put while the next camera is scanned) and a per-warp region large enough for the sort.
-constexpr int FU_REGION_F4 = 4 * FU_HOIST;                                                   // 4 KB
-constexpr int FU_REGION_EPI_F4 = ((SW_WARP_MAX + SW_BINS) * 4 + 15) / 16;                     // 5 KB
-static_assert(FU_REGION_EPI_F4 >= FU_REGION_F4, "the sort region also holds the triangle records");
+constexpr int FU_REGION_F4 = 4 * FU_HOIST;  // 4 KB
 
-// a warp's shared memory: triangle records (hoisted: 4 planes x FU_HOIST; chunked: 32 x 3; EPI: also the sort's
-// keys and counters), the camera record(s), and the ring of FU_STAGE grid positions in which the survivors of the
-// cull wait for their packet.  (Staging the coordinates as well, so that the ray set-up needs no second trip
-// through L1, was measured: 48 KB of shared memory per CTA instead of 36 shrink L1, 3.11 ms against 3.07 ms at cfg4.)
-template <bool EPI, bool MESH>
+// a warp's shared memory: triangle records (hoisted: 4 planes x FU_HOIST; chunked: 32 x 3), the camera record,
+// and the ring of FU_STAGE grid positions in which the survivors of the cull wait for their packet.  (Staging the
+// coordinates as well, so that the ray set-up needs no second trip through L1, was measured: 48 KB of shared
+// memory per CTA instead of 36 shrink L1, 3.11 ms against 3.07 ms at cfg4.)
+template <bool MESH>
 struct alignas(16) FuWarpSmem {
-  float4 rec[EPI ? FU_REGION_EPI_F4 : MESH ? FU_REGION_F4 : 1];
-  double cam[EPI ? 2 : 1][16];
+  float4 rec[MESH ? FU_REGION_F4 : 1];
+  double cam[16];
   uint32_t stage[FU_STAGE];
 };
 
-template <int OCC, bool COUNT, int MIN_CTAS, bool WALK, bool EPI = false>
+template <int OCC, bool COUNT, int MIN_CTAS, bool WALK>
 __global__ void __launch_bounds__(FU_WARPS * 32, fu_min_ctas(MIN_CTAS)) k_visibility_fused(FusedArgs a) {
   // One block of shared memory per warp (FuWarpSmem), addressed through ONE opaque 32-bit register: with three
   // separate arrays indexed by the warp number the compiler re-derived every address from %tid and the shared
   // window at each use (5-10 instructions, eight times per chunk / packet: profiles/r02w_sass_dynamic_fused.txt).
-  typedef FuWarpSmem<EPI, OCC == FU_OCC_MESH> WarpSmem;
+  typedef FuWarpSmem<OCC == FU_OCC_MESH> WarpSmem;
   __shared__ WarpSmem s_w[FU_WARPS];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (EPI && blockIdx.x == 0 && warp == 0) {
-    epilogue_scanner(a, lane);
-    return;
-  }
   uint32_t w_s = (uint32_t)__cvta_generic_to_shared(&s_w[warp]);
   asm volatile("" : "+r"(w_s));
   WarpSmem *const w = reinterpret_cast<WarpSmem *>(__cvta_shared_to_generic((size_t)w_s));
-  int cur = 0;  // EPI: the record slot of the camera being scanned
-  double *c = w->cam[0];
-  bool pending = false;  // EPI: a finished camera waits for its epilogue
-  uint64_t pend_cam = 0;
-  uint32_t pend_n = 0, pend_ev0 = 0;
+  double *const c = w->cam;
   uint32_t *stage = w->stage;
   unsigned long long found_total = 0;
   unsigned n_vis_nodes = 0, n_tri = 0;
@@ -1117,7 +892,6 @@ __global__ void __launch_bounds__(FU_WARPS * 32, fu_min_ctas(MIN_CTAS)) k_visibi
       if ((uint32_t)lane < a.tri_cap) l0 = mylist[lane];
       if ((uint32_t)lane + 32u < a.tri_cap) l1 = mylist[lane + 32];
     }
-    if (EPI) c = w->cam[cur];
     if (lane < 15) c[lane] = creg;
     __syncwarp();
     // launched without waiting for the plan's totals (sizes and variant from the previous pass): a camera
@@ -1127,10 +901,7 @@ __global__ void __launch_bounds__(FU_WARPS * 32, fu_min_ctas(MIN_CTAS)) k_visibi
     if (misfit && lane == 0)
       atomicOr(&a.counters[12], (unsigned long long)((uint64_t)ev1 > a.scratch_cap ? FU_FLAG_SCRATCH : FU_FLAG_NEED_WALK));
     if (planned_rows == 0u || misfit) {  // nothing to scan (ball outside the data, NaN centre, ...)
-      if (lane == 0) {
-        a.vis_count[slot] = 0;
-        if (EPI) *(volatile uint32_t *)(a.status + cam) = EPI_READY;
-      }
+      if (lane == 0) a.vis_count[slot] = 0;
       continue;
     }
     const float ox = d2f(cen.x), oy = d2f(cen.y), oz = d2f(cen.z);
@@ -1255,23 +1026,8 @@ __global__ void __launch_bounds__(FU_WARPS * 32, fu_min_ctas(MIN_CTAS)) k_visibi
       found_total += qn;
     }
     nvis = nvis < out_cap ? nvis : out_cap;
-    if (lane == 0) {
-      a.vis_count[slot] = nvis;
-      if (EPI) *(volatile uint32_t *)(a.status + cam) = EPI_READY | nvis;
-    }
-    if (EPI) {
-      __syncwarp();
-      if (pending)
-        epilogue_sort_write(a, pend_cam, pend_n, pend_ev0, w->cam[cur ^ 1], reinterpret_cast<uint32_t *>(w->rec), lane);
-      pending = true;
-      pend_cam = cam;
-      pend_n = nvis;
-      pend_ev0 = ev0;
-      cur ^= 1;
-    }
+    if (lane == 0) a.vis_count[slot] = nvis;
   }
-  if (EPI && pending)
-    epilogue_sort_write(a, pend_cam, pend_n, pend_ev0, w->cam[cur ^ 1], reinterpret_cast<uint32_t *>(w->rec), lane);
   if (lane == 0) {
     if (found_total) atomicAdd(&a.counters[4], found_total);
     if (COUNT) {

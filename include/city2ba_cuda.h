@@ -60,13 +60,10 @@ uint64_t c2b_kernel_launches(void);
  *   packet_bvh (1)               list overflow: 1 lane = node packet traversal, 0 per-ray stackless walk
  *   trilist_warp (-1 auto|0|1)   leaf lists built by one warp / one thread per camera
  *   batches (0 auto)             camera batches of the host-buffer call
- *   fu_occ3 (0)                  fused kernel at 3 CTAs/SM
  *   grid_cell_factor (0.25)      point-grid cell side / max_dist
  *   optimistic (1)               later passes on a ctx launch their kernels without waiting for the plan's totals
  *                                (sizes and kernel variant from the previous pass, checked by the kernels)
  *   cold_staged (1)              first host-buffer call on a ctx: CSR in unpinned memory through a pinned ring
- *   epilogue (0)                 1: sort + CSR write inside the fused kernel (scanner warp + deferred per-camera
- *                                epilogue) instead of the count scan + k_sort_write; measured slower, kept for study
  *   stage_threads (4)            host threads staging a PAGEABLE input array through the pinned ring (0: leave
  *                                the pageable copy to the driver)
  *   bal_chunk_bytes (2^25)       byte budget of one chunk of c2b_write_bal* (device buffer and pinned ring slot);

@@ -13,7 +13,7 @@ import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SO = os.path.join(ROOT, "city2ba_b200", "libcity2ba_cuda.so")
-KERNEL = sys.argv[1] if len(sys.argv) > 1 else "k_visibility_fusedILi0ELb0ELi4ELb0ELb0"   # <MESH, no count, 4 CTAs, no walk, no epilogue>
+KERNEL = sys.argv[1] if len(sys.argv) > 1 else "k_visibility_fusedILi0ELb0ELi4ELb0E"   # <MESH, no count, 4 CTAs, no walk>
 
 
 def functions_of(path):

@@ -351,8 +351,9 @@ def test_list_modes_agree(c2b, ctx, orc, cfg2):
         assert_same_graph(c2b.visibility_graph(scene, cams, pts, 10.0, ctx=ctx), ref, "packet bvh")
         ctx.tune("packet_bvh", 0)
         assert_same_graph(c2b.visibility_graph(scene, cams, pts, 10.0, ctx=ctx), ref, "per-ray walk")
-        with pytest.raises(c2b.C2BError, match="unknown hook"):
-            ctx.tune("no_such_hook", 1)
+        for name in ("no_such_hook", "epilogue", "fu_occ3"):
+            with pytest.raises(c2b.C2BError, match="unknown hook"):
+                ctx.tune(name, 1)
     finally:
         ctx.tune("reset", 0)
 
@@ -612,32 +613,6 @@ def test_predicate_mt_matches_oracle_mt(c2b, ctx, orc, cfg2, mode):
         assert_same_graph(w, v, f"{name}/{mode} watertight default")
         differs += int(w.num_observations != g.num_observations)
     assert differs > 0   # the two predicates do not decide every end-point ray alike (DESIGN.md section 2)
-
-
-@pytest.mark.parametrize("occlusion", ["mesh", "analytic", "none"])
-def test_in_kernel_epilogue_gives_the_same_graph(c2b, ctx, orc, cfg2, occlusion, request):
-    """hook epilogue = 1: the fused kernel sorts every camera's list and writes its CSR records itself (a
-    scanner warp publishes the count prefix, the epilogue is deferred by one camera) — same graph as the
-    default count scan + k_sort_write path, at cfg2 and on a denser problem with cameras above 1,024 points
-    (which fall back to the two-kernel tail)"""
-    request.addfinalizer(lambda: ctx.tune("reset", 0))
-    cams, pts, xyz, tri = cfg2
-    scene = c2b.Scene(xyz, tri, ctx=ctx) if occlusion == "mesh" else None
-    want = c2b.visibility_graph(scene, cams, pts, 10.0, occlusion=occlusion, ctx=ctx)
-    dense_pts = orc.grid_points(300, 2)
-    dense_cams = orc.grid_cameras(4, 2)
-    dscene = c2b.Scene(*orc.city_mesh(2), ctx=ctx) if occlusion == "mesh" else None
-    want_dense = c2b.visibility_graph(dscene, dense_cams, dense_pts, 30.0, occlusion=occlusion, ctx=ctx)
-    ctx.tune("epilogue", 1)
-    got = c2b.visibility_graph(scene, cams, pts, 10.0, occlusion=occlusion, ctx=ctx)
-    got_dense = c2b.visibility_graph(dscene, dense_cams, dense_pts, 30.0, occlusion=occlusion, ctx=ctx)
-    for g, w in ((got, want), (got_dense, want_dense)):
-        assert np.array_equal(g.offsets, w.offsets) and np.array_equal(g.point_idx, w.point_idx)
-        assert np.array_equal(g.uv, w.uv)
-    if occlusion == "none":
-        assert want_dense.counts().max() > 1024     # the large-camera fallback ran
-    if occlusion == "mesh":
-        assert_same_graph(got, orc.visibility_graph(xyz, tri, cams, pts, 10.0), "epilogue")
 
 
 def test_first_call_on_a_fresh_ctx_returns_the_same_graph(c2b, orc, cfg2):
