@@ -103,9 +103,23 @@ class BalStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class BalReadStats(C.Structure):
+    """c2b_bal_read_stats: sizes, bytes and chunks read, tokens converted on the host, whether the observations were
+    regrouped by camera, host ms in pread(2), device ms of the chunk copies and of the parse kernels"""
+    _fields_ = [
+        ("n_cameras", C.c_uint64), ("n_points", C.c_uint64), ("n_obs", C.c_uint64),
+        ("bytes", C.c_uint64), ("chunks", C.c_uint64), ("slow_tokens", C.c_uint64),
+        ("regrouped", C.c_uint32), ("reserved", C.c_uint32),
+        ("ms_read", C.c_float), ("ms_h2d", C.c_float), ("ms_parse", C.c_float),
+    ]
+
+    def to_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
 CULL_GRID, CULL_EXHAUSTIVE = 0, 1
 BAL_TEXT, BAL_BINARY = 0, 1
-ERR_INVALID, ERR_IO = -1, -7
+ERR_INVALID, ERR_IO, ERR_PARSE = -1, -7, -8
 OCC_MESH, OCC_NONE, OCC_ANALYTIC = 0, 1, 2
 PRED_WATERTIGHT, PRED_MT = 0, 1
 
@@ -122,11 +136,11 @@ EXPORTS = [
     "c2b_add_drift", "c2b_add_drift_normalized", "c2b_add_noise", "c2b_add_sin_noise", "c2b_noise_timing",
     "c2b_add_drift_resident", "c2b_add_noise_resident", "c2b_add_sin_noise_resident", "c2b_download_problem",
     "c2b_mean_std", "c2b_cull_problem", "c2b_cull_problem_resident", "c2b_write_bal", "c2b_write_bal_resident",
-    "c2b_generate_world_points_uniform",
+    "c2b_read_bal_resident", "c2b_generate_world_points_uniform",
     "c2b_grid_num_cameras", "c2b_grid_num_points", "c2b_grid_cameras", "c2b_grid_points",
     "c2b_line_cameras", "c2b_line_points", "c2b_city_mesh", "c2b_camera_center",
     "c2b_camera_project_world", "c2b_camera_project", "c2b_camera_from_position_direction",
-    "c2b_camera_transform", "c2b_camera_to_vec",
+    "c2b_camera_transform", "c2b_camera_to_vec", "c2b_camera_from_vec",
 ]
 
 _lib = None
@@ -204,6 +218,7 @@ def lib():
     L.c2b_cull_problem_resident.argtypes = [vp, C.POINTER(CullStats)]
     L.c2b_write_bal.argtypes = [vp, C.c_char_p, i32, pd, u64, pd, u64, C.POINTER(u64), pu32, pd, C.POINTER(BalStats)]
     L.c2b_write_bal_resident.argtypes = [vp, C.c_char_p, i32, C.POINTER(BalStats)]
+    L.c2b_read_bal_resident.argtypes = [vp, C.c_char_p, i32, C.POINTER(BalReadStats)]
     L.c2b_probe_fp64.argtypes = [vp, pd]
     L.c2b_generate_world_points_uniform.argtypes = [vp, pf, u64, pu32, u64, pd, u64, u64, dbl, u64, pd,
                                                     C.POINTER(u64)]
@@ -228,6 +243,8 @@ def lib():
     L.c2b_camera_transform.restype = None
     L.c2b_camera_to_vec.argtypes = [pd, pd]
     L.c2b_camera_to_vec.restype = None
+    L.c2b_camera_from_vec.argtypes = [pd, pd]
+    L.c2b_camera_from_vec.restype = None
     _lib = L
     return L
 

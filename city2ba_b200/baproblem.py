@@ -576,6 +576,21 @@ class BAProblem:
         return cls.new(cams, pts, list(zip(ci, pi, ou.tolist(), ov.tolist())))
 
     @classmethod
+    def from_file_gpu(cls, path, ctx=None, stats=None):
+        """from_file() with the file parsed on the GPU (c2b_read_bal_resident), then the problem and its CSR
+        downloaded.  The file's problem REPLACES the ctx's resident problem.  Raises what from_file raises: ParseError,
+        IOError_, AssertionError for an observation index out of range.  `stats`, a dict if given, receives the read's
+        stats (bytes, chunks, slow_tokens, regrouped, ms_read, ms_h2d, ms_parse)."""
+        from .generate import ResidentProblem
+        rp = ResidentProblem(ctx or context())
+        st = rp.read(path)
+        if stats is not None:
+            stats.update(st)
+        cams, pts = rp.download_problem(st["n_cameras"], st["n_points"])
+        g = rp.download()
+        return cls(cams, pts, VisGraph(g.offsets, g.point_idx.astype(np.uint64), g.uv.reshape(-1, 2)))
+
+    @classmethod
     def from_file(cls, path):
         """src/baproblem.rs:697-706"""
         ext = str(path).rsplit(".", 1)[-1]

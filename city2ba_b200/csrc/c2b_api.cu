@@ -2,6 +2,7 @@
 // host-side orchestration of the kernels: upload -> (grid build) -> cull -> radix sort ->
 // warp-cooperative BVH traversal -> compaction -> download.
 #include <algorithm>
+#include <charconv>
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -16,11 +17,13 @@
 #if defined(__linux__)
 #include <cerrno>
 #include <fcntl.h>
+#include <unistd.h>
 #include <sys/mman.h>
 #include <sys/stat.h>
 #endif
 
 #include "c2b_bal.cuh"
+#include "c2b_bal_read.cuh"
 #include "c2b_bvh.cuh"
 #include "c2b_common.cuh"
 #include "c2b_compact.cuh"
@@ -279,11 +282,16 @@ struct CtxExtra {
   // BAL writer (c2b_bal.cuh): window lengths / offsets, two chunk buffers, camera 9-vectors, pinned chunk ring
   DevBuf bal_scan, bal_out[2], bal_vecs;
   PinBuf bal_ring;
+  // BAL reader (c2b_bal_read.cuh): per-observation camera, per-camera counts, slow-token records of two chunks,
+  // error offsets / token counter
+  DevBuf bal_cam, bal_cnt, bal_slow[2], bal_small;
   ~CtxExtra() {
     pg_idx.release();
     pg_uv.release();
     pin_out.release();
-    for (DevBuf *b : {&bal_scan, &bal_out[0], &bal_out[1], &bal_vecs}) b->release();
+    for (DevBuf *b : {&bal_scan, &bal_out[0], &bal_out[1], &bal_vecs, &bal_cam, &bal_cnt, &bal_slow[0], &bal_slow[1],
+                      &bal_small})
+      b->release();
     bal_ring.release();
   }
   GridCache grid;
@@ -2782,5 +2790,459 @@ int c2b_write_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_s
                   ctx->out_idx[sel].as<uint32_t>(), ctx->out_uv[sel].as<double>(), C, P, O};
   return bal_stream(ctx, path, format, v, out);
 }
+
+// ---- reading BAL files (c2b_bal_read.cuh) ----------------------------------------------------------------------------
+namespace {
+constexpr unsigned long long BAL_NO_ERR = ~0ull;
+
+// pread until `want` bytes or the end of the file; the bytes read, or -1 with errno
+int64_t bal_pread(int fd, char *dst, uint64_t want, uint64_t off, double &ms) {
+  const auto t0 = std::chrono::steady_clock::now();
+  uint64_t got = 0;
+  while (got < want) {
+    const ssize_t r = ::pread(fd, dst + got, want - got, (off_t)(off + got));
+    if (r < 0 && errno == EINTR) continue;
+    if (r < 0) return -1;
+    if (r == 0) break;
+    got += (uint64_t)r;
+  }
+  ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  return (int64_t)got;
+}
+
+struct BalReadState {
+  c2b_ctx *ctx;
+  CtxExtra *x;
+  const char *path;
+  int fd;
+  uint64_t size, B;
+  uint64_t C = 0, P = 0, O = 0;
+  BalEvents events;
+  double ms_read = 0;
+  float ms_h2d = 0, ms_parse = 0;
+  uint64_t chunks = 0, bytes = 0, slow = 0;
+  uint32_t regrouped = 0;
+  unsigned long long *d_err = nullptr;  // [0] malformed token, [1] index out of range; then u64 base, u32 total, ...
+  double *vecs = nullptr, *pts = nullptr;
+  // the device times of the chunk in ring slot `slot` (its parse has finished)
+  void add_times(int slot) {
+    float a = 0, b = 0;
+    cudaEventElapsedTime(&a, events.e[slot][0], events.e[slot][1]);
+    cudaEventElapsedTime(&b, events.e[slot][2], events.e[slot][3]);
+    ms_h2d += a;
+    ms_parse += b;
+  }
+};
+
+// C, P and O known: checks the limits and sizes the resident arrays (the old resident problem is gone from here on)
+int bal_read_alloc(BalReadState &s) {
+  c2b_ctx *ctx = s.ctx;
+  CtxExtra *x = s.x;
+  if (s.C >= 0xffffffffull || s.P >= 0xffffffffull || s.O >= 0xffffffffull)
+    return set_error(C2B_ERR_INVALID, "c2b_read_bal_resident: %s: C = %llu, P = %llu, O = %llu; each must be below "
+                     "2^32 - 1", s.path, (unsigned long long)s.C, (unsigned long long)s.P, (unsigned long long)s.O);
+  const int sel = ctx->out_sel;
+  C2B_TRY(ctx->out_offsets[sel].ensure((s.C + 1) * 8));
+  C2B_TRY(ctx->out_idx[sel].ensure(std::max<uint64_t>(s.O, 1) * 4));
+  C2B_TRY(ctx->out_uv[sel].ensure(std::max<uint64_t>(s.O, 1) * 16));
+  C2B_TRY(x->bal_vecs.ensure(std::max<uint64_t>(s.C, 1) * 72));
+  C2B_TRY(c2b_points_device_buffer(ctx, s.P, &s.pts));
+  s.vecs = x->bal_vecs.as<double>();
+  C2B_TRY(x->bal_out[0].ensure(s.B));
+  C2B_TRY(x->bal_out[1].ensure(s.B));
+  C2B_TRY(x->bal_small.ensure(64));
+  s.d_err = x->bal_small.as<unsigned long long>();
+  C2B_CUDA(cudaMemsetAsync(s.d_err, 0xff, 16, ctx->stream));
+  C2B_CUDA(cudaMemsetAsync(s.d_err + 2, 0, 48, ctx->stream));
+  return C2B_OK;
+}
+
+// the observations in file order (idx / uv of set `sel`, cam_of) -> the CSR grouped by camera, in file order within
+// a camera: offsets from a per-camera count and scan; a stable sort by camera and a gather when the file was not
+// already camera-major
+int bal_group(BalReadState &s) {
+  c2b_ctx *ctx = s.ctx;
+  CtxExtra *x = s.x;
+  cudaStream_t st = ctx->stream;
+  const uint64_t C = s.C, O = s.O;
+  const int sel = ctx->out_sel;
+  C2B_TRY(x->bal_cnt.ensure((C + 1) * 4));
+  uint32_t *cnt = x->bal_cnt.as<uint32_t>();
+  uint32_t *unordered = reinterpret_cast<uint32_t *>(s.d_err + 4);
+  C2B_CUDA(cudaMemsetAsync(cnt, 0, (C + 1) * 4, st));
+  if (O) {
+    k_bal_cam_count<<<blocks_for(O, BALR_THREADS), BALR_THREADS, 0, st>>>(x->bal_cam.as<uint32_t>(), O, cnt, unordered);
+    C2B_KERNEL_CHECK();
+  }
+  C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, unordered, 4, cudaMemcpyDeviceToHost, st));
+  C2B_CUDA(cudaStreamSynchronize(st));
+  s.regrouped = *ctx->h_small.as<uint32_t>() ? 1u : 0u;
+  const int fs = s.regrouped ? sel ^ 1 : sel;
+  C2B_TRY(ctx->out_offsets[fs].ensure((C + 1) * 8));
+  C2B_TRY(exclusive_scan_u32(st, cnt, cnt, C, nullptr, ctx->scan_tmp));
+  k_bal_offsets<<<blocks_for(C + 1, BALR_THREADS), BALR_THREADS, 0, st>>>(cnt, C, O, ctx->out_offsets[fs].as<uint64_t>());
+  C2B_KERNEL_CHECK();
+  if (s.regrouped) {
+    C2B_TRY(ctx->out_idx[fs].ensure(O * 4));
+    C2B_TRY(ctx->out_uv[fs].ensure(O * 16));
+    for (int i = 0; i < 2; ++i) {
+      C2B_TRY(ctx->sort_keys[i].ensure(O * 8));
+      C2B_TRY(ctx->sort_vals[i].ensure(O * 4));
+    }
+    uint64_t *keys[2] = {ctx->sort_keys[0].as<uint64_t>(), ctx->sort_keys[1].as<uint64_t>()};
+    uint32_t *vals[2] = {ctx->sort_vals[0].as<uint32_t>(), ctx->sort_vals[1].as<uint32_t>()};
+    k_bal_regroup_keys<<<blocks_for(O, BALR_THREADS), BALR_THREADS, 0, st>>>(x->bal_cam.as<uint32_t>(), O, keys[0], vals[0]);
+    C2B_KERNEL_CHECK();
+    int res = 0;
+    C2B_TRY(radix_sort_pairs(st, keys, vals, O, bit_length(C - 1), ctx->sort_hist, ctx->scan_tmp, &res));
+    k_bal_regroup_gather<<<blocks_for(O, BALR_THREADS), BALR_THREADS, 0, st>>>(
+        vals[res], O, ctx->out_idx[sel].as<uint32_t>(), ctx->out_uv[sel].as<double2>(), ctx->out_idx[fs].as<uint32_t>(),
+        ctx->out_uv[fs].as<double2>());
+    C2B_KERNEL_CHECK();
+    ctx->out_sel = fs;
+  }
+  return C2B_OK;
+}
+
+int bal_read_text(BalReadState &s) {
+  c2b_ctx *ctx = s.ctx;
+  CtxExtra *x = s.x;
+  cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+  const uint64_t B = s.B;
+  char *ring = x->bal_ring.as<char>();
+  auto &ev = s.events.e;
+  // the header, on the host, from the first chunk
+  const int64_t got0 = bal_pread(s.fd, ring, std::min(B, s.size), 0, s.ms_read);
+  if (got0 < 0) return set_error(C2B_ERR_IO, "cannot read %s: %s", s.path, strerror(errno));
+  uint64_t hdr[3];
+  {
+    uint64_t i = 0;
+    for (int k = 0; k < 3; ++k) {
+      while (i < (uint64_t)got0 && bal_ws(ring[i])) ++i;
+      if (i == (uint64_t)got0) {
+        if ((uint64_t)got0 == s.size)
+          return set_error(C2B_ERR_PARSE, "%s: byte %llu: the file ends inside the header", s.path, (unsigned long long)s.size);
+        return set_error(C2B_ERR_PARSE, "%s: byte %llu: the header does not fit in one chunk (bal_chunk_bytes)", s.path,
+                         (unsigned long long)i);
+      }
+      const uint64_t b = i;
+      while (i < (uint64_t)got0 && !bal_ws(ring[i])) ++i;
+      if (i == (uint64_t)got0 && (uint64_t)got0 < s.size)
+        return set_error(C2B_ERR_PARSE, "%s: byte %llu: the header does not fit in one chunk (bal_chunk_bytes)", s.path,
+                         (unsigned long long)b);
+      if (!bal_parse_index(ring + b, (uint32_t)(i - b), hdr[k]))
+        return set_error(C2B_ERR_PARSE, "%s: byte %llu: malformed header count", s.path, (unsigned long long)b);
+    }
+  }
+  s.C = hdr[0], s.P = hdr[1], s.O = hdr[2];
+  // 3 + 4 O + 9 C + 3 P tokens of at least one byte, separated by at least one byte
+  const unsigned __int128 need = (unsigned __int128)3 + (unsigned __int128)4 * s.O + (unsigned __int128)9 * s.C +
+                                 (unsigned __int128)3 * s.P;
+  if (2 * need - 1 > s.size)
+    return set_error(C2B_ERR_PARSE, "%s: byte 0: the header's counts need more bytes than the file has (%llu)", s.path,
+                     (unsigned long long)s.size);
+  C2B_TRY(bal_read_alloc(s));
+  const uint64_t C = s.C, P = s.P, O = s.O, n_tok = (uint64_t)need;
+  C2B_TRY(x->bal_cam.ensure(std::max<uint64_t>(O, 1) * 4));
+  const uint64_t max_words = (B + 31) / 32;
+  C2B_TRY(x->bal_scan.ensure(max_words * 8 + 64));
+  // a slow token has more than 19 digits: at most B / 20 + 1 of them per chunk
+  C2B_TRY(x->bal_slow[0].ensure((B / 20 + 2) * sizeof(BalSlow)));
+  C2B_TRY(x->bal_slow[1].ensure((B / 20 + 2) * sizeof(BalSlow)));
+  uint32_t *words = x->bal_scan.as<uint32_t>(), *first = words + max_words, *total = first + max_words;
+  uint64_t *base = reinterpret_cast<uint64_t *>(s.d_err + 2);
+  uint32_t *n_slow = reinterpret_cast<uint32_t *>(s.d_err + 3);  // [0], [1]: the two chunk buffers
+  const int sel = ctx->out_sel;
+  BalTextArgs a{};
+  a.C = C, a.P = P, a.O = O;
+  a.cam_of = x->bal_cam.as<uint32_t>();
+  a.idx = ctx->out_idx[sel].as<uint32_t>();
+  a.uv = ctx->out_uv[sel].as<double>();
+  a.vecs = s.vecs;
+  a.pts = s.pts;
+  a.err = s.d_err;
+  a.words = words;
+  a.first = first;
+  a.base = base;
+  // per ring slot, in pinned memory once the chunk's parse is done: its slow-token count and the running ordinal
+  uint64_t *h_tail = ctx->h_small.as<uint64_t>() + 4;
+  std::vector<uint64_t> slow_pairs;  // (ordinal, bits)
+  std::vector<BalSlow> recs;
+  uint64_t ordinals_done = 0;
+  // chunk j's parse is finished: its times, its slow tokens converted from the ring slot's bytes
+  auto drain = [&](uint64_t j, uint32_t n_bytes) -> int {
+    const int slot = (int)(j % BAL_RING);
+    C2B_CUDA(cudaEventSynchronize(ev[slot][3]));
+    s.add_times(slot);
+    const uint32_t k = (uint32_t)h_tail[2 * slot];
+    ordinals_done = h_tail[2 * slot + 1];
+    if (k) {
+      recs.resize(k);
+      C2B_CUDA(cudaMemcpyAsync(recs.data(), x->bal_slow[j % 2].p, (size_t)k * sizeof(BalSlow), cudaMemcpyDeviceToHost,
+                               ctx->aux_stream));
+      C2B_CUDA(cudaStreamSynchronize(ctx->aux_stream));
+      const char *bytes = ring + (size_t)slot * B;
+      for (const BalSlow &r : recs) {
+        const uint32_t len = r.len & 0x7fffffffu;
+        if (r.pos + len > n_bytes) return set_error(C2B_ERR_CUDA, "BAL reader: slow token record out of its chunk");
+        const char *t = bytes + r.pos, *e = t + len;
+        const bool neg = *t == '-';
+        if (*t == '-' || *t == '+') ++t;
+        double v = 0;
+        const auto res = std::from_chars(t, e, v, std::chars_format::general);
+        if (res.ptr != e || (res.ec != std::errc() && res.ec != std::errc::result_out_of_range))
+          return set_error(C2B_ERR_PARSE, "%s: malformed number (host conversion)", s.path);
+        if (res.ec == std::errc::result_out_of_range) v = (r.len & 0x80000000u) ? INFINITY : 0.0;
+        if (neg) v = -v;
+        uint64_t bits;
+        memcpy(&bits, &v, 8);
+        slow_pairs.push_back(r.ordinal);
+        slow_pairs.push_back(bits);
+      }
+      s.slow += k;
+    }
+    return C2B_OK;
+  };
+  uint64_t read_pos = (uint64_t)got0, chunk_off = 0, have = (uint64_t)got0;
+  uint64_t prev_n = 0, tail = 0;
+  int64_t pending = -1;
+  uint32_t pending_n = 0;
+  for (uint64_t k = 0;; ++k) {
+    const int slot = (int)(k % BAL_RING);
+    char *sp = ring + (size_t)slot * B;
+    if (k > 0) {
+      // the slot's previous chunk (k - 3) left with the copy that preceded chunk k - 2's parse, which was drained
+      memcpy(sp, ring + (size_t)((k - 1) % BAL_RING) * B + prev_n, tail);
+      const int64_t r = bal_pread(s.fd, sp + tail, B - tail, read_pos, s.ms_read);
+      if (r < 0) return set_error(C2B_ERR_IO, "cannot read %s: %s", s.path, strerror(errno));
+      read_pos += (uint64_t)r;
+      have = tail + (uint64_t)r;
+    }
+    const bool eof = read_pos >= s.size;
+    uint64_t n = have;
+    if (!eof) {
+      while (n > 0 && !bal_ws(sp[n - 1])) --n;
+      if (n == 0)
+        return set_error(C2B_ERR_PARSE, "%s: byte %llu: a token longer than bal_chunk_bytes (%llu)", s.path,
+                         (unsigned long long)chunk_off, (unsigned long long)B);
+    }
+    if (n) {
+      const uint32_t nw = (uint32_t)((n + 31) / 32);
+      char *dbuf = x->bal_out[k % 2].as<char>();
+      C2B_CUDA(cudaEventRecord(ev[slot][0], cp));
+      C2B_CUDA(cudaMemcpyAsync(dbuf, sp, n, cudaMemcpyHostToDevice, cp));
+      C2B_CUDA(cudaEventRecord(ev[slot][1], cp));
+      C2B_CUDA(cudaStreamWaitEvent(st, ev[slot][1], 0));
+      C2B_CUDA(cudaEventRecord(ev[slot][2], st));
+      C2B_CUDA(cudaMemsetAsync(n_slow + (k % 2), 0, 4, st));
+      k_bal_tok_flags<<<blocks_for(n, BALR_THREADS), BALR_THREADS, 0, st>>>(dbuf, (uint32_t)n, words, first);
+      C2B_KERNEL_CHECK();
+      C2B_TRY(exclusive_scan_u32(st, first, first, nw, total, ctx->scan_tmp));
+      a.buf = dbuf;
+      a.n = (uint32_t)n;
+      a.file_off = chunk_off;
+      a.slow = x->bal_slow[k % 2].as<BalSlow>();
+      a.n_slow = n_slow + (k % 2);
+      k_bal_parse_text<<<blocks_for(nw, BALR_THREADS), BALR_THREADS, 0, st>>>(a, nw);
+      C2B_KERNEL_CHECK();
+      k_bal_tok_advance<<<1, 1, 0, st>>>(base, total);
+      C2B_KERNEL_CHECK();
+      C2B_CUDA(cudaMemcpyAsync(h_tail + 2 * slot, n_slow + (k % 2), 4, cudaMemcpyDeviceToHost, st));
+      C2B_CUDA(cudaMemcpyAsync(h_tail + 2 * slot + 1, base, 8, cudaMemcpyDeviceToHost, st));
+      C2B_CUDA(cudaEventRecord(ev[slot][3], st));
+      ++s.chunks;
+    }
+    // lag one: the previous chunk's slow tokens, while this one is on its way
+    if (pending >= 0) C2B_TRY(drain((uint64_t)pending, pending_n));
+    pending = n ? (int64_t)k : -1;
+    pending_n = (uint32_t)n;
+    if (eof || ordinals_done >= n_tok) break;  // tokens after the points are never read
+    chunk_off += n;
+    prev_n = n;
+    tail = have - n;
+  }
+  if (pending >= 0) C2B_TRY(drain((uint64_t)pending, pending_n));
+  s.bytes = read_pos;
+  C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, s.d_err, 24, cudaMemcpyDeviceToHost, st));
+  C2B_CUDA(cudaStreamSynchronize(st));
+  const unsigned long long *h = ctx->h_small.as<unsigned long long>();
+  if (h[0] != BAL_NO_ERR) return set_error(C2B_ERR_PARSE, "%s: byte %llu: malformed token", s.path, h[0]);
+  if (h[2] < n_tok)
+    return set_error(C2B_ERR_PARSE, "%s: byte %llu: the file ends after %llu of the %llu tokens its header needs", s.path,
+                     (unsigned long long)s.size, (unsigned long long)h[2], (unsigned long long)n_tok);
+  if (h[1] != BAL_NO_ERR)
+    return set_error(C2B_ERR_INVALID, "%s: byte %llu: observation index out of range (camera >= %llu or point >= %llu)",
+                     s.path, h[1], (unsigned long long)C, (unsigned long long)P);
+  if (!slow_pairs.empty()) {
+    const uint64_t ns = slow_pairs.size() / 2;
+    C2B_TRY(x->bal_slow[0].ensure(ns * 16));
+    C2B_CUDA(cudaMemcpyAsync(x->bal_slow[0].p, slow_pairs.data(), ns * 16, cudaMemcpyHostToDevice, st));
+    k_bal_scatter_slow<<<blocks_for(ns, BALR_THREADS), BALR_THREADS, 0, st>>>(x->bal_slow[0].as<uint64_t>(), ns, C, O,
+                                                                              a.uv, s.vecs, s.pts);
+    C2B_KERNEL_CHECK();
+  }
+  return bal_group(s);
+}
+
+int bal_read_binary(BalReadState &s) {
+  c2b_ctx *ctx = s.ctx;
+  CtxExtra *x = s.x;
+  cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+  const uint64_t B = s.B, W = B / 8;
+  char *ring = x->bal_ring.as<char>();
+  auto &ev = s.events.e;
+  unsigned char h24[24];
+  const int64_t g = bal_pread(s.fd, reinterpret_cast<char *>(h24), 24, 0, s.ms_read);
+  if (g < 0) return set_error(C2B_ERR_IO, "cannot read %s: %s", s.path, strerror(errno));
+  if (g < 24) return set_error(C2B_ERR_PARSE, "%s: byte %llu: truncated binary BAL file", s.path, (unsigned long long)g);
+  auto be = [](const unsigned char *b) {
+    uint64_t v = 0;
+    for (int k = 0; k < 8; ++k) v = (v << 8) | b[k];
+    return v;
+  };
+  s.C = be(h24), s.P = be(h24 + 8), s.O = be(h24 + 16);
+  if (s.C > s.size / 80 || s.P > s.size / 24 || s.O > s.size / 24)
+    return set_error(C2B_ERR_PARSE, "%s: byte 0: binary BAL header counts exceed the file size", s.path);
+  const uint64_t C = s.C, P = s.P, O = s.O;
+  const uint64_t words = 3 + C + 3 * O + 9 * C + 3 * P;
+  if (s.size < 8 * words)
+    return set_error(C2B_ERR_PARSE, "%s: byte %llu: truncated binary BAL file (%llu bytes needed)", s.path,
+                     (unsigned long long)s.size, (unsigned long long)(8 * words));
+  C2B_TRY(bal_read_alloc(s));
+  const int sel = ctx->out_sel;
+  std::vector<uint64_t> off(C + 1, 0);
+  uint64_t c = 0, seen = 0, next = 3;  // next: word of camera c's count
+  BalBinArgs a{};
+  a.C = C, a.P = P, a.O = O;
+  uint64_t *d_off = ctx->out_offsets[sel].as<uint64_t>();
+  a.off = d_off;
+  a.idx = ctx->out_idx[sel].as<uint32_t>();
+  a.uv = ctx->out_uv[sel].as<double>();
+  a.vecs = s.vecs;
+  a.pts = s.pts;
+  a.err = s.d_err;
+  for (uint64_t k = 0, w0 = 0; w0 < words; ++k, w0 += W) {
+    const int slot = (int)(k % BAL_RING);
+    char *sp = ring + (size_t)slot * B;
+    const uint64_t n = std::min(W, words - w0);
+    if (k >= BAL_RING) {  // the slot's previous chunk has been copied and parsed
+      C2B_CUDA(cudaEventSynchronize(ev[slot][3]));
+      s.add_times(slot);
+    }
+    const int64_t r = bal_pread(s.fd, sp, 8 * n, 8 * w0, s.ms_read);
+    if (r < 0) return set_error(C2B_ERR_IO, "cannot read %s: %s", s.path, strerror(errno));
+    if ((uint64_t)r < 8 * n)
+      return set_error(C2B_ERR_PARSE, "%s: byte %llu: truncated binary BAL file", s.path,
+                       (unsigned long long)(8 * w0 + (uint64_t)r));
+    // the chain of count words inside this chunk
+    const uint64_t c0 = c;
+    while (c < C && next < w0 + n) {
+      const uint64_t cnt = be(reinterpret_cast<const unsigned char *>(sp) + 8 * (next - w0));
+      if (cnt > O - seen)
+        return set_error(C2B_ERR_PARSE, "%s: byte %llu: camera %llu's observation count %llu exceeds the %llu left",
+                         s.path, (unsigned long long)(8 * next), (unsigned long long)c, (unsigned long long)cnt,
+                         (unsigned long long)(O - seen));
+      off[c] = seen;
+      seen += cnt;
+      ++c;
+      next = 3 + c + 3 * seen;
+    }
+    char *dbuf = x->bal_out[k % 2].as<char>();
+    if (k >= 2) C2B_CUDA(cudaStreamWaitEvent(cp, ev[(k - 2) % BAL_RING][3], 0));  // chunk k - 2 left dbuf
+    C2B_CUDA(cudaEventRecord(ev[slot][0], cp));
+    if (c > c0)
+      C2B_CUDA(cudaMemcpyAsync(d_off + c0, off.data() + c0, (c - c0) * 8, cudaMemcpyHostToDevice, cp));
+    C2B_CUDA(cudaMemcpyAsync(dbuf, sp, 8 * n, cudaMemcpyHostToDevice, cp));
+    C2B_CUDA(cudaEventRecord(ev[slot][1], cp));
+    C2B_CUDA(cudaStreamWaitEvent(st, ev[slot][1], 0));
+    C2B_CUDA(cudaEventRecord(ev[slot][2], st));
+    a.buf = reinterpret_cast<const uint64_t *>(dbuf);
+    a.w0 = w0;
+    a.n = n;
+    a.c_known = c;
+    k_bal_parse_binary<<<blocks_for(n, BALR_THREADS), BALR_THREADS, 0, st>>>(a);
+    C2B_KERNEL_CHECK();
+    C2B_CUDA(cudaEventRecord(ev[slot][3], st));
+    ++s.chunks;
+    s.bytes += 8 * n;
+  }
+  C2B_CUDA(cudaStreamSynchronize(st));
+  for (uint64_t k = s.chunks >= BAL_RING ? s.chunks - BAL_RING : 0; k < s.chunks; ++k) s.add_times((int)(k % BAL_RING));
+  if (seen != O)
+    return set_error(C2B_ERR_PARSE, "%s: byte %llu: the cameras' observation counts sum to %llu, the header says %llu",
+                     s.path, (unsigned long long)(8 * (3 + C + 3 * seen)), (unsigned long long)seen,
+                     (unsigned long long)O);
+  off[C] = O;
+  C2B_CUDA(cudaMemcpyAsync(d_off + C, off.data() + C, 8, cudaMemcpyHostToDevice, st));
+  C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, s.d_err, 16, cudaMemcpyDeviceToHost, st));
+  C2B_CUDA(cudaStreamSynchronize(st));
+  const unsigned long long bad = ctx->h_small.as<unsigned long long>()[1];
+  if (bad != BAL_NO_ERR)
+    return set_error(C2B_ERR_INVALID, "%s: byte %llu: observation index out of range (point >= %llu)", s.path, bad,
+                     (unsigned long long)P);
+  return C2B_OK;
+}
+}  // namespace
+
+int c2b_read_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_read_stats *out) {
+  if (!ctx || !path) return set_error(C2B_ERR_INVALID, "c2b_read_bal_resident: null argument");
+  if (format != C2B_BAL_TEXT && format != C2B_BAL_BINARY)
+    return set_error(C2B_ERR_INVALID, "c2b_read_bal_resident: unknown format %d", format);
+  CtxExtra *x = extra_of(ctx);
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  // whatever happens below, the previous resident problem is replaced
+  x->have_result = x->have_cameras = x->have_points = false;
+  x->host_call_last = false;
+  x->grid.valid = false;
+  BalReadState s{ctx, x, path, -1, 0, x->tun.bal_chunk_bytes};
+  s.fd = open(path, O_RDONLY | O_CLOEXEC);
+  if (s.fd < 0) return set_error(C2B_ERR_IO, "cannot open %s: %s", path, strerror(errno));
+  int rc = [&]() -> int {
+    struct stat sb;
+    if (fstat(s.fd, &sb) != 0 || !S_ISREG(sb.st_mode)) return set_error(C2B_ERR_IO, "%s is not a regular file", path);
+    s.size = (uint64_t)sb.st_size;
+    C2B_TRY(s.events.create());
+    x->bal_ring.node = ctx->numa_node;
+    C2B_TRY(x->bal_ring.ensure(BAL_RING * s.B));
+    C2B_TRY(ctx->h_small.ensure(256));
+    C2B_TRY(format == C2B_BAL_TEXT ? bal_read_text(s) : bal_read_binary(s));
+    // install as c2b_cull_problem_resident does: camera records on the host (from_vec), points, CSR
+    const uint64_t C = s.C, P = s.P, O = s.O;
+    std::vector<double> vecs(9 * C), cams(15 * C);
+    if (C) C2B_CUDA(cudaMemcpyAsync(vecs.data(), s.vecs, C * 72, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    for (uint64_t c = 0; c < C; ++c) c2b_camera_from_vec(&vecs[9 * c], &cams[15 * c]);
+    C2B_TRY(c2b_upload_cameras(ctx, cams.data(), C));
+    C2B_TRY(c2b_points_commit(ctx, P));
+    ctx->out_C = C;
+    ctx->out_O = O;
+    C2B_CUDA(cudaStreamSynchronize(st));
+    x->have_result = true;
+    return C2B_OK;
+  }();
+  close(s.fd);
+  if (rc != C2B_OK) {
+    cudaStreamSynchronize(st);
+    cudaStreamSynchronize(ctx->copy_stream);
+    x->have_result = x->have_cameras = x->have_points = false;
+    return rc;
+  }
+  if (out) {
+    memset(out, 0, sizeof *out);
+    out->n_cameras = s.C;
+    out->n_points = s.P;
+    out->n_obs = s.O;
+    out->bytes = s.bytes;
+    out->chunks = s.chunks;
+    out->slow_tokens = s.slow;
+    out->regrouped = s.regrouped;
+    out->ms_read = (float)s.ms_read;
+    out->ms_h2d = s.ms_h2d;
+    out->ms_parse = s.ms_parse;
+  }
+  return C2B_OK;
+}
+
 
 }  // extern "C"

@@ -176,12 +176,10 @@ void c2b_camera_transform(const double *cam, const double dR[9], const double dl
   memcpy(cam_out, out, sizeof out);
 }
 
-// SnavelyCamera::to_vec (src/baproblem.rs:192-202, to_rodrigues :93-102): the same operations in the same order as
-// include/city2ba.hpp's to_vec / to_rodrigues / detail::quat_from_mat, so that the BAL writer's camera lines equal
-// the C++ mirror's bit for bit (acos is the host libm's; the device's differs)
-void c2b_camera_to_vec(const double *cam, double out[9]) {
-  auto M = [&](int c, int r) { return cam[c * 3 + r]; };
-  double q[4];
+// cgmath Quaternion::from(Matrix3) (Shepperd branches) as include/city2ba.hpp's detail::quat_from_mat: m column-major,
+// q = (s, x, y, z)
+static void quat_from_mat(const double *m, double q[4]) {
+  auto M = [&](int c, int r) { return m[c * 3 + r]; };
   const double trace = (M(0, 0) + M(1, 1)) + M(2, 2);
   if (trace >= 0.0) {
     double s = std::sqrt(1.0 + trace);
@@ -204,6 +202,14 @@ void c2b_camera_to_vec(const double *cam, double out[9]) {
     s = 0.5 / s;
     q[0] = (M(0, 1) - M(1, 0)) * s, q[1] = (M(0, 2) + M(2, 0)) * s, q[2] = (M(2, 1) + M(1, 2)) * s, q[3] = z;
   }
+}
+
+// SnavelyCamera::to_vec (src/baproblem.rs:192-202, to_rodrigues :93-102): the same operations in the same order as
+// include/city2ba.hpp's to_vec / to_rodrigues / detail::quat_from_mat, so that the BAL writer's camera lines equal
+// the C++ mirror's bit for bit (acos is the host libm's; the device's differs)
+void c2b_camera_to_vec(const double *cam, double out[9]) {
+  double q[4];
+  quat_from_mat(cam, q);
   const double angle = 2.0 * std::acos(std::max(-1.0, std::min(1.0, q[0])));
   const double d = 1.0 - q[0] * q[0];
   if (d < 2.220446049250313e-16) {
@@ -215,6 +221,37 @@ void c2b_camera_to_vec(const double *cam, double out[9]) {
     for (int k = 0; k < 3; ++k) out[k] = a[k] * inv * angle;
   }
   for (int k = 0; k < 6; ++k) out[3 + k] = cam[9 + k];
+}
+
+// SnavelyCamera::from_vec (src/baproblem.rs:180-190, from_rodrigues :78-90): the operations of include/city2ba.hpp's
+// from_vec / from_rodrigues / from_axis_angle / detail::mat_from_quat in the same order, so that the BAL reader's
+// camera records equal the C++ mirror's bit for bit (sin / cos / sqrt are the host libm's; the device's differ)
+void c2b_camera_from_vec(const double v[9], double *cam_out) {
+  const double x[3] = {v[0], v[1], v[2]};
+  double R[9];
+  const double theta2 = (x[0] * x[0] + x[1] * x[1]) + x[2] * x[2];
+  if (theta2 > 2.220446049250313e-16) {
+    const double angle = std::sqrt(theta2), inv = 1.0 / angle;
+    const double a[3] = {x[0] * inv, x[1] * inv, x[2] * inv};
+    const double s = std::sin(angle), c = std::cos(angle), k = 1.0 - c;
+    const double m[9] = {k * a[0] * a[0] + c,        k * a[0] * a[1] + s * a[2], k * a[0] * a[2] - s * a[1],
+                         k * a[0] * a[1] - s * a[2], k * a[1] * a[1] + c,        k * a[1] * a[2] + s * a[0],
+                         k * a[0] * a[2] + s * a[1], k * a[1] * a[2] - s * a[0], k * a[2] * a[2] + c};
+    memcpy(R, m, sizeof R);
+  } else {
+    const double m[9] = {1.0, x[2], -x[1], -x[2], 1.0, x[0], x[1], -x[0], 1.0};
+    double q[4];
+    quat_from_mat(m, q);
+    const double s = q[0], qx = q[1], y = q[2], z = q[3];
+    const double x2 = qx + qx, y2 = y + y, z2 = z + z;
+    const double xx2 = x2 * qx, xy2 = x2 * y, xz2 = x2 * z, yy2 = y2 * y, yz2 = y2 * z, zz2 = z2 * z;
+    const double sy2 = y2 * s, sz2 = z2 * s, sx2 = x2 * s;
+    const double r[9] = {1.0 - yy2 - zz2, xy2 + sz2, xz2 - sy2, xy2 - sz2, 1.0 - xx2 - zz2, yz2 + sx2,
+                         xz2 + sy2, yz2 - sx2, 1.0 - xx2 - yy2};
+    memcpy(R, r, sizeof R);
+  }
+  memcpy(cam_out, R, sizeof R);
+  for (int k = 0; k < 6; ++k) cam_out[9 + k] = v[3 + k];
 }
 
 }  // extern "C"

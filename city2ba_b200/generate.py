@@ -352,6 +352,28 @@ class ResidentProblem:
             raise
         return st.to_dict()
 
+    def read(self, path) -> dict:
+        """BAProblem::from_file into HBM (c2b_read_bal_resident): .bal text or .bbal binary by the extension, streamed
+        to the device and parsed there.  The file's problem replaces the resident one; afterwards download /
+        download_problem / reprojection_error / add_* / cull / write see it.  Raises ParseError on a malformed or
+        short file, IOError_ when it cannot be read, AssertionError on an observation index out of range (the errors
+        of BAProblem.from_file).  Returns the stats: n_cameras, n_points, n_obs, bytes, chunks, slow_tokens (numbers
+        converted on the host), regrouped, ms_read (host time in pread(2)), ms_h2d, ms_parse (device time)."""
+        from .baproblem import BAProblem, IOError_, ParseError
+        fmt = _lib.BAL_BINARY if BAProblem._bal_binary(path) else _lib.BAL_TEXT
+        st = _lib.BalReadStats()
+        try:
+            check(lib().c2b_read_bal_resident(self.ctx.handle, str(path).encode(), fmt, C.byref(st)))
+        except _lib.C2BError as e:
+            if e.code == _lib.ERR_PARSE:
+                raise ParseError(str(e)) from e
+            if e.code == _lib.ERR_IO:
+                raise IOError_(str(e)) from e
+            if e.code == _lib.ERR_INVALID and "index out of range" in str(e):
+                raise AssertionError(str(e)) from e
+            raise
+        return st.to_dict()
+
 
 def generate_world_points_uniform(xyz, tri, cameras, num_points, max_dist, seed=None, ctx=None) -> np.ndarray:
     """src/generate.rs:356-420 on the GPU: `num_points` points on the mesh (area-weighted triangle,

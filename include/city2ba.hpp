@@ -55,7 +55,10 @@ struct Error : std::runtime_error {
 namespace detail {
 inline void check(int rc) {
   if (rc == C2B_OK) return;
-  throw Error(rc == C2B_ERR_EMPTY ? Error::EmptyProblem : rc == C2B_ERR_IO ? Error::IOError : Error::Gpu,
+  throw Error(rc == C2B_ERR_EMPTY   ? Error::EmptyProblem
+              : rc == C2B_ERR_IO    ? Error::IOError
+              : rc == C2B_ERR_PARSE ? Error::ParseError
+                                    : Error::Gpu,
               c2b_last_error());
 }
 inline void require(bool ok, const char *what) {
@@ -1186,6 +1189,35 @@ struct BAProblem {
       throw Error(Error::IOError, "unknown file extension: " + path);
     }
     return ba;  // possibly empty, like the reference's from_file; EmptyProblem is run_generate's (src/bin/city2ba.rs:550-554)
+  }
+  // the same file parsed on the GPU (c2b_read_bal_resident): it becomes the ctx's resident problem, then the cameras,
+  // points and CSR are downloaded.  Errors as above: Error::ParseError, Error::IOError, std::logic_error for an
+  // observation index out of range.  stats (optional) receives sizes, chunks, slow tokens and the read / copy / parse
+  // times.
+  static BAProblem from_file(const Context &ctx, const std::string &path, c2b_bal_read_stats *stats = nullptr) {
+    const c2b_bal_format format = bal_format(path);
+    c2b_bal_read_stats st;
+    const int rc = c2b_read_bal_resident(ctx.handle(), path.c_str(), format, &st);
+    if (rc == C2B_ERR_INVALID && std::strstr(c2b_last_error(), "index out of range"))
+      throw std::logic_error(c2b_last_error());
+    detail::check(rc);
+    if (stats) *stats = st;
+    BAProblem ba;
+    std::vector<double> cams(st.n_cameras * C2B_CAM_STRIDE), pts(st.n_points * 3);
+    detail::check(c2b_download_problem(ctx.handle(), cams.data(), pts.data()));
+    ba.cameras.resize(st.n_cameras);
+    for (size_t i = 0; i < st.n_cameras; ++i) std::memcpy(ba.cameras[i].rec, &cams[i * C2B_CAM_STRIDE], sizeof ba.cameras[i].rec);
+    ba.points.resize(st.n_points);
+    for (size_t i = 0; i < st.n_points; ++i) std::memcpy(ba.points[i].data(), &pts[3 * i], 3 * sizeof(double));
+    c2b_obs obs;
+    detail::check(c2b_download_obs(ctx.handle(), &obs));
+    ba.vis_graph.resize(st.n_cameras);
+    for (size_t i = 0; i < st.n_cameras; ++i) {
+      ba.vis_graph[i].reserve(obs.offsets[i + 1] - obs.offsets[i]);
+      for (uint64_t k = obs.offsets[i]; k < obs.offsets[i + 1]; ++k)
+        ba.vis_graph[i].push_back({(size_t)obs.point_idx[k], {obs.uv[2 * k], obs.uv[2 * k + 1]}});
+    }
+    return ba;
   }
   // impl Display, src/baproblem.rs:788-801
   std::string to_string() const {

@@ -32,7 +32,8 @@ typedef enum {
   C2B_ERR_OOM = -4,       /* device or pinned-host allocation failed                      */
   C2B_ERR_EMPTY = -5,     /* empty problem (reference: Error::EmptyProblem, src/baproblem.rs:36) */
   C2B_ERR_NCCL = -6,      /* libnccl.so.2 could not be loaded, or an NCCL call failed (multi-GPU entries only) */
-  C2B_ERR_IO = -7         /* a file could not be created, or a write was short (reference: Error::IOError) */
+  C2B_ERR_IO = -7,        /* a file could not be created or opened, or a write was short (reference: Error::IOError) */
+  C2B_ERR_PARSE = -8      /* a BAL file does not follow its grammar or ends early (reference: Error::ParseError) */
 } c2b_status;
 
 typedef struct c2b_ctx c2b_ctx;
@@ -66,7 +67,8 @@ uint64_t c2b_kernel_launches(void);
  *   cold_staged (1)              first host-buffer call on a ctx: CSR in unpinned memory through a pinned ring
  *   stage_threads (4)            host threads staging a PAGEABLE input array through the pinned ring (0: leave
  *                                the pageable copy to the driver)
- *   bal_chunk_bytes (2^25)       byte budget of one chunk of c2b_write_bal* (device buffer and pinned ring slot);
+ *   bal_chunk_bytes (2^25)       byte budget of one chunk of c2b_write_bal* and c2b_read_bal_resident (device buffer
+ *                                and pinned ring slot);
  *                                at least 4096, rounded down to a multiple of 8
  * Unknown names are C2B_ERR_INVALID. */
 int c2b_tune(c2b_ctx *ctx, const char *name, double value);
@@ -347,6 +349,36 @@ int c2b_write_bal(c2b_ctx *ctx, const char *path, int format, const double *cams
  * in the cases c2b_cull_problem_resident refuses */
 int c2b_write_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_stats *out);
 
+/* ---- reading BAL files (BAProblem::from_file, src/baproblem.rs:580-706) -----------------------------------------
+ * The file is streamed to the device in chunks of at most bal_chunk_bytes (pinned ring -> device buffer), parsed
+ * there, and becomes the ctx's RESIDENT problem: cameras (c2b_camera_from_vec of the file's 9-vectors, on the host),
+ * points, and the CSR grouped by camera in file order (BAProblem::new, src/baproblem.rs:342-355).  Afterwards
+ * c2b_download_obs[_into], c2b_download_problem, c2b_reprojection_error_resident, c2b_add_*_resident,
+ * c2b_cull_problem_resident and c2b_write_bal_resident work on it.
+ *   C2B_BAL_TEXT    tokens separated by ASCII whitespace: "C P O", O x "c p u v", 9C camera numbers, 3P point
+ *                   numbers; tokens after them are ignored.  Indices are digits only (nom's digit1, fitting a u64);
+ *                   numbers follow Rust's f64::from_str ([+-]? digits with optional '.', optional exponent, or
+ *                   inf / infinity / nan in any case), correctly rounded (round half to even) for any digit count.
+ *                   A token longer than bal_chunk_bytes is C2B_ERR_PARSE.
+ *   C2B_BAL_BINARY  the layout c2b_write_bal writes; doubles are copied bit for bit; trailing bytes are ignored.
+ * C2B_ERR_PARSE: a malformed token (the message names the byte offset of the first), too few tokens, header counts
+ * the file cannot hold, a truncated binary file, binary counts that exceed what is left or do not sum to O.
+ * C2B_ERR_INVALID: an observation's camera or point index out of range (BAProblem::new's asserts), C, P or O not
+ * below 2^32 - 1, an unknown format.  C2B_ERR_IO: the file cannot be opened or read.  After any failure there is no
+ * resident problem (the entries above refuse with C2B_ERR_INVALID).  out may be NULL. */
+typedef struct {
+  uint64_t n_cameras, n_points, n_obs;
+  uint64_t bytes;       /* bytes of the file read */
+  uint64_t chunks;
+  uint64_t slow_tokens; /* numbers the device could not round on its own, converted on the host (std::from_chars) */
+  uint32_t regrouped;   /* 1 when the observations were not in camera order and were grouped on the device */
+  uint32_t reserved;
+  float ms_read;        /* host wall time in pread(2), summed */
+  float ms_h2d;         /* device time of the chunk copies, summed (CUDA events) */
+  float ms_parse;       /* device time of the parse kernels, summed (CUDA events) */
+} c2b_bal_read_stats;
+int c2b_read_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_read_stats *out);
+
 /* ---- input generation on the GPU -------------------------------------------------------------------
  * replaces generate_world_points_uniform (src/generate.rs:356-420): num_points world points, each
  * on an area-weighted random triangle (all index triples of all models, concatenated), uniform
@@ -385,6 +417,9 @@ void c2b_camera_transform(const double *cam, const double dR[9], const double dl
 /* SnavelyCamera::to_vec (src/baproblem.rs:192-202): [rodrigues 3, translation 3, f, k1, k2], the same operations
  * as include/city2ba.hpp's to_vec, bit for bit */
 void c2b_camera_to_vec(const double *cam, double out[9]);
+/* SnavelyCamera::from_vec (src/baproblem.rs:180-190): the record of a 9-vector, the same operations as
+ * include/city2ba.hpp's from_vec (both branches of from_rodrigues), bit for bit */
+void c2b_camera_from_vec(const double v[9], double *cam_out);
 
 #ifdef __cplusplus
 }

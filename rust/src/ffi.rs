@@ -57,6 +57,16 @@ pub struct c2b_bal_stats {
     pub ms_encode: c_float, pub ms_d2h: c_float, pub ms_write: c_float,
 }
 
+// BAL files read on the GPU into the resident problem (c2b_read_bal_resident)
+pub const C2B_ERR_PARSE: c_int = -8;
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct c2b_bal_read_stats {
+    pub n_cameras: u64, pub n_points: u64, pub n_obs: u64,
+    pub bytes: u64, pub chunks: u64, pub slow_tokens: u64,
+    pub regrouped: u32, pub reserved: u32,
+    pub ms_read: c_float, pub ms_h2d: c_float, pub ms_parse: c_float,
+}
+
 // Embree's RTCRay layout (48 bytes): what embree_rs::Ray wraps (src/generate.rs:253-262, :457-464)
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct c2b_ray48 {
@@ -151,6 +161,8 @@ extern "C" {
                          uv: *const c_double, out: *mut c2b_bal_stats) -> c_int;
     pub fn c2b_write_bal_resident(ctx: *mut c2b_ctx, path: *const c_char, format: c_int,
                                   out: *mut c2b_bal_stats) -> c_int;
+    pub fn c2b_read_bal_resident(ctx: *mut c2b_ctx, path: *const c_char, format: c_int,
+                                 out: *mut c2b_bal_read_stats) -> c_int;
     // ---- input generation ----
     pub fn c2b_generate_world_points_uniform(ctx: *mut c2b_ctx, xyz: *const c_float, nv: u64, tri: *const u32,
                                              nt: u64, cams: *const c_double, c: u64, num_points: u64,
@@ -175,4 +187,5 @@ extern "C" {
     pub fn c2b_camera_transform(cam: *const c_double, d_r: *const c_double, dloc: *const c_double,
                                 cam_out: *mut c_double);
     pub fn c2b_camera_to_vec(cam: *const c_double, out: *mut c_double);
+    pub fn c2b_camera_from_vec(v: *const c_double, cam_out: *mut c_double);
 }
