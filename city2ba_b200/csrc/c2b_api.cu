@@ -125,6 +125,17 @@ struct Tunables {
 struct PageBuf {
   void *p = nullptr;
   size_t cap = 0;
+  PageBuf() = default;
+  PageBuf(PageBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, (size_t)0)) {}
+  PageBuf &operator=(PageBuf &&o) noexcept {
+    if (this != &o) {
+      release();
+      p = std::exchange(o.p, nullptr);
+      cap = std::exchange(o.cap, (size_t)0);
+    }
+    return *this;
+  }
+  ~PageBuf() { release(); }
   int ensure_fresh(size_t bytes) {  // contents are not kept
     if (bytes <= cap) return C2B_OK;
     release();
@@ -155,6 +166,7 @@ struct PageBuf {
     return reinterpret_cast<T *>(p);
   }
 };
+static_assert(!std::is_copy_constructible<PageBuf>::value, "PageBuf is move-only");
 
 // Device -> pageable host memory through a pinned ring: `threads` host threads, each with its own stream and two
 // 2 MB ring slots, take 2 MB chunks off a queue: DMA into a slot, then memcpy the slot to its destination (the
@@ -216,8 +228,8 @@ class Drainer {
   };
   void loop(int device, char *slots) {
     cudaError_t e = cudaSetDevice(device);
-    cudaStream_t st = nullptr;
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
+    Stream st;  // destroyed on this thread, with `device` current
+    if (e == cudaSuccess && st.create(cudaStreamNonBlocking) != C2B_OK) e = cudaGetLastError();
     for (int turn = 0;; ++turn) {
       Chunk c;
       {
@@ -245,7 +257,6 @@ class Drainer {
       cv_done_.notify_all();
       if (e != cudaSuccess) break;
     }
-    if (st) cudaStreamDestroy(st);
     cv_done_.notify_all();
   }
   int n_ = 0;
@@ -272,7 +283,9 @@ struct PassMemo {
   bool valid = false, any_overflow = false, big = false;
 };
 
-struct CtxExtra {
+}  // namespace
+
+struct c2b::CtxExtra {
   Tunables tun;
   CallHist hist;
   PassMemo memo;
@@ -285,15 +298,6 @@ struct CtxExtra {
   // BAL reader (c2b_bal_read.cuh): per-observation camera, per-camera counts, slow-token records of two chunks,
   // error offsets / token counter
   DevBuf bal_cam, bal_cnt, bal_slow[2], bal_small;
-  ~CtxExtra() {
-    pg_idx.release();
-    pg_uv.release();
-    pin_out.release();
-    for (DevBuf *b : {&bal_scan, &bal_out[0], &bal_out[1], &bal_vecs, &bal_cam, &bal_cnt, &bal_slow[0], &bal_slow[1],
-                      &bal_small})
-      b->release();
-    bal_ring.release();
-  }
   GridCache grid;
   uint64_t points_version = 0;
   double pts_bounds[6] = {0, 0, 0, 0, 0, 0};
@@ -304,18 +308,7 @@ struct CtxExtra {
   uint64_t res_candidates = 0;
 };
 
-}  // namespace
-
-// c2b_ctx carries its non-POD extras behind one pointer so the struct in c2b_common.cuh stays plain
-static std::vector<std::pair<c2b_ctx *, CtxExtra *>> &extras() {
-  static std::vector<std::pair<c2b_ctx *, CtxExtra *>> v;
-  return v;
-}
-static CtxExtra *extra_of(c2b_ctx *ctx) {
-  for (auto &e : extras())
-    if (e.first == ctx) return e.second;
-  return nullptr;
-}
+c2b_ctx::~c2b_ctx() = default;
 
 static bool tune(Tunables &t, const char *name, double v) {
   const std::string n(name);
@@ -367,19 +360,20 @@ int c2b_init(int device, c2b_ctx **out) {
   if (prop.major < 10)
     return set_error(C2B_ERR_NO_DEVICE, "device %d is sm_%d%d; this library is built for sm_100a only",
                      device, prop.major, prop.minor);
-  c2b_ctx *ctx = new (std::nothrow) c2b_ctx();
+  // freed with everything built so far by any early return below (the device is current)
+  std::unique_ptr<c2b_ctx> ctx(new (std::nothrow) c2b_ctx());
   if (!ctx) return set_error(C2B_ERR_OOM, "out of host memory");
   ctx->device = device;
   ctx->sm_count = prop.multiProcessorCount;
-  C2B_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
-  for (int i = 0; i < EV_COUNT; ++i) C2B_CUDA(cudaEventCreate(&ctx->ev[i]));
-  C2B_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-  C2B_CUDA(cudaStreamCreateWithFlags(&ctx->aux_stream, cudaStreamNonBlocking));
-  C2B_CUDA(cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
-  C2B_CUDA(cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming));
+  C2B_TRY(ctx->stream.create(cudaStreamNonBlocking));
+  for (int i = 0; i < EV_COUNT; ++i) C2B_TRY(ctx->ev[i].create());
+  C2B_TRY(ctx->copy_stream.create(cudaStreamNonBlocking));
+  C2B_TRY(ctx->aux_stream.create(cudaStreamNonBlocking));
+  C2B_TRY(ctx->ev_fork.create(cudaEventDisableTiming));
+  C2B_TRY(ctx->ev_join.create(cudaEventDisableTiming));
   for (int i = 0; i < 2; ++i) {
-    C2B_CUDA(cudaEventCreateWithFlags(&ctx->ev_ready[i], cudaEventDisableTiming));
-    C2B_CUDA(cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming));
+    C2B_TRY(ctx->ev_ready[i].create(cudaEventDisableTiming));
+    C2B_TRY(ctx->ev_copied[i].create(cudaEventDisableTiming));
   }
   // NUMA node of the device (sysfs), for the pinned staging / result buffers (see PinBuf)
   {
@@ -405,7 +399,7 @@ int c2b_init(int device, c2b_ctx **out) {
     C2B_CUDA(cudaMemcpyToSymbol(g_sc_tab, sc, sizeof sc));
     C2B_CUDA(cudaMemcpyToSymbol(g_ln_tab, ln, sizeof ln));
   }
-  CtxExtra *x = new CtxExtra();
+  ctx->extra = std::make_unique<CtxExtra>();
   {
     struct { const char *env, *name; } hooks[] = {
         {"C2B_PARTS_LOG2", "parts_log2"}, {"C2B_TRILIST_CAP", "trilist_cap"}, {"C2B_MAX_PAIRS", "max_pairs"},
@@ -414,20 +408,19 @@ int c2b_init(int device, c2b_ctx **out) {
         {"C2B_STAGE_THREADS", "stage_threads"}, {"C2B_OPTIMISTIC", "optimistic"}, {"C2B_COLD_STAGED", "cold_staged"},
         {"C2B_BAL_CHUNK_BYTES", "bal_chunk_bytes"}};
     for (auto &h : hooks)
-      if (const char *e = getenv(h.env)) (void)tune(x->tun, h.name, atof(e));
+      if (const char *e = getenv(h.env)) (void)tune(ctx->extra->tun, h.name, atof(e));
   }
-  extras().push_back({ctx, x});
-  *out = ctx;
+  *out = ctx.release();
   return C2B_OK;
 }
 
 int c2b_tune(c2b_ctx *ctx, const char *name, double value) {
   if (!ctx || !name) return set_error(C2B_ERR_INVALID, "c2b_tune: null argument");
   if (!strcmp(name, "reset")) {
-    extra_of(ctx)->tun = Tunables();
+    ctx->extra->tun = Tunables();
     return C2B_OK;
   }
-  if (!tune(extra_of(ctx)->tun, name, value)) return set_error(C2B_ERR_INVALID, "c2b_tune: unknown hook '%s'", name);
+  if (!tune(ctx->extra->tun, name, value)) return set_error(C2B_ERR_INVALID, "c2b_tune: unknown hook '%s'", name);
   return C2B_OK;
 }
 
@@ -437,41 +430,6 @@ void c2b_shutdown(c2b_ctx *ctx) {
   cudaStreamSynchronize(ctx->stream);
   if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
   if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream);
-  DevBuf *bufs[] = {&ctx->cams, &ctx->cam_center, &ctx->pts, &ctx->stage, &ctx->cell_of_pt,
-                    &ctx->cell_start, &ctx->cell_cursor, &ctx->grid_x, &ctx->grid_y, &ctx->grid_z,
-                    &ctx->grid_idx, &ctx->pool_key, &ctx->pool_uv, &ctx->cam_count, &ctx->counters,
-                    &ctx->sort_keys[0], &ctx->sort_keys[1], &ctx->sort_vals[0], &ctx->sort_vals[1],
-                    &ctx->sort_hist, &ctx->scan_tmp[0], &ctx->scan_tmp[1], &ctx->scan_tmp[2],
-                    &ctx->vis_words, &ctx->word_prefix, &ctx->out_offsets[0], &ctx->out_idx[0],
-                    &ctx->out_uv[0], &ctx->out_offsets[1], &ctx->out_idx[1], &ctx->out_uv[1],
-                    &ctx->misc, &ctx->tri_list, &ctx->tri_count, &ctx->pts_aos, &ctx->ev_off,
-                    &ctx->vis_count, &ctx->seg_off, &ctx->scratch_idx, &ctx->plan_rows, &ctx->plan_row_count,
-                    &ctx->nz_cams, &ctx->nz_centers, &ctx->nz_pts, &ctx->nz_uv, &ctx->nz_scratch,
-                    &ctx->cams_all, &ctx->pr_parent, &ctx->pr_size,
-                    &ctx->pr_cam_cnt, &ctx->pr_pt_cnt, &ctx->pr_words, &ctx->pr_prefix, &ctx->pr_small};
-  for (auto *b : bufs) b->release();
-  for (int i = 0; i < 2; ++i)
-    for (DevBuf *b : {&ctx->pr_cams[i], &ctx->pr_pts[i], &ctx->pr_off[i], &ctx->pr_idx[i], &ctx->pr_uv[i]}) b->release();
-  PinBuf *pins[] = {&ctx->pin_in, &ctx->h_offsets, &ctx->h_idx, &ctx->h_uv, &ctx->h_small};
-  for (auto *p : pins) p->release();
-  for (int i = 0; i < EV_COUNT; ++i)
-    if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
-  for (int i = 0; i < 2; ++i) {
-    if (ctx->ev_ready[i]) cudaEventDestroy(ctx->ev_ready[i]);
-    if (ctx->ev_copied[i]) cudaEventDestroy(ctx->ev_copied[i]);
-  }
-  if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-  if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
-  if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
-  if (ctx->ev_join) cudaEventDestroy(ctx->ev_join);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  auto &v = extras();
-  for (size_t i = 0; i < v.size(); ++i)
-    if (v[i].first == ctx) {
-      delete v[i].second;
-      v.erase(v.begin() + i);
-      break;
-    }
   delete ctx;
 }
 
@@ -499,9 +457,7 @@ int c2b_scene_create(c2b_ctx *ctx, const float *xyz, uint64_t nv, const uint32_t
   sc->device = ctx->device;
   int rc = bvh_build(ctx, sc, xyz, nv, keep.data(), keep.size() / 3);
   if (rc != C2B_OK) {
-    sc->nodes.release();
-    sc->tris.release();
-    delete sc;
+    delete sc;  // ctx->device is current
     return rc;
   }
   *out = sc;
@@ -521,8 +477,6 @@ uint64_t c2b_scene_num_nodes(const c2b_scene *scene) { return scene ? scene->n_n
 void c2b_scene_destroy(c2b_scene *scene) {
   if (!scene) return;
   cudaSetDevice(scene->device);
-  scene->nodes.release();
-  scene->tris.release();
   delete scene;
 }
 
@@ -604,7 +558,7 @@ void c2b_vis_options_default(c2b_vis_options *opt) {
 int copy_in(c2b_ctx *ctx, void *d, const void *h, size_t bytes, cudaMemcpyKind kind) {
   cudaStream_t st = ctx->stream;
   if (bytes == 0) return C2B_OK;
-  const int T = extra_of(ctx)->tun.stage_threads;
+  const int T = ctx->extra->tun.stage_threads;
   constexpr size_t CH = 2u << 20;  // pinning the ring itself costs ~1 ms per MB: keep it small
   bool pageable = false;
   if (kind == cudaMemcpyHostToDevice && T > 0 && bytes >= (64u << 10)) {
@@ -640,8 +594,9 @@ int copy_in(c2b_ctx *ctx, void *d, const void *h, size_t bytes, cudaMemcpyKind k
   for (int t = 0; t < nt; ++t)
     workers.emplace_back([=, &err]() {
       cudaError_t e = cudaSetDevice(device);
-      cudaEvent_t ev[2] = {nullptr, nullptr};
-      for (int k = 0; k < 2 && e == cudaSuccess; ++k) e = cudaEventCreateWithFlags(&ev[k], cudaEventDisableTiming);
+      Event ev[2];  // destroyed on this thread, with `device` current
+      for (int k = 0; k < 2 && e == cudaSuccess; ++k)
+        if (ev[k].create(cudaEventDisableTiming) != C2B_OK) e = cudaGetLastError();
       size_t turn = 0;
       for (size_t c = (size_t)t; c < n_chunks && e == cudaSuccess; c += (size_t)nt, ++turn) {
         const int slot = (int)(turn & 1);
@@ -654,10 +609,7 @@ int copy_in(c2b_ctx *ctx, void *d, const void *h, size_t bytes, cudaMemcpyKind k
         if (e == cudaSuccess) e = cudaEventRecord(ev[slot], st);
       }
       for (int k = 0; k < 2; ++k)
-        if (ev[k]) {
-          if (e == cudaSuccess) e = cudaEventSynchronize(ev[k]);
-          cudaEventDestroy(ev[k]);
-        }
+        if (ev[k] && e == cudaSuccess) e = cudaEventSynchronize(ev[k]);
       err[(size_t)t] = e;
     });
   for (auto &w : workers) w.join();
@@ -688,7 +640,7 @@ int c2b_points_commit(c2b_ctx *ctx, uint64_t P) {
   if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_points_commit: null ctx");
   if (P * 24 > ctx->pts_aos.cap) return set_error(C2B_ERR_INVALID, "c2b_points_commit: %llu points exceed the buffer", (unsigned long long)P);
   if (P >= 0xffffffffull) return set_error(C2B_ERR_INVALID, "too many points (%llu)", (unsigned long long)P);
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   C2B_CUDA(cudaSetDevice(ctx->device));
   ctx->P = P;
   x->points_version++;
@@ -732,14 +684,14 @@ int c2b_upload_points_device(c2b_ctx *ctx, const double *d_pts, uint64_t P) {
 
 int c2b_drop_point_grid(c2b_ctx *ctx) {
   if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_drop_point_grid: null ctx");
-  extra_of(ctx)->grid.valid = false;
+  ctx->extra->grid.valid = false;
   return C2B_OK;
 }
 
 int c2b_upload_cameras(c2b_ctx *ctx, const double *cams, uint64_t C) {
   if (!ctx || (C && !cams)) return set_error(C2B_ERR_INVALID, "c2b_upload_cameras: null argument");
   if (C >= 0xffffffffull) return set_error(C2B_ERR_INVALID, "too many cameras (%llu)", (unsigned long long)C);
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   C2B_CUDA(cudaSetDevice(ctx->device));
   ctx->C = C;
   x->have_cameras = true;
@@ -758,7 +710,7 @@ int c2b_upload_cameras(c2b_ctx *ctx, const double *cams, uint64_t C) {
 // cameras [first, first + count) of the call's device copy (ctx->cams_all) become the resident cameras:
 // what c2b_upload_cameras does for a batch, without touching host memory again
 static int select_cameras(c2b_ctx *ctx, uint64_t first, uint64_t count) {
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   ctx->C = count;
   x->have_cameras = true;
   x->have_result = false;
@@ -1233,14 +1185,14 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
 int c2b_visibility_graph_resident(c2b_ctx *ctx, const c2b_scene *scene, double max_dist,
                                   const c2b_vis_options *opt_in, c2b_obs *stats) {
   const int rc = visibility_resident_impl(ctx, scene, max_dist, opt_in, stats);
-  if (ctx) extra_of(ctx)->host_call_last = false;
+  if (ctx) ctx->extra->host_call_last = false;
   return rc == ERR_TOO_LARGE ? C2B_ERR_INVALID : rc;
 }
 
 static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double max_dist,
                                     const c2b_vis_options *opt_in, c2b_obs *stats) {
   if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_visibility_graph_resident: null ctx");
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (!x->have_points || !x->have_cameras)
     return set_error(C2B_ERR_INVALID, "upload cameras and points first");
   c2b_vis_options opt;
@@ -1434,7 +1386,7 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
 
 int c2b_download_obs(c2b_ctx *ctx, c2b_obs *out) {
   if (!ctx || !out) return set_error(C2B_ERR_INVALID, "c2b_download_obs: null argument");
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (!x->have_result) return set_error(C2B_ERR_INVALID, "no resident result to download");
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
@@ -1473,7 +1425,7 @@ __global__ void k_add_u64(uint64_t *v, uint64_t n, uint64_t add) {
 int c2b_download_obs_into(c2b_ctx *ctx, uint64_t obs_base, uint64_t *offsets_dst, uint32_t *idx_dst, double *uv_dst,
                           int with_end, float *ms_d2h) {
   if (!ctx || !offsets_dst) return set_error(C2B_ERR_INVALID, "c2b_download_obs_into: null argument");
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (!x->have_result) return set_error(C2B_ERR_INVALID, "no resident result to download");
   const uint64_t C = ctx->out_C, O = ctx->out_O;
   if (O && (!idx_dst || !uv_dst)) return set_error(C2B_ERR_INVALID, "c2b_download_obs_into: null result array");
@@ -1515,8 +1467,7 @@ int grow_pinned(c2b_ctx *ctx, PinBuf &b, size_t need, size_t used) {
   nb.node = b.node;
   C2B_TRY(nb.ensure(need + need / 16));
   if (used) memcpy(nb.p, b.p, used);
-  b.release();
-  b = nb;
+  b = std::move(nb);
   return C2B_OK;
 }
 }  // namespace
@@ -1527,7 +1478,7 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
   if (!ctx || !out) return set_error(C2B_ERR_INVALID, "c2b_visibility_graph: null argument");
   if (C && !cams) return set_error(C2B_ERR_INVALID, "c2b_visibility_graph: null camera array");
   C2B_CUDA(cudaSetDevice(ctx->device));
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   // pts == NULL: use the points already resident on the device (c2b_upload_points[_device])
   const bool resident_pts = P && !pts;
   if (resident_pts && !(x->have_points && ctx->P == P))
@@ -1565,11 +1516,11 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
   }
   const uint64_t n_batches = bounds.size() - 1;
 
-  cudaEvent_t u0, u1, d0, d1;
-  C2B_CUDA(cudaEventCreate(&u0));
-  C2B_CUDA(cudaEventCreate(&u1));
-  C2B_CUDA(cudaEventCreate(&d0));
-  C2B_CUDA(cudaEventCreate(&d1));
+  Event u0, u1, d0, d1;
+  C2B_TRY(u0.create());
+  C2B_TRY(u1.create());
+  C2B_TRY(d0.create());
+  C2B_TRY(d1.create());
   c2b_obs acc;
   memset(&acc, 0, sizeof acc);
   int rc = C2B_OK;
@@ -1653,8 +1604,7 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
             PageBuf bigger;
             C2B_TRY(bigger.ensure_fresh(2 * std::max<size_t>(need, 1) * unit));
             if (obs_base) memcpy(bigger.p, pb->p, obs_base * unit);
-            pb->release();
-            *pb = bigger;
+            *pb = std::move(bigger);
           }
         }
         if (!copy_started) {
@@ -1703,10 +1653,6 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
   };
   rc = run();
   x->grid_locked = false;
-  cudaEventDestroy(u0);
-  cudaEventDestroy(u1);
-  cudaEventDestroy(d0);
-  cudaEventDestroy(d1);
   ctx->out_sel = 0;
   x->have_result = false;  // the resident state now holds the last batch only
   x->host_call_last = true;
@@ -1744,7 +1690,7 @@ void c2b_obs_free(c2b_ctx *ctx, c2b_obs *obs) {
 
 int c2b_reprojection_error_resident(c2b_ctx *ctx, double norm, double *out) {
   if (!ctx || !out) return set_error(C2B_ERR_INVALID, "c2b_reprojection_error_resident: null argument");
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (!x->have_result) return set_error(C2B_ERR_INVALID, "no resident result");
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
@@ -1782,9 +1728,9 @@ struct NoiseView {
 // device time of the last noise call: [0] upload, [1] statistics + kernels, [2] download
 struct NoiseTimer {
   c2b_ctx *ctx;
-  cudaEvent_t ev[4] = {};
+  Event ev[4];
   explicit NoiseTimer(c2b_ctx *c) : ctx(c) {
-    for (auto &e : ev) cudaEventCreate(&e);
+    for (auto &e : ev) (void)e.create();
     cudaEventRecord(ev[0], ctx->stream);
   }
   void mark(int k) { cudaEventRecord(ev[k], ctx->stream); }
@@ -1794,9 +1740,6 @@ struct NoiseTimer {
       if (cudaEventElapsedTime(&t, ev[k], ev[k + 1]) != cudaSuccess) (void)cudaGetLastError();
       ctx->noise_ms[k] = t;
     }
-  }
-  ~NoiseTimer() {
-    for (auto &e : ev) cudaEventDestroy(e);
   }
 };
 
@@ -1869,7 +1812,7 @@ int noise_upload(c2b_ctx *ctx, NoiseView &v, const double *cams, uint64_t C, con
 
 // the resident problem as a NoiseView (cameras + points of the last uploads, (u, v) of the last resident pass)
 int resident_view(c2b_ctx *ctx, NoiseView &v, const char *who) {
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (!x->have_points || !x->have_cameras) return set_error(C2B_ERR_INVALID, "%s: upload cameras and points first", who);
   v.cams = ctx->cams.as<double>();
   v.centers = ctx->cam_center.as<double>();
@@ -1889,7 +1832,7 @@ int resident_refresh(c2b_ctx *ctx, bool cams_moved, bool pts_moved) {
     C2B_KERNEL_CHECK();
   }
   if (pts_moved) {
-    CtxExtra *x = extra_of(ctx);
+    CtxExtra *x = ctx->extra.get();
     const bool had = x->have_result;
     C2B_TRY(c2b_points_commit(ctx, ctx->P));
     x->have_result = had;  // the CSR is still the graph of this problem
@@ -2027,17 +1970,17 @@ int c2b_add_noise(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64_t 
   // The observations (16 B each way, by far the largest array) stream through the GPU in chunks on the copy
   // stream while cameras and points are handled on the main one: PCIe is full duplex, so chunk k's download
   // overlaps chunk k+1's upload and the call costs about one direction of the transfer, not two.
-  cudaEvent_t obs_done = nullptr;
+  Event obs_done;
   if (O) {
     const uint64_t chunk = std::max<uint64_t>(1u << 20, (O + 15) / 16);
     C2B_TRY(ctx->nz_uv.ensure(std::min(O, 2 * chunk) * 16));
     double2 *buf = ctx->nz_uv.as<double2>();
-    cudaEvent_t slot_free[2] = {nullptr, nullptr}, up[2] = {nullptr, nullptr};
+    Event slot_free[2], up[2];
     for (int k = 0; k < 2; ++k) {
-      C2B_CUDA(cudaEventCreateWithFlags(&slot_free[k], cudaEventDisableTiming));
-      C2B_CUDA(cudaEventCreateWithFlags(&up[k], cudaEventDisableTiming));
+      C2B_TRY(slot_free[k].create(cudaEventDisableTiming));
+      C2B_TRY(up[k].create(cudaEventDisableTiming));
     }
-    C2B_CUDA(cudaEventCreateWithFlags(&obs_done, cudaEventDisableTiming));
+    C2B_TRY(obs_done.create(cudaEventDisableTiming));
     // uploads + kernels on the aux stream, downloads on the copy stream; two slots
     cudaStream_t ax = ctx->aux_stream;
     uint64_t k = 0;
@@ -2055,10 +1998,6 @@ int c2b_add_noise(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64_t 
       C2B_CUDA(cudaEventRecord(slot_free[slot], cs));
     }
     C2B_CUDA(cudaEventRecord(obs_done, cs));
-    for (int q = 0; q < 2; ++q) {
-      cudaEventDestroy(slot_free[q]);
-      cudaEventDestroy(up[q]);
-    }
   }
   C2B_TRY(noise_upload(ctx, v, cams, C, pts, P));
   tm.mark(1);
@@ -2066,10 +2005,7 @@ int c2b_add_noise(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64_t 
   tm.mark(2);
   if (C) C2B_CUDA(cudaMemcpyAsync(cams, v.cams, C * 120, cudaMemcpyDeviceToHost, st));
   if (P && point_std != 0.0) C2B_CUDA(cudaMemcpyAsync(pts, v.pts, P * 24, cudaMemcpyDeviceToHost, st));
-  if (obs_done) {
-    C2B_CUDA(cudaStreamWaitEvent(st, obs_done, 0));
-    cudaEventDestroy(obs_done);
-  }
+  if (obs_done) C2B_CUDA(cudaStreamWaitEvent(st, obs_done, 0));
   tm.mark(3);
   C2B_CUDA(cudaStreamSynchronize(st));
   tm.finish();
@@ -2247,79 +2183,72 @@ int c2b_generate_world_points_uniform(c2b_ctx *ctx, const float *xyz, uint64_t n
     }
   }
   DevBuf d_tv, d_cdf, d_cs, d_cen, d_cand, d_keep, d_rank, d_out, d_small;
-  auto cleanup = [&]() {
-    for (DevBuf *b : {&d_tv, &d_cdf, &d_cs, &d_cen, &d_cand, &d_keep, &d_rank, &d_out, &d_small}) b->release();
-  };
-  int rc = [&]() -> int {
-    C2B_TRY(d_tv.ensure(tv.size() * 16));
-    C2B_TRY(d_cdf.ensure(nt * 8));
-    C2B_TRY(d_cs.ensure((cells + 1) * 4));
-    C2B_TRY(d_cen.ensure(C * 24));
-    C2B_TRY(d_out.ensure(num_points * 24));
-    C2B_TRY(d_small.ensure(64));
-    C2B_CUDA(cudaMemcpyAsync(d_tv.p, tv.data(), tv.size() * 16, cudaMemcpyHostToDevice, st));
-    C2B_CUDA(cudaMemcpyAsync(d_cdf.p, cdf.data(), nt * 8, cudaMemcpyHostToDevice, st));
-    C2B_CUDA(cudaMemcpyAsync(d_cs.p, cell_start.data(), (cells + 1) * 4, cudaMemcpyHostToDevice, st));
-    C2B_CUDA(cudaMemcpyAsync(d_cen.p, cen_sorted.data(), C * 24, cudaMemcpyHostToDevice, st));
-    SampleArgs a;
-    a.tri_v = d_tv.as<float4>();
-    a.cdf = d_cdf.as<double>();
-    a.nt = nt;
-    a.total = run;
-    a.g = g;
-    a.cell_start = d_cs.as<uint32_t>();
-    a.cen = d_cen.as<double>();
-    a.max_d2 = max_dist * max_dist;
-    a.seed = seed;
-    const uint64_t threshold = 10 * num_points;
-    uint64_t got = 0, consumed = 0;
-    while (got < num_points) {
-      const uint64_t want = num_points - got;
-      const uint64_t n = std::min<uint64_t>(want + want / 4 + 1024, 1ull << 26);
-      C2B_TRY(d_cand.ensure(n * 24));
-      C2B_TRY(d_keep.ensure((n + 1) * 4));
-      C2B_TRY(d_rank.ensure((n + 1) * 4));
-      a.first = consumed;
-      a.n = n;
-      a.cand = d_cand.as<double>();
-      a.keep = d_keep.as<uint32_t>();
-      C2B_CUDA(cudaMemsetAsync(d_small.p, 0, 64, st));
-      k_sample_points<<<blocks_for(n, 256), 256, 0, st>>>(a);
-      C2B_KERNEL_CHECK();
-      uint32_t *d_total = d_small.as<uint32_t>() + 4;
-      C2B_TRY(exclusive_scan_u32(st, a.keep, d_rank.as<uint32_t>(), n, d_total, ctx->scan_tmp));
-      k_sample_compact<<<blocks_for(n, 256), 256, 0, st>>>(a.cand, a.keep, d_rank.as<uint32_t>(), n, got, num_points,
-                                                           d_out.as<double>(), d_small.as<unsigned long long>());
-      C2B_KERNEL_CHECK();
-      unsigned long long h[4];
-      C2B_CUDA(cudaMemcpyAsync(h, d_small.p, 32, cudaMemcpyDeviceToHost, st));
-      C2B_CUDA(cudaStreamSynchronize(st));
-      uint32_t accepted;
-      memcpy(&accepted, reinterpret_cast<const char *>(h) + 16, 4);
-      if (got + accepted >= num_points) {
-        // h[0] = round-local index of the candidate that completed the request
-        const uint64_t used = consumed + h[0] + 1;
-        if (used - num_points >= threshold)
-          return set_error(C2B_ERR_INVALID, "Failed to generate enough points. %llu successes, %llu failures, %llu "
-                                            "requested points.", (unsigned long long)num_points,
-                           (unsigned long long)(used - num_points), (unsigned long long)num_points);
-        got = num_points;
-        break;
-      }
-      got += accepted;
-      consumed += n;
-      if (consumed - got >= threshold)
-        return set_error(C2B_ERR_INVALID, "Failed to generate enough points. %llu successes, %llu failures, %llu "
-                                          "requested points.", (unsigned long long)got,
-                         (unsigned long long)(consumed - got), (unsigned long long)num_points);
-    }
-    C2B_CUDA(cudaMemcpyAsync(pts_out, d_out.p, num_points * 24, cudaMemcpyDeviceToHost, st));
+  C2B_TRY(d_tv.ensure(tv.size() * 16));
+  C2B_TRY(d_cdf.ensure(nt * 8));
+  C2B_TRY(d_cs.ensure((cells + 1) * 4));
+  C2B_TRY(d_cen.ensure(C * 24));
+  C2B_TRY(d_out.ensure(num_points * 24));
+  C2B_TRY(d_small.ensure(64));
+  C2B_CUDA(cudaMemcpyAsync(d_tv.p, tv.data(), tv.size() * 16, cudaMemcpyHostToDevice, st));
+  C2B_CUDA(cudaMemcpyAsync(d_cdf.p, cdf.data(), nt * 8, cudaMemcpyHostToDevice, st));
+  C2B_CUDA(cudaMemcpyAsync(d_cs.p, cell_start.data(), (cells + 1) * 4, cudaMemcpyHostToDevice, st));
+  C2B_CUDA(cudaMemcpyAsync(d_cen.p, cen_sorted.data(), C * 24, cudaMemcpyHostToDevice, st));
+  SampleArgs a;
+  a.tri_v = d_tv.as<float4>();
+  a.cdf = d_cdf.as<double>();
+  a.nt = nt;
+  a.total = run;
+  a.g = g;
+  a.cell_start = d_cs.as<uint32_t>();
+  a.cen = d_cen.as<double>();
+  a.max_d2 = max_dist * max_dist;
+  a.seed = seed;
+  const uint64_t threshold = 10 * num_points;
+  uint64_t got = 0, consumed = 0;
+  while (got < num_points) {
+    const uint64_t want = num_points - got;
+    const uint64_t n = std::min<uint64_t>(want + want / 4 + 1024, 1ull << 26);
+    C2B_TRY(d_cand.ensure(n * 24));
+    C2B_TRY(d_keep.ensure((n + 1) * 4));
+    C2B_TRY(d_rank.ensure((n + 1) * 4));
+    a.first = consumed;
+    a.n = n;
+    a.cand = d_cand.as<double>();
+    a.keep = d_keep.as<uint32_t>();
+    C2B_CUDA(cudaMemsetAsync(d_small.p, 0, 64, st));
+    k_sample_points<<<blocks_for(n, 256), 256, 0, st>>>(a);
+    C2B_KERNEL_CHECK();
+    uint32_t *d_total = d_small.as<uint32_t>() + 4;
+    C2B_TRY(exclusive_scan_u32(st, a.keep, d_rank.as<uint32_t>(), n, d_total, ctx->scan_tmp));
+    k_sample_compact<<<blocks_for(n, 256), 256, 0, st>>>(a.cand, a.keep, d_rank.as<uint32_t>(), n, got, num_points,
+                                                         d_out.as<double>(), d_small.as<unsigned long long>());
+    C2B_KERNEL_CHECK();
+    unsigned long long h[4];
+    C2B_CUDA(cudaMemcpyAsync(h, d_small.p, 32, cudaMemcpyDeviceToHost, st));
     C2B_CUDA(cudaStreamSynchronize(st));
-    return C2B_OK;
-  }();
-  cleanup();
-  if (rc == C2B_OK) *n_out = num_points;
-  return rc;
+    uint32_t accepted;
+    memcpy(&accepted, reinterpret_cast<const char *>(h) + 16, 4);
+    if (got + accepted >= num_points) {
+      // h[0] = round-local index of the candidate that completed the request
+      const uint64_t used = consumed + h[0] + 1;
+      if (used - num_points >= threshold)
+        return set_error(C2B_ERR_INVALID, "Failed to generate enough points. %llu successes, %llu failures, %llu "
+                                          "requested points.", (unsigned long long)num_points,
+                         (unsigned long long)(used - num_points), (unsigned long long)num_points);
+      got = num_points;
+      break;
+    }
+    got += accepted;
+    consumed += n;
+    if (consumed - got >= threshold)
+      return set_error(C2B_ERR_INVALID, "Failed to generate enough points. %llu successes, %llu failures, %llu "
+                                        "requested points.", (unsigned long long)got,
+                       (unsigned long long)(consumed - got), (unsigned long long)num_points);
+  }
+  C2B_CUDA(cudaMemcpyAsync(pts_out, d_out.p, num_points * 24, cudaMemcpyDeviceToHost, st));
+  C2B_CUDA(cudaStreamSynchronize(st));
+  *n_out = num_points;
+  return C2B_OK;
 }
 
 int c2b_probe_fp64(c2b_ctx *ctx, double *dfma_per_s) {
@@ -2328,9 +2257,9 @@ int c2b_probe_fp64(c2b_ctx *ctx, double *dfma_per_s) {
   C2B_TRY(ctx->misc.ensure(8));
   cudaStream_t st = ctx->stream;
   const int blocks = ctx->sm_count * 8, threads = 256, iters = 4096;
-  cudaEvent_t e0, e1;
-  C2B_CUDA(cudaEventCreate(&e0));
-  C2B_CUDA(cudaEventCreate(&e1));
+  Event e0, e1;
+  C2B_TRY(e0.create());
+  C2B_TRY(e1.create());
   float best = 0.0f;
   for (int rep = 0; rep < 4; ++rep) {  // first repetition warms up
     C2B_CUDA(cudaEventRecord(e0, st));
@@ -2342,8 +2271,6 @@ int c2b_probe_fp64(c2b_ctx *ctx, double *dfma_per_s) {
     C2B_CUDA(cudaEventElapsedTime(&ms, e0, e1));
     if (rep && (best == 0.0f || ms < best)) best = ms;
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
   *dfma_per_s = (double)blocks * threads * iters * PROBE_CHAINS / (best * 1e-3);
   return C2B_OK;
 }
@@ -2360,20 +2287,6 @@ int c2b_mean_std(c2b_ctx *ctx, const double *cams, uint64_t C, const double *pts
 }
 
 // ---- BAProblem::cull: LCC + remove_singletons to a fixed point (c2b_graph_cull.cuh) -------------------------
-namespace {
-struct CullEvents {  // timing events of one cull call
-  cudaEvent_t e[4] = {};
-  int create() {
-    for (auto &x : e) C2B_CUDA(cudaEventCreate(&x));
-    return C2B_OK;
-  }
-  ~CullEvents() {
-    for (auto x : e)
-      if (x) cudaEventDestroy(x);
-  }
-};
-}  // namespace
-
 static int cull_limits(uint64_t C, uint64_t P, uint64_t O, const char *who) {
   if (C + P >= 0xffffffffull)
     return set_error(C2B_ERR_INVALID, "%s: %llu cameras + %llu points exceed the 32-bit entity ids (C + P < 2^32 - 1)",
@@ -2401,9 +2314,8 @@ int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64
   C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
   C2B_TRY(ctx->pr_small.ensure(64));
   C2B_TRY(ctx->h_small.ensure(256));
-  CullEvents events;
-  C2B_TRY(events.create());
-  cudaEvent_t *ev = events.e;
+  Event ev[4];  // timing
+  for (auto &e : ev) C2B_TRY(e.create());
   int rc = [&]() -> int {
     C2B_CUDA(cudaEventRecord(ev[0], st));
     if (C) C2B_TRY(copy_in(ctx, ctx->pr_cams[0].p, cams, C * 120, cudaMemcpyHostToDevice));
@@ -2460,7 +2372,7 @@ int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64
 
 int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
   if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: null ctx");
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (x->host_call_last)
     return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: the resident CSR is the last camera batch of the "
                                       "host-buffer c2b_visibility_graph, not the graph of an uploaded problem; run "
@@ -2477,9 +2389,8 @@ int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
   PruneSet sets[2] = {{&ctx->cams, &ctx->pts_aos, &ctx->out_offsets[sel], &ctx->out_idx[sel], &ctx->out_uv[sel]},
                       {&ctx->pr_cams[1], &ctx->pr_pts[1], &ctx->out_offsets[sel ^ 1], &ctx->out_idx[sel ^ 1],
                        &ctx->out_uv[sel ^ 1]}};
-  CullEvents events;
-  C2B_TRY(events.create());
-  cudaEvent_t *ev = events.e;
+  Event ev[4];  // timing
+  for (auto &e : ev) C2B_TRY(e.create());
   int cur = 0;
   uint32_t it = 0;
   int rc = [&]() -> int {
@@ -2528,20 +2439,6 @@ namespace {
 constexpr int BAL_RING = 3;                 // pinned chunk slots: D2H of chunk k while chunk k-1 is written
 constexpr uint32_t BAL_WINDOW = 1u << 20;   // lines per length pass: 2^20 lines of <= 2952 bytes keep the u32 scan exact
 
-struct BalEvents {  // per ring slot: encode start / end (ctx stream), copy start / end (copy stream)
-  cudaEvent_t e[BAL_RING][4] = {};
-  int create() {
-    for (auto &s : e)
-      for (auto &x : s) C2B_CUDA(cudaEventCreate(&x));
-    return C2B_OK;
-  }
-  ~BalEvents() {
-    for (auto &s : e)
-      for (auto x : s)
-        if (x) cudaEventDestroy(x);
-  }
-};
-
 // the camera 9-vectors of C records (host memory) -> x->bal_vecs
 int bal_upload_vecs(c2b_ctx *ctx, CtxExtra *x, const double *cams, uint64_t C) {
   C2B_TRY(x->bal_vecs.ensure(std::max<uint64_t>(C, 1) * 72));
@@ -2557,7 +2454,7 @@ int bal_upload_vecs(c2b_ctx *ctx, CtxExtra *x, const double *cams, uint64_t C) {
 // the ctx stream into device buffer k % 2, its copy on the copy stream into ring slot k % 3, then write(2) on a
 // writer thread; the host waits only for the chunk's line count (text) and for a free ring slot.
 int bal_stream(c2b_ctx *ctx, const char *path, int format, const BalView &v, c2b_bal_stats *out) {
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   const uint64_t B = x->tun.bal_chunk_bytes;
   const bool text = format == C2B_BAL_TEXT;
   cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
@@ -2569,9 +2466,9 @@ int bal_stream(c2b_ctx *ctx, const char *path, int format, const BalView &v, c2b
     C2B_TRY(x->bal_scan.ensure((size_t)(BAL_WINDOW + 1) * 4));
     C2B_TRY(ctx->h_small.ensure(256));
   }
-  BalEvents events;
-  C2B_TRY(events.create());
-  auto &ev = events.e;
+  Event ev[BAL_RING][4];  // per ring slot: encode start / end (ctx stream), copy start / end (copy stream)
+  for (auto &slot : ev)
+    for (auto &e : slot) C2B_TRY(e.create());
   const int fd = open(path, O_WRONLY | O_CREAT | O_TRUNC | O_CLOEXEC, 0666);
   if (fd < 0) return set_error(C2B_ERR_IO, "cannot create %s: %s", path, strerror(errno));
   struct stat sb;
@@ -2730,7 +2627,7 @@ int c2b_write_bal(c2b_ctx *ctx, const char *path, int format, const double *cams
   if (O && (!point_idx || !uv)) return set_error(C2B_ERR_INVALID, "c2b_write_bal: null observation array");
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   // the cull's host-entry buffers (set 0): never the resident problem
   C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
   C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
@@ -2771,7 +2668,7 @@ int c2b_write_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_s
   if (!ctx || !path) return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: null argument");
   if (format != C2B_BAL_TEXT && format != C2B_BAL_BINARY)
     return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: unknown format %d", format);
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   if (x->host_call_last)
     return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: the resident CSR is the last camera batch of the "
                                       "host-buffer c2b_visibility_graph, not the graph of an uploaded problem; run "
@@ -2817,7 +2714,7 @@ struct BalReadState {
   int fd;
   uint64_t size, B;
   uint64_t C = 0, P = 0, O = 0;
-  BalEvents events;
+  Event ev[BAL_RING][4] = {};  // per ring slot: H2D start / end (copy stream), parse start / end (ctx stream)
   double ms_read = 0;
   float ms_h2d = 0, ms_parse = 0;
   uint64_t chunks = 0, bytes = 0, slow = 0;
@@ -2827,8 +2724,8 @@ struct BalReadState {
   // the device times of the chunk in ring slot `slot` (its parse has finished)
   void add_times(int slot) {
     float a = 0, b = 0;
-    cudaEventElapsedTime(&a, events.e[slot][0], events.e[slot][1]);
-    cudaEventElapsedTime(&b, events.e[slot][2], events.e[slot][3]);
+    cudaEventElapsedTime(&a, ev[slot][0], ev[slot][1]);
+    cudaEventElapsedTime(&b, ev[slot][2], ev[slot][3]);
     ms_h2d += a;
     ms_parse += b;
   }
@@ -2910,7 +2807,7 @@ int bal_read_text(BalReadState &s) {
   cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
   const uint64_t B = s.B;
   char *ring = x->bal_ring.as<char>();
-  auto &ev = s.events.e;
+  auto &ev = s.ev;
   // the header, on the host, from the first chunk
   const int64_t got0 = bal_pread(s.fd, ring, std::min(B, s.size), 0, s.ms_read);
   if (got0 < 0) return set_error(C2B_ERR_IO, "cannot read %s: %s", s.path, strerror(errno));
@@ -3090,7 +2987,7 @@ int bal_read_binary(BalReadState &s) {
   cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
   const uint64_t B = s.B, W = B / 8;
   char *ring = x->bal_ring.as<char>();
-  auto &ev = s.events.e;
+  auto &ev = s.ev;
   unsigned char h24[24];
   const int64_t g = bal_pread(s.fd, reinterpret_cast<char *>(h24), 24, 0, s.ms_read);
   if (g < 0) return set_error(C2B_ERR_IO, "cannot read %s: %s", s.path, strerror(errno));
@@ -3188,7 +3085,7 @@ int c2b_read_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_re
   if (!ctx || !path) return set_error(C2B_ERR_INVALID, "c2b_read_bal_resident: null argument");
   if (format != C2B_BAL_TEXT && format != C2B_BAL_BINARY)
     return set_error(C2B_ERR_INVALID, "c2b_read_bal_resident: unknown format %d", format);
-  CtxExtra *x = extra_of(ctx);
+  CtxExtra *x = ctx->extra.get();
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   // whatever happens below, the previous resident problem is replaced
@@ -3202,7 +3099,8 @@ int c2b_read_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_re
     struct stat sb;
     if (fstat(s.fd, &sb) != 0 || !S_ISREG(sb.st_mode)) return set_error(C2B_ERR_IO, "%s is not a regular file", path);
     s.size = (uint64_t)sb.st_size;
-    C2B_TRY(s.events.create());
+    for (auto &slot : s.ev)
+      for (auto &e : slot) C2B_TRY(e.create());
     x->bal_ring.node = ctx->numa_node;
     C2B_TRY(x->bal_ring.ensure(BAL_RING * s.B));
     C2B_TRY(ctx->h_small.ensure(256));

@@ -243,26 +243,6 @@ struct BvhScratch {
   DevBuf xyz, tri, bounds, keys[2], vals[2], hist, left, right, first, last, par_i, par_l, leaf_box,
       int_box, visit;
   DevBuf scan_tmp[3];
-  void release() {
-    xyz.release();
-    tri.release();
-    bounds.release();
-    keys[0].release();
-    keys[1].release();
-    vals[0].release();
-    vals[1].release();
-    hist.release();
-    left.release();
-    right.release();
-    first.release();
-    last.release();
-    par_i.release();
-    par_l.release();
-    leaf_box.release();
-    int_box.release();
-    visit.release();
-    for (auto &t : scan_tmp) t.release();
-  }
 };
 
 // h_tri holds only valid (non-degenerate, in-range) triples.
@@ -274,76 +254,72 @@ inline int bvh_build(c2b_ctx *ctx, c2b_scene *sc, const float *h_xyz, uint64_t n
   if (nt == 0) return C2B_OK;
   if (nt >= 0x7fffffffull / 2) return set_error(C2B_ERR_INVALID, "too many triangles (%llu)", (unsigned long long)nt);
   BvhScratch s;
-  int rc = [&]() -> int {
-    C2B_TRY(s.xyz.ensure(nv * 12));
-    C2B_TRY(s.tri.ensure(nt * 12));
-    C2B_CUDA(cudaMemcpyAsync(s.xyz.p, h_xyz, nv * 12, cudaMemcpyHostToDevice, st));
-    C2B_CUDA(cudaMemcpyAsync(s.tri.p, h_tri, nt * 12, cudaMemcpyHostToDevice, st));
-    C2B_TRY(s.bounds.ensure(24));
-    uint32_t init[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
-    C2B_CUDA(cudaMemcpyAsync(s.bounds.p, init, 24, cudaMemcpyHostToDevice, st));
-    int nb = (int)((nt + 255) / 256);
-    int nb_red = nb < 4 * ctx->sm_count ? nb : 4 * ctx->sm_count;
-    k_bvh_bounds<<<nb_red, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), nt,
-                                         s.bounds.as<uint32_t>());
+  C2B_TRY(s.xyz.ensure(nv * 12));
+  C2B_TRY(s.tri.ensure(nt * 12));
+  C2B_CUDA(cudaMemcpyAsync(s.xyz.p, h_xyz, nv * 12, cudaMemcpyHostToDevice, st));
+  C2B_CUDA(cudaMemcpyAsync(s.tri.p, h_tri, nt * 12, cudaMemcpyHostToDevice, st));
+  C2B_TRY(s.bounds.ensure(24));
+  uint32_t init[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
+  C2B_CUDA(cudaMemcpyAsync(s.bounds.p, init, 24, cudaMemcpyHostToDevice, st));
+  int nb = (int)((nt + 255) / 256);
+  int nb_red = nb < 4 * ctx->sm_count ? nb : 4 * ctx->sm_count;
+  k_bvh_bounds<<<nb_red, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), nt,
+                                       s.bounds.as<uint32_t>());
+  C2B_KERNEL_CHECK();
+  for (int b = 0; b < 2; ++b) {
+    C2B_TRY(s.keys[b].ensure(nt * 8));
+    C2B_TRY(s.vals[b].ensure(nt * 4));
+  }
+  k_bvh_morton<<<nb, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), nt,
+                                   s.bounds.as<uint32_t>(), s.keys[0].as<uint64_t>(),
+                                   s.vals[0].as<uint32_t>());
+  C2B_KERNEL_CHECK();
+  uint64_t *keys[2] = {s.keys[0].as<uint64_t>(), s.keys[1].as<uint64_t>()};
+  uint32_t *vals[2] = {s.vals[0].as<uint32_t>(), s.vals[1].as<uint32_t>()};
+  int res = 0;
+  C2B_TRY(radix_sort_pairs(st, keys, vals, nt, 63, s.hist, s.scan_tmp, &res));
+  C2B_TRY(sc->tris.ensure(nt * 48));
+  C2B_TRY(sc->nodes.ensure(sc->n_nodes * 32));
+  C2B_TRY(s.leaf_box.ensure(nt * 24));
+  uint64_t ni = nt - 1;
+  if (ni) {
+    C2B_TRY(s.left.ensure(ni * 4));
+    C2B_TRY(s.right.ensure(ni * 4));
+    C2B_TRY(s.first.ensure(ni * 4));
+    C2B_TRY(s.last.ensure(ni * 4));
+    C2B_TRY(s.par_i.ensure(ni * 4));
+    C2B_TRY(s.int_box.ensure(ni * 24));
+    C2B_TRY(s.visit.ensure(ni * 4));
+    C2B_CUDA(cudaMemsetAsync(s.visit.p, 0, ni * 4, st));
+    C2B_TRY(s.par_l.ensure(nt * 4));
+    k_bvh_karras<<<(int)((ni + 255) / 256), 256, 0, st>>>(
+        keys[res], (int64_t)nt, s.left.as<uint32_t>(), s.right.as<uint32_t>(),
+        s.first.as<uint32_t>(), s.last.as<uint32_t>(), s.par_i.as<uint32_t>(),
+        s.par_l.as<uint32_t>());
     C2B_KERNEL_CHECK();
-    for (int b = 0; b < 2; ++b) {
-      C2B_TRY(s.keys[b].ensure(nt * 8));
-      C2B_TRY(s.vals[b].ensure(nt * 4));
-    }
-    k_bvh_morton<<<nb, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), nt,
-                                     s.bounds.as<uint32_t>(), s.keys[0].as<uint64_t>(),
-                                     s.vals[0].as<uint32_t>());
-    C2B_KERNEL_CHECK();
-    uint64_t *keys[2] = {s.keys[0].as<uint64_t>(), s.keys[1].as<uint64_t>()};
-    uint32_t *vals[2] = {s.vals[0].as<uint32_t>(), s.vals[1].as<uint32_t>()};
-    int res = 0;
-    C2B_TRY(radix_sort_pairs(st, keys, vals, nt, 63, s.hist, s.scan_tmp, &res));
-    C2B_TRY(sc->tris.ensure(nt * 48));
-    C2B_TRY(sc->nodes.ensure(sc->n_nodes * 32));
-    C2B_TRY(s.leaf_box.ensure(nt * 24));
-    uint64_t ni = nt - 1;
-    if (ni) {
-      C2B_TRY(s.left.ensure(ni * 4));
-      C2B_TRY(s.right.ensure(ni * 4));
-      C2B_TRY(s.first.ensure(ni * 4));
-      C2B_TRY(s.last.ensure(ni * 4));
-      C2B_TRY(s.par_i.ensure(ni * 4));
-      C2B_TRY(s.int_box.ensure(ni * 24));
-      C2B_TRY(s.visit.ensure(ni * 4));
-      C2B_CUDA(cudaMemsetAsync(s.visit.p, 0, ni * 4, st));
-      C2B_TRY(s.par_l.ensure(nt * 4));
-      k_bvh_karras<<<(int)((ni + 255) / 256), 256, 0, st>>>(
-          keys[res], (int64_t)nt, s.left.as<uint32_t>(), s.right.as<uint32_t>(),
-          s.first.as<uint32_t>(), s.last.as<uint32_t>(), s.par_i.as<uint32_t>(),
-          s.par_l.as<uint32_t>());
-      C2B_KERNEL_CHECK();
-    }
-    k_bvh_refit<<<nb, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), vals[res], (int64_t)nt,
-                                    s.left.as<uint32_t>(), s.right.as<uint32_t>(),
-                                    s.par_i.as<uint32_t>(), s.par_l.as<uint32_t>(),
-                                    sc->tris.as<float4>(), s.leaf_box.as<float>(),
-                                    s.int_box.as<float>(), s.visit.as<uint32_t>());
-    C2B_KERNEL_CHECK();
-    k_bvh_layout<<<(int)((sc->n_nodes + 255) / 256), 256, 0, st>>>(
-        (int64_t)nt, s.left.as<uint32_t>(), s.right.as<uint32_t>(), s.first.as<uint32_t>(),
-        s.last.as<uint32_t>(), s.par_i.as<uint32_t>(), s.par_l.as<uint32_t>(),
-        s.leaf_box.as<float>(), s.int_box.as<float>(), sc->nodes.as<float4>());
-    C2B_KERNEL_CHECK();
-    uint32_t hb[6];
-    C2B_CUDA(cudaMemcpyAsync(hb, s.bounds.p, 24, cudaMemcpyDeviceToHost, st));
-    C2B_CUDA(cudaStreamSynchronize(st));
-    for (int k = 0; k < 3; ++k) {
-      uint32_t a = hb[k], b = hb[3 + k];
-      uint32_t ua = (a & 0x80000000u) ? (a & 0x7fffffffu) : ~a;
-      uint32_t ub = (b & 0x80000000u) ? (b & 0x7fffffffu) : ~b;
-      memcpy(&sc->lo[k], &ua, 4);
-      memcpy(&sc->hi[k], &ub, 4);
-    }
-    return C2B_OK;
-  }();
-  s.release();
-  return rc;
+  }
+  k_bvh_refit<<<nb, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), vals[res], (int64_t)nt,
+                                  s.left.as<uint32_t>(), s.right.as<uint32_t>(),
+                                  s.par_i.as<uint32_t>(), s.par_l.as<uint32_t>(),
+                                  sc->tris.as<float4>(), s.leaf_box.as<float>(),
+                                  s.int_box.as<float>(), s.visit.as<uint32_t>());
+  C2B_KERNEL_CHECK();
+  k_bvh_layout<<<(int)((sc->n_nodes + 255) / 256), 256, 0, st>>>(
+      (int64_t)nt, s.left.as<uint32_t>(), s.right.as<uint32_t>(), s.first.as<uint32_t>(),
+      s.last.as<uint32_t>(), s.par_i.as<uint32_t>(), s.par_l.as<uint32_t>(),
+      s.leaf_box.as<float>(), s.int_box.as<float>(), sc->nodes.as<float4>());
+  C2B_KERNEL_CHECK();
+  uint32_t hb[6];
+  C2B_CUDA(cudaMemcpyAsync(hb, s.bounds.p, 24, cudaMemcpyDeviceToHost, st));
+  C2B_CUDA(cudaStreamSynchronize(st));
+  for (int k = 0; k < 3; ++k) {
+    uint32_t a = hb[k], b = hb[3 + k];
+    uint32_t ua = (a & 0x80000000u) ? (a & 0x7fffffffu) : ~a;
+    uint32_t ub = (b & 0x80000000u) ? (b & 0x7fffffffu) : ~b;
+    memcpy(&sc->lo[k], &ua, 4);
+    memcpy(&sc->hi[k], &ub, 4);
+  }
+  return C2B_OK;
 }
 
 }  // namespace c2b

@@ -7,7 +7,10 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 #if defined(__linux__)
 #include <sys/syscall.h>
@@ -60,17 +63,24 @@ inline std::atomic<uint64_t> &launch_counter() {
     C2B_CUDA(cudaGetLastError());    \
   } while (0)
 
-// grow-only device buffer
+// grow-only device buffer, freed by its destructor: its owner makes the buffer's device current first
 struct DevBuf {
   void *p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, (size_t)0)) {}
+  DevBuf &operator=(DevBuf &&o) noexcept {
+    if (this != &o) {
+      release();
+      p = std::exchange(o.p, nullptr);
+      cap = std::exchange(o.cap, (size_t)0);
+    }
+    return *this;
+  }
+  ~DevBuf() { release(); }
   int ensure(size_t bytes) {
     if (bytes <= cap) return C2B_OK;
-    if (p) {
-      cudaFree(p);
-      p = nullptr;
-      cap = 0;
-    }
+    release();
     size_t want = bytes + bytes / 4 + 256;
     cudaError_t e = cudaMalloc(&p, want);
     if (e != cudaSuccess) {
@@ -127,13 +137,23 @@ struct PinBuf {
   size_t cap = 0;
   int node = -1;  // NUMA node of the GPU these buffers feed (-1: unknown / off)
   bool portable = false;  // every device of the process may DMA into it (the one host CSR of c2b_visibility_graph_multi)
+  PinBuf() = default;
+  PinBuf(PinBuf &&o) noexcept
+      : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, (size_t)0)), node(o.node), portable(o.portable) {}
+  PinBuf &operator=(PinBuf &&o) noexcept {
+    if (this != &o) {
+      release();
+      p = std::exchange(o.p, nullptr);
+      cap = std::exchange(o.cap, (size_t)0);
+      node = o.node;
+      portable = o.portable;
+    }
+    return *this;
+  }
+  ~PinBuf() { release(); }
   int ensure(size_t bytes) {
     if (bytes <= cap) return C2B_OK;
-    if (p) {
-      cudaFreeHost(p);
-      p = nullptr;
-      cap = 0;
-    }
+    release();
     // pinning costs ~0.5 s per GB on this pool's hosts (profiles/r02b_alloc_probe.txt): large buffers get
     // little slack, small ones a quarter
     size_t want = bytes + (bytes > (64u << 20) ? bytes / 32 : bytes / 4) + 256;
@@ -159,6 +179,44 @@ struct PinBuf {
   }
 };
 
+// An owned event or stream: create() makes it (a C2B_* status), the destructor or release() destroys it, with the
+// owner's device current.  Converts to the raw handle for the runtime calls.
+template <class H, cudaError_t (*make)(H *, unsigned), cudaError_t (*destroy)(H)>
+class CudaHandle {
+ public:
+  CudaHandle() = default;
+  CudaHandle(CudaHandle &&o) noexcept : h_(std::exchange(o.h_, nullptr)) {}
+  CudaHandle &operator=(CudaHandle &&o) noexcept {
+    if (this != &o) {
+      release();
+      h_ = std::exchange(o.h_, nullptr);
+    }
+    return *this;
+  }
+  ~CudaHandle() { release(); }
+  int create(unsigned flags = 0) {
+    release();
+    C2B_CUDA(make(&h_, flags));
+    return C2B_OK;
+  }
+  void release() {
+    if (h_) destroy(h_);
+    h_ = nullptr;
+  }
+  operator H() const { return h_; }
+
+ private:
+  H h_ = nullptr;
+};
+using Event = CudaHandle<cudaEvent_t, cudaEventCreateWithFlags, cudaEventDestroy>;
+using Stream = CudaHandle<cudaStream_t, cudaStreamCreateWithFlags, cudaStreamDestroy>;
+
+static_assert(!std::is_copy_constructible<DevBuf>::value && !std::is_copy_constructible<PinBuf>::value &&
+                  !std::is_copy_constructible<Event>::value && !std::is_copy_constructible<Stream>::value,
+              "owners of device resources are move-only");
+
+struct CtxExtra;  // per-context state of c2b_api.cu (tunables, caches, BAL buffers)
+
 enum StageEvent {
   EV_START = 0,
   EV_H2D,
@@ -182,11 +240,16 @@ struct c2b_scene {
   c2b::DevBuf tris;   // float4[3*n_tris]: v0, v1, v2 in leaf (Morton) order
 };
 
+// Owns everything it lists; ~c2b_ctx (c2b_api.cu, where CtxExtra is complete) runs with `device` current.  The
+// streams come first so that they are destroyed last.
 struct c2b_ctx {
   int device = 0;
   int sm_count = 148;
-  cudaStream_t stream = nullptr;
-  cudaEvent_t ev[c2b::EV_COUNT] = {};
+  c2b::Stream stream;
+  c2b::Stream copy_stream;
+  c2b::Stream aux_stream;  // leaf lists beside the plan (visibility_grid_fused)
+  std::unique_ptr<c2b::CtxExtra> extra;
+  c2b::Event ev[c2b::EV_COUNT];
 
   // resident problem
   uint64_t C = 0, P = 0;
@@ -213,10 +276,8 @@ struct c2b_ctx {
   c2b::DevBuf out_offsets[2], out_idx[2], out_uv[2];
   int out_sel = 0;
   uint64_t out_C = 0, out_O = 0;
-  cudaStream_t copy_stream = nullptr;
-  cudaStream_t aux_stream = nullptr;  // leaf lists beside the plan (visibility_grid_fused)
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  cudaEvent_t ev_ready[2] = {}, ev_copied[2] = {};
+  c2b::Event ev_fork, ev_join;
+  c2b::Event ev_ready[2], ev_copied[2];
   c2b::DevBuf misc;  // small scratch (reductions)
   c2b::DevBuf tri_list, tri_count;  // per-camera leaf lists for list-driven traversal
   // fused grid schedule: per-camera plan (row points -> scratch slice), visible counts, CSR offsets
@@ -234,4 +295,6 @@ struct c2b_ctx {
 
   // host results
   c2b::PinBuf h_offsets, h_idx, h_uv, h_small;
+
+  ~c2b_ctx();
 };

@@ -21,6 +21,7 @@
 #include <chrono>
 #include <condition_variable>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <string>
@@ -148,10 +149,10 @@ struct c2b_multi {
   c2b_ctx *ctx[C2B_MAX_GPUS] = {};
   ncclComm_t comm[C2B_MAX_GPUS] = {};
   bool have_comm = false;
-  Worker *worker[C2B_MAX_GPUS] = {};
+  std::unique_ptr<Worker> worker[C2B_MAX_GPUS];
   DevBuf d_counts[C2B_MAX_GPUS];
   PinBuf h_counts[C2B_MAX_GPUS];
-  cudaEvent_t ev[C2B_MAX_GPUS][4] = {};
+  Event ev[C2B_MAX_GPUS][4];
   PinBuf h_offsets, h_idx, h_uv;  // the ONE host CSR
   std::mutex mu;
   // share of the cameras each GPU gets: equal at first, then following each GPU's measured speed (pass + slab
@@ -222,8 +223,10 @@ int c2b_init_multi(int n_gpus, const int *devices, c2b_multi **out) {
     const int rc = c2b_init(m->dev[g], &m->ctx[g]);
     if (rc != C2B_OK) return fail(rc);
     if (cudaSetDevice(m->dev[g]) != cudaSuccess) return fail(set_error(C2B_ERR_CUDA, "cudaSetDevice(%d) failed", m->dev[g]));
-    for (auto &e : m->ev[g])
-      if (cudaEventCreate(&e) != cudaSuccess) return fail(set_error(C2B_ERR_CUDA, "cudaEventCreate failed"));
+    for (auto &e : m->ev[g]) {
+      const int rc = e.create();
+      if (rc != C2B_OK) return fail(rc);
+    }
     if (m->d_counts[g].ensure(C2B_MAX_GPUS * 8) != C2B_OK || m->h_counts[g].ensure(C2B_MAX_GPUS * 8) != C2B_OK)
       return fail(C2B_ERR_OOM);
   }
@@ -246,8 +249,8 @@ int c2b_init_multi(int n_gpus, const int *devices, c2b_multi **out) {
     m->have_comm = true;
   }
   for (int g = 0; g < n_gpus; ++g) {
-    m->worker[g] = new Worker();
-    Worker *w = m->worker[g];
+    m->worker[g] = std::make_unique<Worker>();
+    Worker *w = m->worker[g].get();
     w->th = std::thread([w]() { w->loop(); });
   }
   *out = m;
@@ -264,21 +267,17 @@ void c2b_shutdown_multi(c2b_multi *m) {
       }
       m->worker[g]->cv.notify_all();
       if (m->worker[g]->th.joinable()) m->worker[g]->th.join();
-      delete m->worker[g];
+      m->worker[g].reset();
     }
   for (int g = 0; g < m->n; ++g) {
     if (!m->ctx[g]) continue;
     cudaSetDevice(m->dev[g]);
     cudaDeviceSynchronize();
     if (m->have_comm && m->comm[g]) nccl().CommDestroy(m->comm[g]);
-    for (auto &e : m->ev[g])
-      if (e) cudaEventDestroy(e);
+    for (auto &e : m->ev[g]) e.release();
     m->d_counts[g].release();
     m->h_counts[g].release();
   }
-  m->h_offsets.release();
-  m->h_idx.release();
-  m->h_uv.release();
   for (int g = 0; g < m->n; ++g)
     if (m->ctx[g]) c2b_shutdown(m->ctx[g]);
   delete m;
