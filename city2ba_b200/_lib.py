@@ -92,6 +92,17 @@ class CullStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
 
 
+class MismatchStats(C.Structure):
+    """c2b_mismatch_stats: selected observations, those whose partner is another observation, and device times"""
+    _fields_ = [
+        ("n_selected", C.c_uint64), ("n_swapped", C.c_uint64),
+        ("ms_h2d", C.c_float), ("ms_compute", C.c_float), ("ms_d2h", C.c_float),
+    ]
+
+    def to_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 class BalStats(C.Structure):
     """c2b_bal_stats: bytes and chunks of one BAL file, device ms of encode / D2H, host ms of write(2)"""
     _fields_ = [
@@ -135,7 +146,8 @@ EXPORTS = [
     "c2b_visibility_graph_resident", "c2b_download_obs", "c2b_reprojection_error_resident",
     "c2b_add_drift", "c2b_add_drift_normalized", "c2b_add_noise", "c2b_add_sin_noise", "c2b_noise_timing",
     "c2b_add_drift_resident", "c2b_add_noise_resident", "c2b_add_sin_noise_resident", "c2b_download_problem",
-    "c2b_mean_std", "c2b_cull_problem", "c2b_cull_problem_resident", "c2b_write_bal", "c2b_write_bal_resident",
+    "c2b_mean_std", "c2b_cull_problem", "c2b_cull_problem_resident",
+    "c2b_add_incorrect_correspondences", "c2b_add_incorrect_correspondences_resident", "c2b_write_bal", "c2b_write_bal_resident",
     "c2b_read_bal_resident", "c2b_generate_world_points_uniform",
     "c2b_grid_num_cameras", "c2b_grid_num_points", "c2b_grid_cameras", "c2b_grid_points",
     "c2b_line_cameras", "c2b_line_points", "c2b_city_mesh", "c2b_camera_center",
@@ -216,6 +228,9 @@ def lib():
     L.c2b_mean_std.argtypes = [vp, pd, u64, pd, u64, pd, pd]
     L.c2b_cull_problem.argtypes = [vp, pd, u64, pd, u64, C.POINTER(u64), pu32, pd, C.POINTER(CullStats)]
     L.c2b_cull_problem_resident.argtypes = [vp, C.POINTER(CullStats)]
+    L.c2b_add_incorrect_correspondences.argtypes = [vp, C.POINTER(u64), u64, pu32, pd, dbl, u64,
+                                                    C.POINTER(MismatchStats)]
+    L.c2b_add_incorrect_correspondences_resident.argtypes = [vp, dbl, u64, C.POINTER(MismatchStats)]
     L.c2b_write_bal.argtypes = [vp, C.c_char_p, i32, pd, u64, pd, u64, C.POINTER(u64), pu32, pd, C.POINTER(BalStats)]
     L.c2b_write_bal_resident.argtypes = [vp, C.c_char_p, i32, C.POINTER(BalStats)]
     L.c2b_read_bal_resident.argtypes = [vp, C.c_char_p, i32, C.POINTER(BalReadStats)]

@@ -32,6 +32,7 @@
 #include "c2b_graph_cull.cuh"
 #include "c2b_internal.h"
 #include "c2b_math.cuh"
+#include "c2b_mismatch.cuh"
 #include "c2b_noise.cuh"
 #include "c2b_sample.cuh"
 #include "c2b_sort.cuh"
@@ -298,6 +299,8 @@ struct c2b::CtxExtra {
   // BAL reader (c2b_bal_read.cuh): per-observation camera, per-camera counts, slow-token records of two chunks,
   // error offsets / token counter
   DevBuf bal_cam, bal_cnt, bal_slow[2], bal_small;
+  // add_incorrect_correspondences (c2b_mismatch.cuh): per-camera counts / bases, selections + picks, flag / counters
+  DevBuf mm_cnt, mm_sel, mm_small;
   GridCache grid;
   uint64_t points_version = 0;
   double pts_bounds[6] = {0, 0, 0, 0, 0, 0};
@@ -2428,6 +2431,131 @@ int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
     out->n_points = P;
     out->n_obs = O;
     out->iterations = it;
+    cudaEventElapsedTime(&out->ms_compute, ev[0], ev[1]);
+  }
+  return C2B_OK;
+}
+
+// ---- noise::add_incorrect_correspondences (c2b_mismatch.cuh) -------------------------------------------------------
+// the message of a failed selection: camera, observation within it, CSR index, and the reference's panic text
+static int mismatch_error(const char *who, const uint64_t *offsets, uint64_t C, unsigned long long err) {
+  const uint64_t o = err >> 1;
+  const uint64_t c = (uint64_t)(std::upper_bound(offsets, offsets + C + 1, o) - offsets) - 1;
+  return set_error(C2B_ERR_INVALID, "%s: camera %llu, observation %llu (CSR index %llu): called `Result::unwrap()` on an "
+                                    "`Err` value: %s",
+                   who, (unsigned long long)c, (unsigned long long)(o - offsets[c]), (unsigned long long)o,
+                   (err & 1) == MM_NEGATIVE_WEIGHT ? "NegativeWeight" : "AllWeightsZero");
+}
+
+int c2b_add_incorrect_correspondences(c2b_ctx *ctx, const uint64_t *offsets, uint64_t C, uint32_t *point_idx,
+                                      const double *uv, double mismatch_chance, uint64_t seed,
+                                      c2b_mismatch_stats *out) {
+  static const char *who = "c2b_add_incorrect_correspondences";
+  if (!ctx || !offsets) return set_error(C2B_ERR_INVALID, "%s: null argument", who);
+  const uint64_t O = offsets[C];
+  if (O && (!point_idx || !uv)) return set_error(C2B_ERR_INVALID, "%s: null observation array", who);
+  C2B_TRY(cull_limits(C, 0, O, who));
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  CtxExtra *x = ctx->extra.get();
+  cudaStream_t st = ctx->stream;
+  // the host-array cull's set 0: never the resident problem
+  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
+  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
+  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
+  C2B_TRY(ctx->pr_small.ensure(64));
+  C2B_TRY(ctx->h_small.ensure(256));
+  Event ev[4];  // timing
+  for (auto &e : ev) C2B_TRY(e.create());
+  int rc = [&]() -> int {
+    C2B_CUDA(cudaEventRecord(ev[0], st));
+    C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
+    if (O) {
+      C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
+      C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
+    }
+    // offsets start at 0 and do not decrease; there is no point count, so no u32 index is out of range
+    uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
+    C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+    const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
+    k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
+        ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, 1ull << 32, flag);
+    C2B_KERNEL_CHECK();
+    C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaEventRecord(ev[1], st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    if (*ctx->h_small.as<uint32_t>() & 1u)
+      return set_error(C2B_ERR_INVALID, "%s: offsets[0] != 0 or the CSR offsets decrease", who);
+    uint64_t ns = 0, nw = 0;
+    unsigned long long err = MM_NO_ERROR;
+    C2B_TRY(mismatch_pass(ctx, MismatchBufs{&x->mm_cnt, &x->mm_sel, &x->mm_small}, ctx->pr_off[0].as<uint64_t>(), C,
+                          ctx->pr_idx[0].as<uint32_t>(), ctx->pr_uv[0].as<double2>(), mismatch_chance, seed, &ns, &nw,
+                          &err));
+    if (err != MM_NO_ERROR) return mismatch_error(who, offsets, C, err);
+    C2B_CUDA(cudaEventRecord(ev[2], st));
+    if (O) C2B_CUDA(cudaMemcpyAsync(point_idx, ctx->pr_idx[0].p, O * 4, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaEventRecord(ev[3], st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    if (out) {
+      memset(out, 0, sizeof *out);
+      out->n_selected = ns;
+      out->n_swapped = nw;
+      cudaEventElapsedTime(&out->ms_h2d, ev[0], ev[1]);
+      cudaEventElapsedTime(&out->ms_compute, ev[1], ev[2]);
+      cudaEventElapsedTime(&out->ms_d2h, ev[2], ev[3]);
+    }
+    return C2B_OK;
+  }();
+  if (rc != C2B_OK) cudaStreamSynchronize(st);
+  return rc;
+}
+
+int c2b_add_incorrect_correspondences_resident(c2b_ctx *ctx, double mismatch_chance, uint64_t seed,
+                                               c2b_mismatch_stats *out) {
+  static const char *who = "c2b_add_incorrect_correspondences_resident";
+  if (!ctx) return set_error(C2B_ERR_INVALID, "%s: null ctx", who);
+  CtxExtra *x = ctx->extra.get();
+  if (x->host_call_last)
+    return set_error(C2B_ERR_INVALID, "%s: the resident CSR is the last camera batch of the host-buffer "
+                                      "c2b_visibility_graph, not the graph of an uploaded problem; run "
+                                      "c2b_visibility_graph_resident first", who);
+  if (!x->have_result || !x->have_points || !x->have_cameras)
+    return set_error(C2B_ERR_INVALID, "%s: no resident result (upload cameras and points, then "
+                                      "c2b_visibility_graph_resident)", who);
+  const uint64_t C = ctx->out_C, O = ctx->out_O;
+  C2B_TRY(cull_limits(C, 0, O, who));
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const int sel = ctx->out_sel;
+  Event ev[2];  // timing
+  for (auto &e : ev) C2B_TRY(e.create());
+  uint64_t ns = 0, nw = 0;
+  unsigned long long err = MM_NO_ERROR;
+  int rc = [&]() -> int {
+    C2B_CUDA(cudaEventRecord(ev[0], st));
+    C2B_TRY(mismatch_pass(ctx, MismatchBufs{&x->mm_cnt, &x->mm_sel, &x->mm_small}, ctx->out_offsets[sel].as<uint64_t>(),
+                          C, ctx->out_idx[sel].as<uint32_t>(), ctx->out_uv[sel].as<double2>(), mismatch_chance, seed,
+                          &ns, &nw, &err));
+    C2B_CUDA(cudaEventRecord(ev[1], st));
+    return C2B_OK;
+  }();
+  if (rc != C2B_OK) {
+    // a failure of the library, not of the input: the point indices may be half permuted
+    cudaStreamSynchronize(st);
+    x->have_result = false;
+    return rc;
+  }
+  if (err != MM_NO_ERROR) {
+    // the resident problem is unchanged; the offsets name the camera in the message
+    std::vector<uint64_t> offsets(C + 1);
+    C2B_CUDA(cudaMemcpyAsync(offsets.data(), ctx->out_offsets[sel].p, (C + 1) * 8, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    return mismatch_error(who, offsets.data(), C, err);
+  }
+  C2B_CUDA(cudaStreamSynchronize(st));
+  if (out) {
+    memset(out, 0, sizeof *out);
+    out->n_selected = ns;
+    out->n_swapped = nw;
     cudaEventElapsedTime(&out->ms_compute, ev[0], ev[1]);
   }
   return C2B_OK;

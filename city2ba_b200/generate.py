@@ -337,6 +337,23 @@ class ResidentProblem:
         check(lib().c2b_cull_problem_resident(self.ctx.handle, C.byref(st)))
         return st.to_dict()
 
+    def add_incorrect_correspondences(self, mismatch_chance, seed=0) -> dict:
+        """noise::add_incorrect_correspondences on the resident CSR, in HBM (c2b_add_incorrect_correspondences_resident):
+        the draws of noise.add_incorrect_correspondences_gpu.  Afterwards download / reprojection_error / cull / write
+        see the edited graph.  Raises AssertionError (AllWeightsZero / NegativeWeight) and leaves the problem unchanged
+        when a selected observation's weights are invalid.  Returns the stats: n_selected, n_swapped, ms_compute."""
+        from .noise import _weight_error
+        st = _lib.MismatchStats()
+        try:
+            check(lib().c2b_add_incorrect_correspondences_resident(self.ctx.handle, float(mismatch_chance),
+                                                                   int(seed) & (2 ** 64 - 1), C.byref(st)))
+        except _lib.C2BError as e:
+            a = _weight_error(e)
+            if a is not None:
+                raise a from e
+            raise
+        return st.to_dict()
+
     def write(self, path) -> dict:
         """BAProblem::write of the resident problem (c2b_write_bal_resident): .bal text or .bbal binary by the
         extension, encoded on the GPU and streamed to disk.  Returns the stats: bytes, chunks, ms_encode, ms_d2h

@@ -111,6 +111,46 @@ def add_incorrect_correspondences(bal: BAProblem, mismatch_chance, seed=None) ->
     return _with_graph(bal, g.offsets, idx, g.uv)
 
 
+def _weight_error(e):
+    """C2BError of a selection with invalid weights -> the host form's AssertionError (same message tail)"""
+    from ._lib import ERR_INVALID, C2BError
+    if isinstance(e, C2BError) and e.code == ERR_INVALID and "called `Result::unwrap()` on an `Err` value" in str(e):
+        return AssertionError(str(e))
+    return None
+
+
+def add_incorrect_correspondences_gpu(bal: BAProblem, mismatch_chance, seed=None, ctx=None, stats=None) -> BAProblem:
+    """add_incorrect_correspondences on the GPU (c2b_add_incorrect_correspondences): the same operation with the
+    library's deterministic draws, a pure function of `seed` (default: a fresh one from os.urandom), so it does not
+    reproduce the numpy draws of the host form.  Raises AssertionError on a selected observation whose image distances
+    are all 0 (AllWeightsZero) or not all finite (NegativeWeight).  Works on copies; `stats`, a dict if given, receives
+    the call's c2b_mismatch_stats (n_selected, n_swapped, device times)."""
+    from ._lib import C2BError, MismatchStats
+    ctx = ctx or context()
+    g = bal.vis_graph
+    off = np.array(g.offsets, np.uint64, order="C")
+    if len(off) != len(bal.cameras) + 1:
+        raise ValueError("cameras and CSR offsets disagree")
+    idx = g.point_idx
+    if len(idx) and int(idx.max()) > 0xffffffff:
+        raise ValueError("point index does not fit 32 bits")
+    idx = np.array(idx, np.uint32, order="C")
+    uv = np.array(g.uv, np.float64, order="C").reshape(-1, 2)
+    st = MismatchStats()
+    try:
+        check(lib().c2b_add_incorrect_correspondences(ctx.handle, off.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                      len(off) - 1, idx.ctypes.data_as(C.POINTER(C.c_uint32)),
+                                                      _p(uv), float(mismatch_chance), _seed(seed), C.byref(st)))
+    except C2BError as e:
+        a = _weight_error(e)
+        if a is not None:
+            raise a from e
+        raise
+    if stats is not None:
+        stats.update(st.to_dict())
+    return _with_graph(bal, off, idx, uv)
+
+
 def drop_features(bal: BAProblem, drop_percent, seed=None) -> BAProblem:
     """src/noise.rs:229-250: every camera keeps floor(len * drop_percent) of its observations, chosen by a shuffle"""
     rng = np.random.default_rng(seed)

@@ -1364,6 +1364,41 @@ inline BAProblem add_incorrect_correspondences(const BAProblem &bal, double mism
   }
   return out;
 }
+// the same on the GPU (c2b_add_incorrect_correspondences), with the library's deterministic draws: a pure function
+// of seed, not the draws of the host form above.  Throws std::logic_error with the host form's text when a selected
+// observation's weights are invalid.  stats (optional) receives the call's counts and device times.
+inline BAProblem add_incorrect_correspondences(const Context &ctx, const BAProblem &bal, double mismatch_chance,
+                                               uint64_t seed, c2b_mismatch_stats *stats = nullptr) {
+  const size_t nc = bal.num_cameras();
+  std::vector<uint64_t> offsets(nc + 1, 0);
+  for (size_t i = 0; i < nc; ++i) offsets[i + 1] = offsets[i] + bal.vis_graph[i].size();
+  std::vector<uint32_t> idx(offsets[nc]);
+  std::vector<double> uv(2 * offsets[nc]);
+  for (size_t i = 0, k = 0; i < nc; ++i)
+    for (const auto &e : bal.vis_graph[i]) {
+      detail::require(e.first <= 0xffffffffull, "point index does not fit 32 bits");
+      idx[k] = (uint32_t)e.first;
+      uv[2 * k] = e.second.first;
+      uv[2 * k + 1] = e.second.second;
+      ++k;
+    }
+  c2b_mismatch_stats st;
+  const int rc = c2b_add_incorrect_correspondences(ctx.handle(), offsets.data(), nc, idx.data(), uv.data(),
+                                                   mismatch_chance, seed, &st);
+  if (rc == C2B_ERR_INVALID) {
+    const std::string m = c2b_last_error();
+    for (const char *kind : {"AllWeightsZero", "NegativeWeight"})
+      if (m.size() >= std::strlen(kind) && m.compare(m.size() - std::strlen(kind), std::string::npos, kind) == 0)
+        throw std::logic_error(std::string("called `Result::unwrap()` on an `Err` value: ") + kind);
+  }
+  detail::check(rc);
+  if (stats) *stats = st;
+  BAProblem out = bal;
+  size_t k = 0;
+  for (auto &o : out.vis_graph)
+    for (auto &e : o) e.first = idx[k++];
+  return out;
+}
 
 // src/noise.rs:229-250: every camera keeps floor(len * drop_percent) of its observations, chosen by a shuffle
 inline BAProblem drop_features(const BAProblem &bal, double drop_percent, uint64_t seed) {

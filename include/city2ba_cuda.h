@@ -320,6 +320,34 @@ int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64
  * and after the host-buffer c2b_visibility_graph (which leaves only its last camera batch resident). */
 int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out);
 
+/* ---- noise::add_incorrect_correspondences (src/noise.rs:180-226) ------------------------------------------------
+ * In every camera of more than one observation, observation i is selected with probability mismatch_chance and swaps
+ * its point index with observation j of the same camera, drawn with weight maxd - |uv_i - uv_j| (maxd the largest such
+ * distance; i itself weighs maxd).  (u, v), offsets, cameras and points are not changed.  Deterministic in seed:
+ * one Philox4x32-10 block per observation (key seed, counter (o lo, o hi, 6, 0)); u from words 0-1 (53 bits) selects
+ * when u <= mismatch_chance; weights are quantised to floor(w / maxd * 2^32) and j is found from words 2-3 by an
+ * integer prefix sum (DESIGN.md §4, "Mismatched correspondences").  The transpositions apply per camera in ascending i.
+ * A selected observation whose distances are not all finite fails with NegativeWeight, one whose distances are all 0
+ * with AllWeightsZero (Rng::weighted): C2B_ERR_INVALID, the message names the lowest such observation and its camera
+ * and ends in "called `Result::unwrap()` on an `Err` value: <kind>"; nothing is changed then. */
+typedef struct {
+  uint64_t n_selected;               /* observations selected (in cameras of more than one observation) */
+  uint64_t n_swapped;                /* selections whose partner is another observation */
+  float ms_h2d, ms_compute, ms_d2h;  /* device time (CUDA events on the ctx stream); h2d/d2h 0 when resident;
+                                        ms_h2d includes the input check */
+} c2b_mismatch_stats;
+/* in place on host arrays: point_idx / uv hold O = offsets[C] entries.  Rejects offsets[0] != 0 and decreasing
+ * offsets with C2B_ERR_INVALID and leaves point_idx untouched.  C and O below 2^32 - 1.  Does not touch the ctx's
+ * resident problem.  out may be NULL. */
+int c2b_add_incorrect_correspondences(c2b_ctx *ctx, const uint64_t *offsets, uint64_t C, uint32_t *point_idx,
+                                      const double *uv, double mismatch_chance, uint64_t seed,
+                                      c2b_mismatch_stats *out);
+/* the same on the resident CSR, in HBM; afterwards c2b_download_obs, c2b_reprojection_error_resident,
+ * c2b_cull_problem_resident and c2b_write_bal_resident see the edited graph.  Refuses in the cases
+ * c2b_cull_problem_resident refuses. */
+int c2b_add_incorrect_correspondences_resident(c2b_ctx *ctx, double mismatch_chance, uint64_t seed,
+                                               c2b_mismatch_stats *out);
+
 /* ---- BAL files (BAProblem::write, src/baproblem.rs:709-764) ----------------------------------------------------
  * The file is encoded on the device and streamed to disk in chunks of at most bal_chunk_bytes: the D2H copy and
  * the host write of one chunk overlap the encoding of the next, and the device and pinned memory of the encoder

@@ -48,6 +48,13 @@ pub struct c2b_cull_stats {
     pub ms_h2d: c_float, pub ms_compute: c_float, pub ms_d2h: c_float,
 }
 
+// noise::add_incorrect_correspondences on the GPU (c2b_add_incorrect_correspondences[_resident])
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct c2b_mismatch_stats {
+    pub n_selected: u64, pub n_swapped: u64,
+    pub ms_h2d: c_float, pub ms_compute: c_float, pub ms_d2h: c_float,
+}
+
 // BAL files on the GPU (c2b_write_bal / c2b_write_bal_resident)
 pub const C2B_BAL_TEXT: c_int = 0;
 pub const C2B_BAL_BINARY: c_int = 1;
@@ -155,6 +162,11 @@ extern "C" {
                             offsets: *mut u64, point_idx: *mut u32, uv: *mut c_double,
                             out: *mut c2b_cull_stats) -> c_int;
     pub fn c2b_cull_problem_resident(ctx: *mut c2b_ctx, out: *mut c2b_cull_stats) -> c_int;
+    pub fn c2b_add_incorrect_correspondences(ctx: *mut c2b_ctx, offsets: *const u64, c: u64, point_idx: *mut u32,
+                                             uv: *const c_double, mismatch_chance: c_double, seed: u64,
+                                             out: *mut c2b_mismatch_stats) -> c_int;
+    pub fn c2b_add_incorrect_correspondences_resident(ctx: *mut c2b_ctx, mismatch_chance: c_double, seed: u64,
+                                                      out: *mut c2b_mismatch_stats) -> c_int;
     // ---- BAL files: a Rust BAProblem::write would call c2b_write_bal with the format of its extension ----
     pub fn c2b_write_bal(ctx: *mut c2b_ctx, path: *const c_char, format: c_int, cams: *const c_double, c: u64,
                          pts: *const c_double, p: u64, offsets: *const u64, point_idx: *const u32,
