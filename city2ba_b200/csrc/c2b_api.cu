@@ -304,10 +304,13 @@ struct c2b::CtxExtra {
   GridCache grid;
   uint64_t points_version = 0;
   double pts_bounds[6] = {0, 0, 0, 0, 0, 0};
-  bool have_points = false, have_cameras = false, have_result = false;
-  // the last pass was the host-buffer c2b_visibility_graph (only its last batch stays).  have_result is already false
-  // then; this only picks the message with which c2b_cull_problem_resident refuses
-  bool host_call_last = false;
+  // the resident problem: cameras and points, set by their own uploads, and what the resident CSR
+  // (ctx->out_*[ctx->out_sel]) holds: nothing usable, the graph of those cameras and points, or the last camera batch
+  // of a host-buffer c2b_visibility_graph.  RESIDENT implies have_cameras and have_points.  Changed only by the
+  // transitions after copy_in (install_cameras, commit_points, install_graph, drop_graph, ...)
+  enum class Graph { NONE, RESIDENT, HOST_BATCH };
+  bool have_points = false, have_cameras = false;
+  Graph graph = Graph::NONE;
   uint64_t res_candidates = 0;
 };
 
@@ -628,29 +631,58 @@ int c2b_internal_copy_in(c2b_ctx *ctx, void *d, const void *h, size_t bytes) {
   return copy_in(ctx, d, h, bytes, cudaMemcpyHostToDevice);
 }
 
-// The AoS point array of the ctx, with room for `capacity` points, for callers that fill it on the device
-// themselves (an NCCL all-gather of per-GPU shards, c2b_multi.cu); followed by c2b_points_commit.
-int c2b_points_device_buffer(c2b_ctx *ctx, uint64_t capacity, double **d_out) {
-  if (!ctx || !d_out) return set_error(C2B_ERR_INVALID, "c2b_points_device_buffer: null argument");
-  C2B_CUDA(cudaSetDevice(ctx->device));
-  C2B_TRY(ctx->pts_aos.ensure(std::max<uint64_t>(capacity, 1) * 24));
-  *d_out = ctx->pts_aos.as<double>();
+// ---- the resident problem: its transitions and the entries' preconditions ------------------------------------
+// camera centres (SoA) of C camera records, on ctx->stream
+static int cam_prep(c2b_ctx *ctx, const double *cams, uint64_t C, double *centers) {
+  if (C == 0) return C2B_OK;
+  k_cam_prep<<<blocks_for(C, 128), 128, 0, ctx->stream>>>(cams, C, centers, centers + C, centers + 2 * C);
+  C2B_KERNEL_CHECK();
   return C2B_OK;
 }
 
-// pts_aos[0, P) is (being) written on ctx->stream: derive the SoA copy and the coordinate bounds
-int c2b_points_commit(c2b_ctx *ctx, uint64_t P) {
-  if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_points_commit: null ctx");
-  if (P * 24 > ctx->pts_aos.cap) return set_error(C2B_ERR_INVALID, "c2b_points_commit: %llu points exceed the buffer", (unsigned long long)P);
-  if (P >= 0xffffffffull) return set_error(C2B_ERR_INVALID, "too many points (%llu)", (unsigned long long)P);
+// the resident CSR is no longer the graph of the resident problem
+static void drop_graph(CtxExtra *x) { x->graph = CtxExtra::Graph::NONE; }
+
+// the CSR of set ctx->out_sel (C cameras, O observations) is the graph of the resident problem
+static void install_graph(c2b_ctx *ctx, uint64_t C, uint64_t O) {
+  ctx->out_C = C;
+  ctx->out_O = O;
+  ctx->extra->graph = CtxExtra::Graph::RESIDENT;
+}
+
+// the host-buffer c2b_visibility_graph leaves the last camera batch of its call in the resident CSR
+static void leave_host_batch(CtxExtra *x) { x->graph = CtxExtra::Graph::HOST_BATCH; }
+
+// nothing of the resident problem is usable any more (its arrays may be half rewritten)
+static void drop_problem(CtxExtra *x) {
+  x->have_cameras = x->have_points = false;
+  x->grid.valid = false;
+  drop_graph(x);
+}
+
+// C camera records at `src` (host or device memory, by `kind`; ctx->cams itself when they are in place already)
+// become the resident cameras, with their centres
+static int install_cameras(c2b_ctx *ctx, const double *src, uint64_t C, cudaMemcpyKind kind) {
   CtxExtra *x = ctx->extra.get();
-  C2B_CUDA(cudaSetDevice(ctx->device));
+  ctx->C = C;
+  x->have_cameras = true;
+  drop_graph(x);
+  if (C == 0) return C2B_OK;
+  C2B_TRY(ctx->cams.ensure(C * 120));
+  C2B_TRY(ctx->cam_center.ensure(C * 24));
+  if (src != ctx->cams.p) C2B_TRY(copy_in(ctx, ctx->cams.p, src, C * 120, kind));
+  return cam_prep(ctx, ctx->cams.as<double>(), C, ctx->cam_center.as<double>());
+}
+
+// pts_aos[0, P) is (being) written on ctx->stream and becomes the resident points (P < 2^32 - 1 and within pts_aos:
+// the caller's to check): derive the SoA copy and the coordinate bounds; the point grid is stale.  The resident graph
+// is left as it is.
+static int commit_points(c2b_ctx *ctx, uint64_t P) {
+  CtxExtra *x = ctx->extra.get();
   ctx->P = P;
   x->points_version++;
   x->grid.valid = false;
   x->have_points = true;
-  x->have_result = false;
-  x->host_call_last = false;
   if (P == 0) return C2B_OK;
   C2B_TRY(ctx->pts.ensure(P * 24));
   double *px = ctx->pts.as<double>(), *py = px + P, *pz = py + P;
@@ -666,6 +698,57 @@ int c2b_points_commit(c2b_ctx *ctx, uint64_t P) {
   C2B_KERNEL_CHECK();
   C2B_CUDA(cudaMemcpyAsync(x->pts_bounds, ctx->misc.p, 48, cudaMemcpyDeviceToHost, ctx->stream));
   return C2B_OK;
+}
+
+// a culled or read problem becomes the resident one: C camera records at `cams` (see install_cameras), the points in
+// pts_aos[0, P) and, as their graph, the CSR of set ctx->out_sel with O observations
+static int adopt_problem(c2b_ctx *ctx, const double *cams, cudaMemcpyKind kind, uint64_t C, uint64_t P, uint64_t O) {
+  C2B_TRY(install_cameras(ctx, cams, C, kind));
+  C2B_TRY(commit_points(ctx, P));
+  install_graph(ctx, C, O);
+  return C2B_OK;
+}
+
+// precondition of the entries that work on the resident cameras and points
+static int need_problem(c2b_ctx *ctx, const char *who) {
+  const CtxExtra *x = ctx->extra.get();
+  if (!x->have_points || !x->have_cameras) return set_error(C2B_ERR_INVALID, "%s: upload cameras and points first", who);
+  return C2B_OK;
+}
+
+// precondition of the entries that work on the resident problem's graph
+static int need_graph(c2b_ctx *ctx, const char *who) {
+  switch (ctx->extra->graph) {
+    case CtxExtra::Graph::RESIDENT:
+      return C2B_OK;
+    case CtxExtra::Graph::HOST_BATCH:
+      return set_error(C2B_ERR_INVALID, "%s: the resident CSR is the last camera batch of the host-buffer "
+                                        "c2b_visibility_graph, not the graph of an uploaded problem; run "
+                                        "c2b_visibility_graph_resident first", who);
+    default:
+      return set_error(C2B_ERR_INVALID, "%s: no resident result (upload cameras and points, then "
+                                        "c2b_visibility_graph_resident)", who);
+  }
+}
+
+// The AoS point array of the ctx, with room for `capacity` points, for callers that fill it on the device
+// themselves (an NCCL all-gather of per-GPU shards, c2b_multi.cu); followed by c2b_points_commit.
+int c2b_points_device_buffer(c2b_ctx *ctx, uint64_t capacity, double **d_out) {
+  if (!ctx || !d_out) return set_error(C2B_ERR_INVALID, "c2b_points_device_buffer: null argument");
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  C2B_TRY(ctx->pts_aos.ensure(std::max<uint64_t>(capacity, 1) * 24));
+  *d_out = ctx->pts_aos.as<double>();
+  return C2B_OK;
+}
+
+// pts_aos[0, P) is (being) written on ctx->stream: the new resident points, of which the resident CSR is no graph
+int c2b_points_commit(c2b_ctx *ctx, uint64_t P) {
+  if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_points_commit: null ctx");
+  if (P * 24 > ctx->pts_aos.cap) return set_error(C2B_ERR_INVALID, "c2b_points_commit: %llu points exceed the buffer", (unsigned long long)P);
+  if (P >= 0xffffffffull) return set_error(C2B_ERR_INVALID, "too many points (%llu)", (unsigned long long)P);
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  drop_graph(ctx->extra.get());
+  return commit_points(ctx, P);
 }
 
 static int upload_points_impl(c2b_ctx *ctx, const double *pts, uint64_t P, cudaMemcpyKind kind) {
@@ -694,38 +777,8 @@ int c2b_drop_point_grid(c2b_ctx *ctx) {
 int c2b_upload_cameras(c2b_ctx *ctx, const double *cams, uint64_t C) {
   if (!ctx || (C && !cams)) return set_error(C2B_ERR_INVALID, "c2b_upload_cameras: null argument");
   if (C >= 0xffffffffull) return set_error(C2B_ERR_INVALID, "too many cameras (%llu)", (unsigned long long)C);
-  CtxExtra *x = ctx->extra.get();
   C2B_CUDA(cudaSetDevice(ctx->device));
-  ctx->C = C;
-  x->have_cameras = true;
-  x->have_result = false;
-  x->host_call_last = false;
-  if (C == 0) return C2B_OK;
-  C2B_TRY(ctx->cams.ensure(C * 120));
-  C2B_TRY(ctx->cam_center.ensure(C * 24));
-  C2B_TRY(copy_in(ctx, ctx->cams.p, cams, C * 120, cudaMemcpyHostToDevice));
-  double *cx = ctx->cam_center.as<double>();
-  k_cam_prep<<<blocks_for(C, 128), 128, 0, ctx->stream>>>(ctx->cams.as<double>(), C, cx, cx + C, cx + 2 * C);
-  C2B_KERNEL_CHECK();
-  return C2B_OK;
-}
-
-// cameras [first, first + count) of the call's device copy (ctx->cams_all) become the resident cameras:
-// what c2b_upload_cameras does for a batch, without touching host memory again
-static int select_cameras(c2b_ctx *ctx, uint64_t first, uint64_t count) {
-  CtxExtra *x = ctx->extra.get();
-  ctx->C = count;
-  x->have_cameras = true;
-  x->have_result = false;
-  if (count == 0) return C2B_OK;
-  C2B_TRY(ctx->cams.ensure(count * 120));
-  C2B_TRY(ctx->cam_center.ensure(count * 24));
-  C2B_CUDA(cudaMemcpyAsync(ctx->cams.p, ctx->cams_all.as<double>() + 15 * first, count * 120, cudaMemcpyDeviceToDevice,
-                           ctx->stream));
-  double *cx = ctx->cam_center.as<double>();
-  k_cam_prep<<<blocks_for(count, 128), 128, 0, ctx->stream>>>(ctx->cams.as<double>(), count, cx, cx + count, cx + 2 * count);
-  C2B_KERNEL_CHECK();
-  return C2B_OK;
+  return install_cameras(ctx, cams, C, cudaMemcpyHostToDevice);
 }
 
 // ---- the pipeline ---------------------------------------------------------------------------------------
@@ -929,9 +982,7 @@ int visibility_grid_fused(c2b_ctx *ctx, CtxExtra *x, const c2b_scene *scene, dou
     C2B_CUDA(cudaMemsetAsync(ctx->out_offsets[sel].p, 0, (C + 1) * 8, st));
     for (int e : {EV_CULL, EV_SORT, EV_TRAVERSE, EV_COMPACT, EV_D2H}) C2B_CUDA(cudaEventRecord(ctx->ev[e], st));
     C2B_CUDA(cudaStreamSynchronize(st));
-    ctx->out_C = C;
-    ctx->out_O = 0;
-    x->have_result = true;
+    install_graph(ctx, C, 0);
     x->res_candidates = 0;
     fill_stats(ctx, stats, C, 0, 0, 0, 0);
     return C2B_OK;
@@ -1172,9 +1223,7 @@ int visibility_grid_fused(c2b_ctx *ctx, CtxExtra *x, const c2b_scene *scene, dou
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_COMPACT], st));
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_D2H], st));
   C2B_CUDA(cudaStreamSynchronize(st));
-  ctx->out_C = C;
-  ctx->out_O = total_obs;
-  x->have_result = true;
+  install_graph(ctx, C, total_obs);
   x->res_candidates = n_cand;
   fill_stats(ctx, stats, C, n_cand, pairs_eval, nodes, tris_t);
   return C2B_OK;
@@ -1188,7 +1237,6 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
 int c2b_visibility_graph_resident(c2b_ctx *ctx, const c2b_scene *scene, double max_dist,
                                   const c2b_vis_options *opt_in, c2b_obs *stats) {
   const int rc = visibility_resident_impl(ctx, scene, max_dist, opt_in, stats);
-  if (ctx) ctx->extra->host_call_last = false;
   return rc == ERR_TOO_LARGE ? C2B_ERR_INVALID : rc;
 }
 
@@ -1196,8 +1244,7 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
                                     const c2b_vis_options *opt_in, c2b_obs *stats) {
   if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_visibility_graph_resident: null ctx");
   CtxExtra *x = ctx->extra.get();
-  if (!x->have_points || !x->have_cameras)
-    return set_error(C2B_ERR_INVALID, "upload cameras and points first");
+  C2B_TRY(need_problem(ctx, "c2b_visibility_graph_resident"));
   c2b_vis_options opt;
   if (opt_in)
     opt = *opt_in;
@@ -1214,7 +1261,7 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const uint64_t C = ctx->C, P = ctx->P;
-  x->have_result = false;
+  drop_graph(x);
 
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_START], st));
   C2B_CUDA(cudaEventRecord(ctx->ev[EV_H2D], st));
@@ -1379,9 +1426,7 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
     memcpy(&total32, reinterpret_cast<const char *>(h_fin) + 48, 4);
     total_obs = total32;
   }
-  ctx->out_C = C;
-  ctx->out_O = total_obs;
-  x->have_result = true;
+  install_graph(ctx, C, total_obs);
   x->res_candidates = n_cand;
   fill_stats(ctx, stats, C, n_cand, pairs_eval, h_fin[2], h_fin[3]);
   return C2B_OK;
@@ -1389,8 +1434,7 @@ static int visibility_resident_impl(c2b_ctx *ctx, const c2b_scene *scene, double
 
 int c2b_download_obs(c2b_ctx *ctx, c2b_obs *out) {
   if (!ctx || !out) return set_error(C2B_ERR_INVALID, "c2b_download_obs: null argument");
-  CtxExtra *x = ctx->extra.get();
-  if (!x->have_result) return set_error(C2B_ERR_INVALID, "no resident result to download");
+  C2B_TRY(need_graph(ctx, "c2b_download_obs"));
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const uint64_t C = ctx->out_C, O = ctx->out_O;
@@ -1428,8 +1472,7 @@ __global__ void k_add_u64(uint64_t *v, uint64_t n, uint64_t add) {
 int c2b_download_obs_into(c2b_ctx *ctx, uint64_t obs_base, uint64_t *offsets_dst, uint32_t *idx_dst, double *uv_dst,
                           int with_end, float *ms_d2h) {
   if (!ctx || !offsets_dst) return set_error(C2B_ERR_INVALID, "c2b_download_obs_into: null argument");
-  CtxExtra *x = ctx->extra.get();
-  if (!x->have_result) return set_error(C2B_ERR_INVALID, "no resident result to download");
+  C2B_TRY(need_graph(ctx, "c2b_download_obs_into"));
   const uint64_t C = ctx->out_C, O = ctx->out_O;
   if (O && (!idx_dst || !uv_dst)) return set_error(C2B_ERR_INVALID, "c2b_download_obs_into: null result array");
   C2B_CUDA(cudaSetDevice(ctx->device));
@@ -1556,7 +1599,7 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
       C2B_TRY(copy_in(ctx, ctx->cams_all.p, cams, C * 120, cudaMemcpyHostToDevice));
     }
     if (grid_mode && n_batches > 1 && C && P) {
-      C2B_TRY(select_cameras(ctx, 0, C));
+      C2B_TRY(install_cameras(ctx, ctx->cams_all.as<double>(), C, cudaMemcpyDeviceToDevice));
       C2B_TRY(ensure_grid(ctx, x, max_dist));
       x->grid_locked = true;
     }
@@ -1575,7 +1618,7 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
         else
           C2B_CUDA(cudaStreamWaitEvent(st, ctx->ev_copied[sel], 0));
       }
-      C2B_TRY(select_cameras(ctx, c0, nc));
+      C2B_TRY(install_cameras(ctx, ctx->cams_all.as<double>() + 15 * c0, nc, cudaMemcpyDeviceToDevice));
       c2b_obs s1;
       const int rcb = visibility_resident_impl(ctx, scene, max_dist, opt, &s1);
       if (rcb == ERR_TOO_LARGE && nc > 1) {
@@ -1657,8 +1700,7 @@ int c2b_visibility_graph(c2b_ctx *ctx, const c2b_scene *scene, const double *cam
   rc = run();
   x->grid_locked = false;
   ctx->out_sel = 0;
-  x->have_result = false;  // the resident state now holds the last batch only
-  x->host_call_last = true;
+  leave_host_batch(x);
   if (rc != C2B_OK) {
     cudaStreamSynchronize(cs);
     return rc;
@@ -1693,8 +1735,7 @@ void c2b_obs_free(c2b_ctx *ctx, c2b_obs *obs) {
 
 int c2b_reprojection_error_resident(c2b_ctx *ctx, double norm, double *out) {
   if (!ctx || !out) return set_error(C2B_ERR_INVALID, "c2b_reprojection_error_resident: null argument");
-  CtxExtra *x = ctx->extra.get();
-  if (!x->have_result) return set_error(C2B_ERR_INVALID, "no resident result");
+  C2B_TRY(need_graph(ctx, "c2b_reprojection_error_resident"));
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const uint64_t C = ctx->out_C, O = ctx->out_O, P = ctx->P;
@@ -1795,7 +1836,6 @@ int device_stats(c2b_ctx *ctx, const NoiseView &v, double mean[3], double sd[3],
 
 // host arrays -> the ctx's noise buffers (grow-only, kept between calls)
 int noise_upload(c2b_ctx *ctx, NoiseView &v, const double *cams, uint64_t C, const double *pts, uint64_t P) {
-  cudaStream_t st = ctx->stream;
   C2B_TRY(ctx->nz_cams.ensure(std::max<uint64_t>(C, 1) * 120));
   C2B_TRY(ctx->nz_centers.ensure(std::max<uint64_t>(C, 1) * 24));
   C2B_TRY(ctx->nz_pts.ensure(std::max<uint64_t>(P, 1) * 24));
@@ -1804,42 +1844,31 @@ int noise_upload(c2b_ctx *ctx, NoiseView &v, const double *cams, uint64_t C, con
   v.pts = ctx->nz_pts.as<double>();
   v.C = C;
   v.P = P;
-  if (C) {
-    C2B_TRY(copy_in(ctx, v.cams, cams, C * 120, cudaMemcpyHostToDevice));
-    k_cam_prep<<<blocks_for(C, 128), 128, 0, st>>>(v.cams, C, v.centers, v.centers + C, v.centers + 2 * C);
-    C2B_KERNEL_CHECK();
-  }
+  if (C) C2B_TRY(copy_in(ctx, v.cams, cams, C * 120, cudaMemcpyHostToDevice));
+  C2B_TRY(cam_prep(ctx, v.cams, C, v.centers));
   if (P) C2B_TRY(copy_in(ctx, v.pts, pts, P * 24, cudaMemcpyHostToDevice));
   return C2B_OK;
 }
 
 // the resident problem as a NoiseView (cameras + points of the last uploads, (u, v) of the last resident pass)
 int resident_view(c2b_ctx *ctx, NoiseView &v, const char *who) {
-  CtxExtra *x = ctx->extra.get();
-  if (!x->have_points || !x->have_cameras) return set_error(C2B_ERR_INVALID, "%s: upload cameras and points first", who);
+  C2B_TRY(need_problem(ctx, who));
+  const bool graph = ctx->extra->graph == CtxExtra::Graph::RESIDENT;
   v.cams = ctx->cams.as<double>();
   v.centers = ctx->cam_center.as<double>();
   v.pts = ctx->pts_aos.as<double>();
   v.C = ctx->C;
   v.P = ctx->P;
-  v.uv = x->have_result ? ctx->out_uv[ctx->out_sel].as<double2>() : nullptr;
-  v.O = x->have_result ? ctx->out_O : 0;
+  v.uv = graph ? ctx->out_uv[ctx->out_sel].as<double2>() : nullptr;
+  v.O = graph ? ctx->out_O : 0;
   return C2B_OK;
 }
 
-// after a resident noise pass: camera centres and the SoA points / bounds / grid follow the new values
+// after a resident noise pass: camera centres and the SoA points / bounds / grid follow the new values (the CSR is still
+// the graph of the problem)
 int resident_refresh(c2b_ctx *ctx, bool cams_moved, bool pts_moved) {
-  if (cams_moved && ctx->C) {
-    double *cx = ctx->cam_center.as<double>();
-    k_cam_prep<<<blocks_for(ctx->C, 128), 128, 0, ctx->stream>>>(ctx->cams.as<double>(), ctx->C, cx, cx + ctx->C, cx + 2 * ctx->C);
-    C2B_KERNEL_CHECK();
-  }
-  if (pts_moved) {
-    CtxExtra *x = ctx->extra.get();
-    const bool had = x->have_result;
-    C2B_TRY(c2b_points_commit(ctx, ctx->P));
-    x->have_result = had;  // the CSR is still the graph of this problem
-  }
+  if (cams_moved) C2B_TRY(cam_prep(ctx, ctx->cams.as<double>(), ctx->C, ctx->cam_center.as<double>()));
+  if (pts_moved) C2B_TRY(commit_points(ctx, ctx->P));
   C2B_CUDA(cudaStreamSynchronize(ctx->stream));
   return C2B_OK;
 }
@@ -2300,6 +2329,48 @@ static int cull_limits(uint64_t C, uint64_t P, uint64_t O, const char *who) {
   return C2B_OK;
 }
 
+// A problem in host arrays -> the host-array entries' buffers on ctx->stream (set 0 of c2b_cull_problem, never the
+// resident problem): the camera records to pr_cams[0] and the points to pr_pts[0] when `cams` / `pts` is not null, the
+// CSR (offsets[C + 1], point_idx and uv [offsets[C]]) to pr_off / pr_idx / pr_uv[0].  Then from_visibility's asserts,
+// on the device: offsets start at 0 and do not decrease, indices < P (2^32 for a CSR without points: no u32 index is
+// out of range).  t0 / t1 (may be null) are recorded before the first copy and after the check's flag has been copied
+// back, before the host waits for it.
+static int host_problem_in(c2b_ctx *ctx, const char *who, const double *cams, uint64_t C, const double *pts, uint64_t P,
+                           const uint64_t *offsets, const uint32_t *point_idx, const double *uv, cudaEvent_t t0,
+                           cudaEvent_t t1) {
+  cudaStream_t st = ctx->stream;
+  const uint64_t O = offsets[C];
+  if (cams) C2B_TRY(ctx->pr_cams[0].ensure(std::max<uint64_t>(C, 1) * 120));
+  if (pts) C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
+  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
+  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
+  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
+  C2B_TRY(ctx->pr_small.ensure(64));
+  C2B_TRY(ctx->h_small.ensure(256));
+  if (t0) C2B_CUDA(cudaEventRecord(t0, st));
+  if (cams && C) C2B_TRY(copy_in(ctx, ctx->pr_cams[0].p, cams, C * 120, cudaMemcpyHostToDevice));
+  if (pts && P) C2B_TRY(copy_in(ctx, ctx->pr_pts[0].p, pts, P * 24, cudaMemcpyHostToDevice));
+  C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
+  if (O) {
+    C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
+    C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
+  }
+  uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
+  C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+  const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
+  k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
+      ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, P, flag);
+  C2B_KERNEL_CHECK();
+  C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
+  if (t1) C2B_CUDA(cudaEventRecord(t1, st));
+  C2B_CUDA(cudaStreamSynchronize(st));
+  const uint32_t bad = *ctx->h_small.as<uint32_t>();
+  if (bad & 1u) return set_error(C2B_ERR_INVALID, "%s: offsets[0] != 0 or the CSR offsets decrease", who);
+  if (bad & 2u)
+    return set_error(C2B_ERR_INVALID, "%s: an observation references a point >= %llu", who, (unsigned long long)P);
+  return C2B_OK;
+}
+
 int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64_t P, uint64_t *offsets,
                      uint32_t *point_idx, double *uv, c2b_cull_stats *out) {
   if (!ctx || !offsets || (C && !cams) || (P && !pts)) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: null argument");
@@ -2310,38 +2381,10 @@ int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64
   cudaStream_t st = ctx->stream;
   PruneSet sets[2];
   for (int i = 0; i < 2; ++i) sets[i] = PruneSet{&ctx->pr_cams[i], &ctx->pr_pts[i], &ctx->pr_off[i], &ctx->pr_idx[i], &ctx->pr_uv[i]};
-  C2B_TRY(ctx->pr_cams[0].ensure(std::max<uint64_t>(C, 1) * 120));
-  C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
-  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
-  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
-  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
-  C2B_TRY(ctx->pr_small.ensure(64));
-  C2B_TRY(ctx->h_small.ensure(256));
   Event ev[4];  // timing
   for (auto &e : ev) C2B_TRY(e.create());
   int rc = [&]() -> int {
-    C2B_CUDA(cudaEventRecord(ev[0], st));
-    if (C) C2B_TRY(copy_in(ctx, ctx->pr_cams[0].p, cams, C * 120, cudaMemcpyHostToDevice));
-    if (P) C2B_TRY(copy_in(ctx, ctx->pr_pts[0].p, pts, P * 24, cudaMemcpyHostToDevice));
-    C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
-    if (O) {
-      C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
-      C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
-    }
-    // from_visibility's asserts, on the device: offsets start at 0 and do not decrease, indices < P
-    uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
-    C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
-    const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
-    k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
-        ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, P, flag);
-    C2B_KERNEL_CHECK();
-    C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
-    C2B_CUDA(cudaEventRecord(ev[1], st));
-    C2B_CUDA(cudaStreamSynchronize(st));
-    const uint32_t bad = *ctx->h_small.as<uint32_t>();
-    if (bad & 1u) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: offsets[0] != 0 or the CSR offsets decrease");
-    if (bad & 2u) return set_error(C2B_ERR_INVALID, "c2b_cull_problem: an observation references a point >= %llu",
-                                   (unsigned long long)P);
+    C2B_TRY(host_problem_in(ctx, "c2b_cull_problem", cams, C, pts, P, offsets, point_idx, uv, ev[0], ev[1]));
     int cur = 0;
     uint64_t c = C, p = P, o = O;
     uint32_t it = 0;
@@ -2375,14 +2418,7 @@ int c2b_cull_problem(c2b_ctx *ctx, double *cams, uint64_t C, double *pts, uint64
 
 int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
   if (!ctx) return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: null ctx");
-  CtxExtra *x = ctx->extra.get();
-  if (x->host_call_last)
-    return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: the resident CSR is the last camera batch of the "
-                                      "host-buffer c2b_visibility_graph, not the graph of an uploaded problem; run "
-                                      "c2b_visibility_graph_resident first");
-  if (!x->have_result || !x->have_points || !x->have_cameras)
-    return set_error(C2B_ERR_INVALID, "c2b_cull_problem_resident: no resident result (upload cameras and points, "
-                                      "then c2b_visibility_graph_resident)");
+  C2B_TRY(need_graph(ctx, "c2b_cull_problem_resident"));
   uint64_t C = ctx->out_C, P = ctx->P, O = ctx->out_O;
   C2B_TRY(cull_limits(C, P, O, "c2b_cull_problem_resident"));
   C2B_CUDA(cudaSetDevice(ctx->device));
@@ -2408,22 +2444,11 @@ int c2b_cull_problem_resident(c2b_ctx *ctx, c2b_cull_stats *out) {
     ctx->out_sel = sel ^ 1;
   }
   if (rc != C2B_OK) {
-    // the resident arrays may be half rewritten: nothing of the resident problem is usable any more
     cudaStreamSynchronize(st);
-    x->have_result = x->have_cameras = x->have_points = false;
+    drop_problem(ctx->extra.get());
     return rc;
   }
-  // the culled problem becomes the resident one: camera centres, SoA points, bounds; the point grid is stale
-  ctx->C = C;
-  ctx->out_C = C;
-  ctx->out_O = O;
-  if (C) {
-    double *cx = ctx->cam_center.as<double>();
-    k_cam_prep<<<blocks_for(C, 128), 128, 0, st>>>(ctx->cams.as<double>(), C, cx, cx + C, cx + 2 * C);
-    C2B_KERNEL_CHECK();
-  }
-  C2B_TRY(c2b_points_commit(ctx, P));
-  x->have_result = true;  // the CSR is the graph of the culled problem
+  C2B_TRY(adopt_problem(ctx, ctx->cams.as<double>(), cudaMemcpyDeviceToDevice, C, P, O));
   C2B_CUDA(cudaStreamSynchronize(st));
   if (out) {
     memset(out, 0, sizeof *out);
@@ -2458,33 +2483,10 @@ int c2b_add_incorrect_correspondences(c2b_ctx *ctx, const uint64_t *offsets, uin
   C2B_CUDA(cudaSetDevice(ctx->device));
   CtxExtra *x = ctx->extra.get();
   cudaStream_t st = ctx->stream;
-  // the host-array cull's set 0: never the resident problem
-  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
-  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
-  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
-  C2B_TRY(ctx->pr_small.ensure(64));
-  C2B_TRY(ctx->h_small.ensure(256));
   Event ev[4];  // timing
   for (auto &e : ev) C2B_TRY(e.create());
   int rc = [&]() -> int {
-    C2B_CUDA(cudaEventRecord(ev[0], st));
-    C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
-    if (O) {
-      C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
-      C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
-    }
-    // offsets start at 0 and do not decrease; there is no point count, so no u32 index is out of range
-    uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
-    C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
-    const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
-    k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
-        ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, 1ull << 32, flag);
-    C2B_KERNEL_CHECK();
-    C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
-    C2B_CUDA(cudaEventRecord(ev[1], st));
-    C2B_CUDA(cudaStreamSynchronize(st));
-    if (*ctx->h_small.as<uint32_t>() & 1u)
-      return set_error(C2B_ERR_INVALID, "%s: offsets[0] != 0 or the CSR offsets decrease", who);
+    C2B_TRY(host_problem_in(ctx, who, nullptr, C, nullptr, 1ull << 32, offsets, point_idx, uv, ev[0], ev[1]));
     uint64_t ns = 0, nw = 0;
     unsigned long long err = MM_NO_ERROR;
     C2B_TRY(mismatch_pass(ctx, MismatchBufs{&x->mm_cnt, &x->mm_sel, &x->mm_small}, ctx->pr_off[0].as<uint64_t>(), C,
@@ -2513,14 +2515,8 @@ int c2b_add_incorrect_correspondences_resident(c2b_ctx *ctx, double mismatch_cha
                                                c2b_mismatch_stats *out) {
   static const char *who = "c2b_add_incorrect_correspondences_resident";
   if (!ctx) return set_error(C2B_ERR_INVALID, "%s: null ctx", who);
+  C2B_TRY(need_graph(ctx, who));
   CtxExtra *x = ctx->extra.get();
-  if (x->host_call_last)
-    return set_error(C2B_ERR_INVALID, "%s: the resident CSR is the last camera batch of the host-buffer "
-                                      "c2b_visibility_graph, not the graph of an uploaded problem; run "
-                                      "c2b_visibility_graph_resident first", who);
-  if (!x->have_result || !x->have_points || !x->have_cameras)
-    return set_error(C2B_ERR_INVALID, "%s: no resident result (upload cameras and points, then "
-                                      "c2b_visibility_graph_resident)", who);
   const uint64_t C = ctx->out_C, O = ctx->out_O;
   C2B_TRY(cull_limits(C, 0, O, who));
   C2B_CUDA(cudaSetDevice(ctx->device));
@@ -2541,7 +2537,7 @@ int c2b_add_incorrect_correspondences_resident(c2b_ctx *ctx, double mismatch_cha
   if (rc != C2B_OK) {
     // a failure of the library, not of the input: the point indices may be half permuted
     cudaStreamSynchronize(st);
-    x->have_result = false;
+    drop_graph(x);
     return rc;
   }
   if (err != MM_NO_ERROR) {
@@ -2754,41 +2750,16 @@ int c2b_write_bal(c2b_ctx *ctx, const char *path, int format, const double *cams
   const uint64_t O = offsets[C];
   if (O && (!point_idx || !uv)) return set_error(C2B_ERR_INVALID, "c2b_write_bal: null observation array");
   C2B_CUDA(cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
   CtxExtra *x = ctx->extra.get();
-  // the cull's host-entry buffers (set 0): never the resident problem
-  C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
-  C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
-  C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
-  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
-  C2B_TRY(ctx->pr_small.ensure(64));
-  C2B_TRY(ctx->h_small.ensure(256));
   int rc = [&]() -> int {
-    if (P) C2B_TRY(copy_in(ctx, ctx->pr_pts[0].p, pts, P * 24, cudaMemcpyHostToDevice));
-    C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
-    if (O) {
-      C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
-      C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
-    }
-    // the checks of c2b_cull_problem (from_visibility's asserts), before the file exists
-    uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
-    C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
-    const uint64_t nv = std::max<uint64_t>(std::max(C, O), 1);
-    k_prune_validate<<<(unsigned)std::min<uint64_t>(prune_blocks(nv), (uint64_t)ctx->sm_count * 8), PR_THREADS, 0, st>>>(
-        ctx->pr_off[0].as<uint64_t>(), C, ctx->pr_idx[0].as<uint32_t>(), O, P, flag);
-    C2B_KERNEL_CHECK();
-    C2B_CUDA(cudaMemcpyAsync(ctx->h_small.p, flag, 4, cudaMemcpyDeviceToHost, st));
-    C2B_CUDA(cudaStreamSynchronize(st));
-    const uint32_t bad = *ctx->h_small.as<uint32_t>();
-    if (bad & 1u) return set_error(C2B_ERR_INVALID, "c2b_write_bal: offsets[0] != 0 or the CSR offsets decrease");
-    if (bad & 2u) return set_error(C2B_ERR_INVALID, "c2b_write_bal: an observation references a point >= %llu",
-                                   (unsigned long long)P);
+    // checked before the file exists; the camera records go to the device as 9-vectors
+    C2B_TRY(host_problem_in(ctx, "c2b_write_bal", nullptr, C, pts, P, offsets, point_idx, uv, nullptr, nullptr));
     C2B_TRY(bal_upload_vecs(ctx, x, cams, C));
     const BalView v{x->bal_vecs.as<double>(), ctx->pr_pts[0].as<double>(), ctx->pr_off[0].as<uint64_t>(),
                     ctx->pr_idx[0].as<uint32_t>(), ctx->pr_uv[0].as<double>(), C, P, O};
     return bal_stream(ctx, path, format, v, out);
   }();
-  if (rc != C2B_OK) cudaStreamSynchronize(st);
+  if (rc != C2B_OK) cudaStreamSynchronize(ctx->stream);
   return rc;
 }
 
@@ -2796,14 +2767,8 @@ int c2b_write_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_s
   if (!ctx || !path) return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: null argument");
   if (format != C2B_BAL_TEXT && format != C2B_BAL_BINARY)
     return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: unknown format %d", format);
+  C2B_TRY(need_graph(ctx, "c2b_write_bal_resident"));
   CtxExtra *x = ctx->extra.get();
-  if (x->host_call_last)
-    return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: the resident CSR is the last camera batch of the "
-                                      "host-buffer c2b_visibility_graph, not the graph of an uploaded problem; run "
-                                      "c2b_visibility_graph_resident first");
-  if (!x->have_result || !x->have_points || !x->have_cameras)
-    return set_error(C2B_ERR_INVALID, "c2b_write_bal_resident: no resident result (upload cameras and points, "
-                                      "then c2b_visibility_graph_resident)");
   C2B_CUDA(cudaSetDevice(ctx->device));
   const uint64_t C = ctx->out_C, P = ctx->P, O = ctx->out_O;
   const int sel = ctx->out_sel;
@@ -3217,9 +3182,7 @@ int c2b_read_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_re
   C2B_CUDA(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   // whatever happens below, the previous resident problem is replaced
-  x->have_result = x->have_cameras = x->have_points = false;
-  x->host_call_last = false;
-  x->grid.valid = false;
+  drop_problem(x);
   BalReadState s{ctx, x, path, -1, 0, x->tun.bal_chunk_bytes};
   s.fd = open(path, O_RDONLY | O_CLOEXEC);
   if (s.fd < 0) return set_error(C2B_ERR_IO, "cannot open %s: %s", path, strerror(errno));
@@ -3239,19 +3202,15 @@ int c2b_read_bal_resident(c2b_ctx *ctx, const char *path, int format, c2b_bal_re
     if (C) C2B_CUDA(cudaMemcpyAsync(vecs.data(), s.vecs, C * 72, cudaMemcpyDeviceToHost, st));
     C2B_CUDA(cudaStreamSynchronize(st));
     for (uint64_t c = 0; c < C; ++c) c2b_camera_from_vec(&vecs[9 * c], &cams[15 * c]);
-    C2B_TRY(c2b_upload_cameras(ctx, cams.data(), C));
-    C2B_TRY(c2b_points_commit(ctx, P));
-    ctx->out_C = C;
-    ctx->out_O = O;
+    C2B_TRY(adopt_problem(ctx, cams.data(), cudaMemcpyHostToDevice, C, P, O));
     C2B_CUDA(cudaStreamSynchronize(st));
-    x->have_result = true;
     return C2B_OK;
   }();
   close(s.fd);
   if (rc != C2B_OK) {
     cudaStreamSynchronize(st);
     cudaStreamSynchronize(ctx->copy_stream);
-    x->have_result = x->have_cameras = x->have_points = false;
+    drop_problem(x);
     return rc;
   }
   if (out) {
