@@ -109,6 +109,8 @@ struct Tunables {
   int trilist_warp = -1;           // leaf lists by one warp per camera (1) / one thread (0); -1 = by camera count
   int batches = 0;                 // camera batches of the host-buffer call; 0 = automatic
   double grid_cell_factor = 0.25;  // point-grid cell side / max_dist
+  int grid_x_split = 8;            // point-grid cells in x are 1/k of the side (a power of two; halved while
+                                   // the grid would exceed its cell budget)
   int stage_threads = 4;           // host threads staging a pageable input through the pinned ring; 0 = let the
                                    // driver copy from pageable memory itself
   int cold_staged = 1;             // first host-buffer call on a ctx returns its CSR in unpinned memory filled
@@ -326,6 +328,11 @@ static bool tune(Tunables &t, const char *name, double v) {
   else if (n == "trilist_warp") t.trilist_warp = v < 0 ? -1 : (v != 0);
   else if (n == "batches") t.batches = std::max(0, (int)v);
   else if (n == "grid_cell_factor") t.grid_cell_factor = v > 0 ? v : 0.25;
+  else if (n == "grid_x_split") {
+    int k = 1;
+    while (k < 64 && 2.0 * k <= v) k *= 2;  // the power of two at or below v, in [1, 64]
+    t.grid_x_split = k;
+  }
   else if (n == "stage_threads") t.stage_threads = std::min(std::max(0, (int)v), 16);
   else if (n == "optimistic") t.optimistic = v != 0;
   else if (n == "cold_staged") t.cold_staged = v != 0;
@@ -411,6 +418,7 @@ int c2b_init(int device, c2b_ctx **out) {
         {"C2B_PARTS_LOG2", "parts_log2"}, {"C2B_TRILIST_CAP", "trilist_cap"}, {"C2B_MAX_PAIRS", "max_pairs"},
         {"C2B_HOIST_MAX", "hoist_max"}, {"C2B_PACKET_BVH", "packet_bvh"}, {"C2B_TRILIST_WARP", "trilist_warp"},
         {"C2B_BATCHES", "batches"}, {"C2B_GRID_CELL_FACTOR", "grid_cell_factor"},
+        {"C2B_GRID_X_SPLIT", "grid_x_split"},
         {"C2B_STAGE_THREADS", "stage_threads"}, {"C2B_OPTIMISTIC", "optimistic"}, {"C2B_COLD_STAGED", "cold_staged"},
         {"C2B_BAL_CHUNK_BYTES", "bal_chunk_bytes"}};
     for (auto &h : hooks)
@@ -422,6 +430,7 @@ int c2b_init(int device, c2b_ctx **out) {
 
 int c2b_tune(c2b_ctx *ctx, const char *name, double value) {
   if (!ctx || !name) return set_error(C2B_ERR_INVALID, "c2b_tune: null argument");
+  ctx->extra->grid.valid = false;  // the cached point grid was built with the old grid_* hooks
   if (!strcmp(name, "reset")) {
     ctx->extra->tun = Tunables();
     return C2B_OK;
@@ -838,9 +847,9 @@ static int build_grid(c2b_ctx *ctx, CtxExtra *x, double max_dist) {
   }
   if (!(h > 0.0) || !std::isfinite(h)) h = 1.0;
   const double max_cells = 4194304.0;  // 2^22
-  auto cells_at = [&](double hh) {
+  auto cells_at = [&](double hh, int split) {
     double total = 1.0;
-    for (int k = 0; k < 3; ++k) total *= std::min(std::floor(ext[k] / hh) + 1.0, 1e9);
+    for (int k = 0; k < 3; ++k) total *= std::min(std::floor(ext[k] / (k == 0 ? hh / split : hh)) + 1.0, 1e9);
     return total;
   };
   x->grid.hinted = false;
@@ -865,7 +874,7 @@ static int build_grid(c2b_ctx *ctx, CtxExtra *x, double max_dist) {
         const double a = std::fmax(g.min_c[k], rlo[k]), b = std::fmin(g.max_c[k], rhi[k]);
         if (ext[k] > 0.0) frac *= a <= b ? std::fmin((b - a) / ext[k], 1.0) : 0.0;
       }
-    if (usable && (cells_at(h) > max_cells || odd_bounds || frac < 0.7)) {
+    if (usable && (cells_at(h, 1) > max_cells || odd_bounds || frac < 0.7)) {
       for (int k = 0; k < 3; ++k) {
         // the reach intersected with the data bounds (which may be infinite); empty: one cell at the reach's edge
         const double a = std::fmax(g.min_c[k], rlo[k]), b = std::fmin(g.max_c[k], rhi[k]);
@@ -882,10 +891,16 @@ static int build_grid(c2b_ctx *ctx, CtxExtra *x, double max_dist) {
       x->grid.hinted = true;
     }
   }
+  // Cells of side h in y and z, h / split in x: a camera scans rows of x-contiguous cells and trims each row to
+  // the x interval its ball and view can reach, so finer x cells read fewer points outside that interval while
+  // the number of rows stays the same.  The split halves until the grid fits the budget; a grid that does not
+  // fit unsplit gets coarser cells.
+  int split = x->tun.grid_x_split;
+  while (split > 1 && cells_at(h, split) > max_cells) split /= 2;
   for (;;) {
     double total = 1.0;
     for (int k = 0; k < 3; ++k) {
-      double nk = std::floor(ext[k] / h) + 1.0;
+      double nk = std::floor(ext[k] / (k == 0 ? h / split : h)) + 1.0;
       if (nk > 1e9) nk = 1e9;
       g.n[k] = (int)nk;
       total *= nk;
@@ -894,6 +909,8 @@ static int build_grid(c2b_ctx *ctx, CtxExtra *x, double max_dist) {
     h *= 1.5;
   }
   g.inv_h = 1.0 / h;
+  g.inv_hx = 1.0 / (h / split);
+  g.hx = 1.0 / g.inv_hx;
   uint64_t n_cells = (uint64_t)g.n[0] * g.n[1] * g.n[2];
   C2B_TRY(ctx->cell_of_pt.ensure(P * 4));
   C2B_TRY(ctx->cell_start.ensure((n_cells + 1) * 4));

@@ -9,9 +9,9 @@
 //                go to an unordered pool as (key = camera << pbits | point, u, v); the pool is then
 //                radix-sorted by key, which yields camera-major, ascending-point order
 //                (src/generate.rs:446).
-//   grid       : points binned into a uniform grid (cell = max_dist/4, built here); one warp per
-//                camera scans the x-contiguous cell rows its max_dist ball touches and resolves
-//                occlusion in the same pass (c2b_fused.cuh).
+//   grid       : points binned into a grid (cells max_dist/4 in y and z, a power-of-two fraction of that
+//                in x, built here); one warp per camera scans the x-contiguous cell rows its max_dist
+//                ball touches and resolves occlusion in the same pass (c2b_fused.cuh).
 #pragma once
 #include "c2b_common.cuh"
 #include "c2b_math.cuh"
@@ -176,7 +176,9 @@ __global__ void __launch_bounds__(CB_THREADS) k_cull_exhaustive(CullArgs a) {
 // ---- grid schedule -----------------------------------------------------------------------------------
 struct GridDesc {
   double lo[3];
-  double inv_h;
+  double inv_h;   // 1 / cell side in y and z
+  double inv_hx;  // 1 / cell side in x: inv_h times the x split (a power of two), so rows hold finer cells
+  double hx;      // 1 / inv_hx (the absolute slack of the x trims, c2b_fused.cuh)
   int n[3];
   int drop;         // 1: points outside [rlo, rhi] (the cameras' reach) are not in the grid at all
   double max_c[3];  // bounds of the points IN the grid (for the ball / grid early-out, rows of edge cells)
@@ -185,7 +187,8 @@ struct GridDesc {
 };
 
 __device__ __forceinline__ int grid_coord(const GridDesc &g, int k, double x) {
-  double t = floor(dmul(dsub(x, g.lo[k]), g.inv_h));  // explicit rounding: binning and range queries agree
+  // explicit rounding: binning and range queries agree
+  double t = floor(dmul(dsub(x, g.lo[k]), k == 0 ? g.inv_hx : g.inv_h));
   int c = t < 0.0 ? 0 : (t >= (double)g.n[k] ? g.n[k] - 1 : (int)t);  // NaN -> comparisons false
   if (!(t == t)) c = 0;
   return c;

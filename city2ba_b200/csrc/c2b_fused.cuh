@@ -110,7 +110,7 @@ __device__ __forceinline__ bool camera_cell_range(const GridDesc &g, const doubl
 
 // trims [x0, x1] to the cells that can hold a point with nx*x + ny*y + nz*z + off <= 0 for y in [y0, y1],
 // z in [z0, z1]; xr bounds |nx*x| over the camera's ball; false = nothing on this row qualifies
-__device__ __forceinline__ bool trim_halfspace(const GridDesc &g, double cell_h, double nx, double ny, double nz,
+__device__ __forceinline__ bool trim_halfspace(const GridDesc &g, double nx, double ny, double nz,
                                                double off, double xr, double mag_floor, double y0, double y1,
                                                double z0, double z1, int &x0, int &x1) {
   // smallest value ny*y + nz*z + off can take on the row (0 * inf is avoided explicitly)
@@ -125,7 +125,7 @@ __device__ __forceinline__ bool trim_halfspace(const GridDesc &g, double cell_h,
     } else {
       const double xlim = ddiv(-dsub(bmin, slack), nx);  // nx*x <= -(bmin - slack)
       if (xlim == xlim) {
-        const double xs = dmul(1e-9, dadd(fabs(xlim), cell_h));
+        const double xs = dmul(1e-9, dadd(fabs(xlim), g.hx));
         if (nx > 0.0) {
           const double xe = dadd(xlim, xs);
           if (xe < g.lo[0]) return false;
@@ -151,7 +151,8 @@ struct RowRange {
   uint32_t start, end;  // grid-ordered points [start, end) of the trimmed row; start >= end: nothing
 };
 
-// The trimmed point range of row (y, z) for the camera record c (15 doubles) with centre cc.  Runs in BOTH
+// The trimmed point range of row (y, z) for the camera record c (15 doubles) with centre cc; cell_h is the cell
+// side in y and z (1 / g.inv_h), the x bounds go through grid_coord and g.hx.  Runs in BOTH
 // k_cam_plan (which sizes each camera's scratch slice) and k_visibility_fused (which scans the rows), so it
 // must round identically in both inlined copies: every operation is an explicit round-to-nearest intrinsic
 // that the compiler cannot contract.
@@ -193,7 +194,7 @@ __device__ __forceinline__ RowRange camera_row(const GridDesc &g, const uint32_t
   const double span = dadd(dadd(dadd(fabs(cc[0]), fabs(cc[1])), fabs(cc[2])), dmul(3.0, fabs(max_dist)));
   const double mag_floor = dmul(dadd(planar_image ? fabs(f) : 0.0, 1.0), dmul(rmax, dadd(span, 1.0)));
   // in front of the camera
-  if (!trim_halfspace(g, cell_h, c[2], c[5], c[8], c[11], dmul(fabs(c[2]), reach), mag_floor, y0, y1, z0, z1, x0, x1))
+  if (!trim_halfspace(g, c[2], c[5], c[8], c[11], dmul(fabs(c[2]), reach), mag_floor, y0, y1, z0, z1, x0, x1))
     return r;
   if (planar_image) {
 #pragma unroll
@@ -202,7 +203,7 @@ __device__ __forceinline__ RowRange camera_row(const GridDesc &g, const uint32_t
       const double sf = (k & 1) ? -f : f;
       const double nx = dadd(dmul(sf, c[row]), c[2]), ny = dadd(dmul(sf, c[3 + row]), c[5]);
       const double nz = dadd(dmul(sf, c[6 + row]), c[8]), off = dadd(dmul(sf, c[9 + row]), c[11]);
-      if (!trim_halfspace(g, cell_h, nx, ny, nz, off, dmul(fabs(nx), reach), mag_floor, y0, y1, z0, z1, x0, x1))
+      if (!trim_halfspace(g, nx, ny, nz, off, dmul(fabs(nx), reach), mag_floor, y0, y1, z0, z1, x0, x1))
         return r;
     }
   }

@@ -62,6 +62,8 @@ uint64_t c2b_kernel_launches(void);
  *   trilist_warp (-1 auto|0|1)   leaf lists built by one warp / one thread per camera
  *   batches (0 auto)             camera batches of the host-buffer call
  *   grid_cell_factor (0.25)      point-grid cell side / max_dist
+ *   grid_x_split (8)             point-grid cells in x are 1/k of the side (rounded down to a power of two, at most
+ *                                64; halved while the grid would exceed 2^22 cells)
  *   optimistic (1)               later passes on a ctx launch their kernels without waiting for the plan's totals
  *                                (sizes and kernel variant from the previous pass, checked by the kernels)
  *   cold_staged (1)              first host-buffer call on a ctx: CSR in unpinned memory through a pinned ring
