@@ -31,6 +31,7 @@
 #include "c2b_fused.cuh"
 #include "c2b_graph_cull.cuh"
 #include "c2b_internal.h"
+#include "c2b_join.cuh"
 #include "c2b_math.cuh"
 #include "c2b_mismatch.cuh"
 #include "c2b_noise.cuh"
@@ -303,6 +304,8 @@ struct c2b::CtxExtra {
   DevBuf bal_cam, bal_cnt, bal_slow[2], bal_small;
   // add_incorrect_correspondences (c2b_mismatch.cuh): per-camera counts / bases, selections + picks, flag / counters
   DevBuf mm_cnt, mm_sel, mm_small;
+  // join_landmarks (c2b_join.cuh): the point tree, the selections, the select histogram, flags / counters
+  JoinBufs jn;
   GridCache grid;
   uint64_t points_version = 0;
   double pts_bounds[6] = {0, 0, 0, 0, 0, 0};
@@ -2348,7 +2351,7 @@ static int cull_limits(uint64_t C, uint64_t P, uint64_t O, const char *who) {
 
 // A problem in host arrays -> the host-array entries' buffers on ctx->stream (set 0 of c2b_cull_problem, never the
 // resident problem): the camera records to pr_cams[0] and the points to pr_pts[0] when `cams` / `pts` is not null, the
-// CSR (offsets[C + 1], point_idx and uv [offsets[C]]) to pr_off / pr_idx / pr_uv[0].  Then from_visibility's asserts,
+// CSR (offsets[C + 1], point_idx and, when `uv` is not null, uv [offsets[C]]) to pr_off / pr_idx / pr_uv[0].  Then from_visibility's asserts,
 // on the device: offsets start at 0 and do not decrease, indices < P (2^32 for a CSR without points: no u32 index is
 // out of range).  t0 / t1 (may be null) are recorded before the first copy and after the check's flag has been copied
 // back, before the host waits for it.
@@ -2361,7 +2364,7 @@ static int host_problem_in(c2b_ctx *ctx, const char *who, const double *cams, ui
   if (pts) C2B_TRY(ctx->pr_pts[0].ensure(std::max<uint64_t>(P, 1) * 24));
   C2B_TRY(ctx->pr_off[0].ensure((C + 1) * 8));
   C2B_TRY(ctx->pr_idx[0].ensure(std::max<uint64_t>(O, 1) * 4));
-  C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
+  if (uv) C2B_TRY(ctx->pr_uv[0].ensure(std::max<uint64_t>(O, 1) * 16));
   C2B_TRY(ctx->pr_small.ensure(64));
   C2B_TRY(ctx->h_small.ensure(256));
   if (t0) C2B_CUDA(cudaEventRecord(t0, st));
@@ -2370,7 +2373,7 @@ static int host_problem_in(c2b_ctx *ctx, const char *who, const double *cams, ui
   C2B_TRY(copy_in(ctx, ctx->pr_off[0].p, offsets, (C + 1) * 8, cudaMemcpyHostToDevice));
   if (O) {
     C2B_TRY(copy_in(ctx, ctx->pr_idx[0].p, point_idx, O * 4, cudaMemcpyHostToDevice));
-    C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
+    if (uv) C2B_TRY(copy_in(ctx, ctx->pr_uv[0].p, uv, O * 16, cudaMemcpyHostToDevice));
   }
   uint32_t *flag = ctx->pr_small.as<uint32_t>() + 8;
   C2B_CUDA(cudaMemsetAsync(flag, 0, 4, st));
@@ -2574,6 +2577,90 @@ int c2b_add_incorrect_correspondences_resident(c2b_ctx *ctx, double mismatch_cha
   return C2B_OK;
 }
 
+
+// ---- noise::join_landmarks (c2b_join.cuh) ------------------------------------------------------------------------
+// the message of an input error of the pass (JN_NO_NEIGHBORS ends in the reference's panic text)
+static int join_error(const char *who, int err, uint64_t P, uint64_t bad_point) {
+  if (err == JN_NO_NEIGHBORS)
+    return set_error(C2B_ERR_INVALID, "%s: observations are selected among %llu point(s): No neighbors?!", who,
+                     (unsigned long long)P);
+  return set_error(C2B_ERR_INVALID, "%s: point %llu has a coordinate that is not finite", who,
+                   (unsigned long long)bad_point);
+}
+
+int c2b_join_landmarks(c2b_ctx *ctx, const double *pts, uint64_t P, const uint64_t *offsets, uint64_t C,
+                       uint32_t *point_idx, double join_percent, uint64_t seed, c2b_join_stats *out) {
+  static const char *who = "c2b_join_landmarks";
+  if (!ctx || !offsets || (P && !pts)) return set_error(C2B_ERR_INVALID, "%s: null argument", who);
+  const uint64_t O = offsets[C];
+  if (O && !point_idx) return set_error(C2B_ERR_INVALID, "%s: null observation array", who);
+  C2B_TRY(cull_limits(C, P, O, who));
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  CtxExtra *x = ctx->extra.get();
+  cudaStream_t st = ctx->stream;
+  Event ev[4];  // timing
+  for (auto &e : ev) C2B_TRY(e.create());
+  int rc = [&]() -> int {
+    C2B_TRY(host_problem_in(ctx, who, nullptr, C, pts, P, offsets, point_idx, nullptr, ev[0], ev[1]));
+    uint64_t ns = 0, nc = 0, bad = 0;
+    int err = JN_OK;
+    C2B_TRY(join_pass(ctx, x->jn, ctx->pr_pts[0].as<double>(), P, ctx->pr_idx[0].as<uint32_t>(), O, join_percent,
+                      seed, &ns, &nc, &err, &bad));
+    if (err != JN_OK) return join_error(who, err, P, bad);
+    C2B_CUDA(cudaEventRecord(ev[2], st));
+    if (ns) C2B_CUDA(cudaMemcpyAsync(point_idx, ctx->pr_idx[0].p, O * 4, cudaMemcpyDeviceToHost, st));
+    C2B_CUDA(cudaEventRecord(ev[3], st));
+    C2B_CUDA(cudaStreamSynchronize(st));
+    if (out) {
+      memset(out, 0, sizeof *out);
+      out->n_selected = ns;
+      out->n_changed = nc;
+      cudaEventElapsedTime(&out->ms_h2d, ev[0], ev[1]);
+      cudaEventElapsedTime(&out->ms_compute, ev[1], ev[2]);
+      cudaEventElapsedTime(&out->ms_d2h, ev[2], ev[3]);
+    }
+    return C2B_OK;
+  }();
+  if (rc != C2B_OK) cudaStreamSynchronize(st);
+  return rc;
+}
+
+int c2b_join_landmarks_resident(c2b_ctx *ctx, double join_percent, uint64_t seed, c2b_join_stats *out) {
+  static const char *who = "c2b_join_landmarks_resident";
+  if (!ctx) return set_error(C2B_ERR_INVALID, "%s: null ctx", who);
+  C2B_TRY(need_graph(ctx, who));
+  CtxExtra *x = ctx->extra.get();
+  const uint64_t C = ctx->out_C, P = ctx->P, O = ctx->out_O;
+  C2B_TRY(cull_limits(C, P, O, who));
+  C2B_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  Event ev[2];  // timing
+  for (auto &e : ev) C2B_TRY(e.create());
+  uint64_t ns = 0, nc = 0, bad = 0;
+  int err = JN_OK;
+  int rc = [&]() -> int {
+    C2B_CUDA(cudaEventRecord(ev[0], st));
+    C2B_TRY(join_pass(ctx, x->jn, ctx->pts_aos.as<double>(), P, ctx->out_idx[ctx->out_sel].as<uint32_t>(), O,
+                      join_percent, seed, &ns, &nc, &err, &bad));
+    C2B_CUDA(cudaEventRecord(ev[1], st));
+    return C2B_OK;
+  }();
+  if (rc != C2B_OK) {
+    // a failure of the library, not of the input: the point indices may be half written
+    cudaStreamSynchronize(st);
+    drop_graph(x);
+    return rc;
+  }
+  if (err != JN_OK) return join_error(who, err, P, bad);  // the resident problem is unchanged
+  C2B_CUDA(cudaStreamSynchronize(st));
+  if (out) {
+    memset(out, 0, sizeof *out);
+    out->n_selected = ns;
+    out->n_changed = nc;
+    cudaEventElapsedTime(&out->ms_compute, ev[0], ev[1]);
+  }
+  return C2B_OK;
+}
 
 // ---- BAL files (c2b_bal.cuh) ----------------------------------------------------------------------------------
 namespace {

@@ -67,30 +67,33 @@ __device__ __forceinline__ uint64_t expand21(uint64_t v) {
   return v;
 }
 
+// 63-bit Morton code of a position given per axis as its fraction u of the bounding box (clamped to [0, 1])
+__device__ __forceinline__ uint64_t morton63(const float u[3]) {
+  uint64_t q[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    const uint64_t v = (uint64_t)(fminf(fmaxf(u[k], 0.0f), 1.0f) * 2097151.0f);
+    q[k] = v > 2097151ull ? 2097151ull : v;
+  }
+  return (expand21(q[0]) << 2) | (expand21(q[1]) << 1) | expand21(q[2]);
+}
+
 __global__ void k_bvh_morton(const float *__restrict__ xyz, const uint32_t *__restrict__ tri,
                              uint64_t nt, const uint32_t *__restrict__ bounds,
                              uint64_t *__restrict__ keys, uint32_t *__restrict__ vals) {
   uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= nt) return;
-  float c[3];
+  float u[3];
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
     float a = xyz[3 * (uint64_t)tri[3 * t] + k], b = xyz[3 * (uint64_t)tri[3 * t + 1] + k],
           d = xyz[3 * (uint64_t)tri[3 * t + 2] + k];
-    float lo = fminf(a, fminf(b, d)), hi = fmaxf(a, fmaxf(b, d));
-    c[k] = 0.5f * lo + 0.5f * hi;
-  }
-  uint64_t q[3];
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
+    float c = 0.5f * fminf(a, fminf(b, d)) + 0.5f * fmaxf(a, fmaxf(b, d));
     float lo = ordered_to_float(bounds[k]), hi = ordered_to_float(bounds[3 + k]);
     float ext = hi - lo;
-    float u = ext > 0.0f ? (c[k] - lo) / ext : 0.0f;
-    u = fminf(fmaxf(u, 0.0f), 1.0f);
-    uint64_t v = (uint64_t)(u * 2097151.0f);
-    q[k] = v > 2097151ull ? 2097151ull : v;
+    u[k] = ext > 0.0f ? (c - lo) / ext : 0.0f;
   }
-  keys[t] = (expand21(q[0]) << 2) | (expand21(q[1]) << 1) | expand21(q[2]);
+  keys[t] = morton63(u);
   vals[t] = (uint32_t)t;
 }
 
@@ -146,32 +149,40 @@ __global__ void k_bvh_karras(const uint64_t *__restrict__ keys, int64_t n,
   if (i == 0) parent_internal[0] = 0xffffffffu;
 }
 
-// leaves: gather the triangle into its Morton slot, compute its box, then climb; the second
-// thread to arrive at an internal node merges the two child boxes (boxes are re-read from global
-// memory after a __threadfence, so they are complete).
-__global__ void k_bvh_refit(const float *__restrict__ xyz, const uint32_t *__restrict__ tri,
-                            const uint32_t *__restrict__ sorted_tri, int64_t n,
-                            const uint32_t *__restrict__ left, const uint32_t *__restrict__ right,
-                            const uint32_t *__restrict__ parent_internal,
-                            const uint32_t *__restrict__ parent_leaf, float4 *__restrict__ tris_out,
-                            float *leaf_box /*6n*/, float *int_box /*6(n-1)*/,
-                            uint32_t *__restrict__ visit) {
+// the leaf of the triangle BVH: leaf s is the triangle of Morton slot s, gathered into tris_out
+struct TriLeaf {
+  const float *xyz;
+  const uint32_t *tri, *sorted_tri;
+  float4 *tris_out;
+  __device__ void operator()(int64_t s, float lo[3], float hi[3]) const {
+    uint64_t t = sorted_tri[s];
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+      uint64_t v = tri[3 * t + j];
+      float x = xyz[3 * v], y = xyz[3 * v + 1], z = xyz[3 * v + 2];
+      tris_out[3 * s + j] = make_float4(x, y, z, 0.0f);
+      lo[0] = fminf(lo[0], x);
+      lo[1] = fminf(lo[1], y);
+      lo[2] = fminf(lo[2], z);
+      hi[0] = fmaxf(hi[0], x);
+      hi[1] = fmaxf(hi[1], y);
+      hi[2] = fmaxf(hi[2], z);
+    }
+  }
+};
+
+// leaves: leaf(s, lo, hi) gathers leaf s into its Morton slot and widens its box, then the thread climbs; the second
+// thread to arrive at an internal node merges the two child boxes (boxes are re-read from global memory after a
+// __threadfence, so they are complete).  Leaf is TriLeaf here, the point buckets of c2b_join.cuh there.
+template <class Leaf>
+__global__ void k_bvh_refit(Leaf leaf, int64_t n, const uint32_t *__restrict__ left,
+                            const uint32_t *__restrict__ right, const uint32_t *__restrict__ parent_internal,
+                            const uint32_t *__restrict__ parent_leaf, float *leaf_box /*6n*/,
+                            float *int_box /*6(n-1)*/, uint32_t *__restrict__ visit) {
   int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= n) return;
-  uint64_t t = sorted_tri[s];
   float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
-#pragma unroll
-  for (int j = 0; j < 3; ++j) {
-    uint64_t v = tri[3 * t + j];
-    float x = xyz[3 * v], y = xyz[3 * v + 1], z = xyz[3 * v + 2];
-    tris_out[3 * s + j] = make_float4(x, y, z, 0.0f);
-    lo[0] = fminf(lo[0], x);
-    lo[1] = fminf(lo[1], y);
-    lo[2] = fminf(lo[2], z);
-    hi[0] = fmaxf(hi[0], x);
-    hi[1] = fmaxf(hi[1], y);
-    hi[2] = fmaxf(hi[2], z);
-  }
+  leaf(s, lo, hi);
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
     leaf_box[6 * s + k] = lo[k];
@@ -298,10 +309,9 @@ inline int bvh_build(c2b_ctx *ctx, c2b_scene *sc, const float *h_xyz, uint64_t n
         s.par_l.as<uint32_t>());
     C2B_KERNEL_CHECK();
   }
-  k_bvh_refit<<<nb, 256, 0, st>>>(s.xyz.as<float>(), s.tri.as<uint32_t>(), vals[res], (int64_t)nt,
-                                  s.left.as<uint32_t>(), s.right.as<uint32_t>(),
-                                  s.par_i.as<uint32_t>(), s.par_l.as<uint32_t>(),
-                                  sc->tris.as<float4>(), s.leaf_box.as<float>(),
+  k_bvh_refit<<<nb, 256, 0, st>>>(TriLeaf{s.xyz.as<float>(), s.tri.as<uint32_t>(), vals[res], sc->tris.as<float4>()},
+                                  (int64_t)nt, s.left.as<uint32_t>(), s.right.as<uint32_t>(),
+                                  s.par_i.as<uint32_t>(), s.par_l.as<uint32_t>(), s.leaf_box.as<float>(),
                                   s.int_box.as<float>(), s.visit.as<uint32_t>());
   C2B_KERNEL_CHECK();
   k_bvh_layout<<<(int)((sc->n_nodes + 255) / 256), 256, 0, st>>>(

@@ -23,8 +23,10 @@
 
 namespace c2b {
 
-// ST_MISMATCH: add_incorrect_correspondences (c2b_mismatch.cuh), one block per observation
-enum { ST_DRIFT_CAM = 1, ST_DRIFT_PT = 2, ST_NOISE_CAM = 3, ST_NOISE_PT = 4, ST_NOISE_OBS = 5, ST_MISMATCH = 6 };
+// ST_MISMATCH: add_incorrect_correspondences (c2b_mismatch.cuh), ST_JOIN: join_landmarks (c2b_join.cuh); one block
+// per observation
+enum { ST_DRIFT_CAM = 1, ST_DRIFT_PT = 2, ST_NOISE_CAM = 3, ST_NOISE_PT = 4, ST_NOISE_OBS = 5, ST_MISMATCH = 6,
+       ST_JOIN = 7 };
 
 __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                               uint32_t k0, uint32_t k1, uint32_t *out) {

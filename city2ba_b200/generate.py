@@ -354,6 +354,23 @@ class ResidentProblem:
             raise
         return st.to_dict()
 
+    def join_landmarks(self, join_percent, seed=0) -> dict:
+        """noise::join_landmarks on the resident points and CSR, in HBM (c2b_join_landmarks_resident): the draws of
+        noise.join_landmarks_gpu.  Afterwards download / reprojection_error / cull / write see the edited graph.
+        Raises AssertionError ("No neighbors?!") with fewer than two points and C2BError on a point that is not
+        finite, and leaves the problem unchanged then.  Returns the stats: n_selected, n_changed, ms_compute."""
+        from .noise import _no_neighbors
+        st = _lib.JoinStats()
+        try:
+            check(lib().c2b_join_landmarks_resident(self.ctx.handle, float(join_percent), int(seed) & (2 ** 64 - 1),
+                                                    C.byref(st)))
+        except _lib.C2BError as e:
+            a = _no_neighbors(e)
+            if a is not None:
+                raise a from e
+            raise
+        return st.to_dict()
+
     def write(self, path) -> dict:
         """BAProblem::write of the resident problem (c2b_write_bal_resident): .bal text or .bbal binary by the
         extension, encoded on the GPU and streamed to disk.  Returns the stats: bytes, chunks, ms_encode, ms_d2h

@@ -151,6 +151,47 @@ def add_incorrect_correspondences_gpu(bal: BAProblem, mismatch_chance, seed=None
     return _with_graph(bal, off, idx, uv)
 
 
+def _no_neighbors(e):
+    """C2BError of a join with fewer than two points -> the host form's AssertionError (same message tail)"""
+    from ._lib import ERR_INVALID, C2BError
+    if isinstance(e, C2BError) and e.code == ERR_INVALID and str(e).endswith("No neighbors?!"):
+        return AssertionError(str(e))
+    return None
+
+
+def join_landmarks_gpu(bal: BAProblem, join_percent, seed=None, ctx=None, stats=None) -> BAProblem:
+    """join_landmarks on the GPU (c2b_join_landmarks): the same operation with the library's deterministic draws, a
+    pure function of `seed` (default: a fresh one from os.urandom), so it does not reproduce the numpy draws of the
+    host form.  The 10 neighbours are exact: the 11 nearest points by (squared distance, index), the first skipped.
+    Raises AssertionError ("No neighbors?!") when observations are selected among fewer than two points, and
+    C2BError when a point is not finite.  Works on copies; `stats`, a dict if given, receives the call's
+    c2b_join_stats (n_selected, n_changed, device times)."""
+    from ._lib import C2BError, JoinStats
+    ctx = ctx or context()
+    g = bal.vis_graph
+    off = np.array(g.offsets, np.uint64, order="C")
+    if len(off) != len(bal.cameras) + 1:
+        raise ValueError("cameras and CSR offsets disagree")
+    idx = g.point_idx
+    if len(idx) and int(idx.max()) > 0xffffffff:
+        raise ValueError("point index does not fit 32 bits")
+    idx = np.array(idx, np.uint32, order="C")
+    pts = np.array(bal.points, np.float64, order="C").reshape(-1, 3)
+    st = JoinStats()
+    try:
+        check(lib().c2b_join_landmarks(ctx.handle, _p(pts), len(pts), off.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                       len(off) - 1, idx.ctypes.data_as(C.POINTER(C.c_uint32)), float(join_percent),
+                                       _seed(seed), C.byref(st)))
+    except C2BError as e:
+        a = _no_neighbors(e)
+        if a is not None:
+            raise a from e
+        raise
+    if stats is not None:
+        stats.update(st.to_dict())
+    return _with_graph(bal, off, idx, g.uv)
+
+
 def drop_features(bal: BAProblem, drop_percent, seed=None) -> BAProblem:
     """src/noise.rs:229-250: every camera keeps floor(len * drop_percent) of its observations, chosen by a shuffle"""
     rng = np.random.default_rng(seed)

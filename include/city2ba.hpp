@@ -1504,6 +1504,40 @@ inline BAProblem join_landmarks(const BAProblem &bal, double join_percent, uint6
   }
   return out;
 }
+// the same on the GPU (c2b_join_landmarks), with the library's deterministic draws: a pure function of seed, not the
+// draws of the host form above; the neighbours are exact, ties by index.  Throws the host form's std::logic_error
+// ("No neighbors?!") when observations are selected among fewer than two points.  stats (optional) receives the
+// call's counts and device times.
+inline BAProblem join_landmarks(const Context &ctx, const BAProblem &bal, double join_percent, uint64_t seed,
+                                c2b_join_stats *stats = nullptr) {
+  const size_t nc = bal.num_cameras(), np = bal.num_points();
+  std::vector<uint64_t> offsets(nc + 1, 0);
+  for (size_t i = 0; i < nc; ++i) offsets[i + 1] = offsets[i] + bal.vis_graph[i].size();
+  std::vector<uint32_t> idx(offsets[nc]);
+  for (size_t i = 0, k = 0; i < nc; ++i)
+    for (const auto &e : bal.vis_graph[i]) {
+      detail::require(e.first <= 0xffffffffull, "point index does not fit 32 bits");
+      idx[k++] = (uint32_t)e.first;
+    }
+  std::vector<double> pts(3 * np);
+  for (size_t i = 0; i < np; ++i)
+    for (int k = 0; k < 3; ++k) pts[3 * i + k] = bal.points[i][k];
+  c2b_join_stats st;
+  const int rc = c2b_join_landmarks(ctx.handle(), pts.data(), np, offsets.data(), nc, idx.data(), join_percent, seed,
+                                    &st);
+  if (rc == C2B_ERR_INVALID) {
+    const std::string m = c2b_last_error(), tail = "No neighbors?!";
+    if (m.size() >= tail.size() && m.compare(m.size() - tail.size(), std::string::npos, tail) == 0)
+      throw std::logic_error(tail);
+  }
+  detail::check(rc);
+  if (stats) *stats = st;
+  BAProblem out = bal;
+  size_t k = 0;
+  for (auto &o : out.vis_graph)
+    for (auto &e : o) e.first = idx[k++];
+  return out;
+}
 }  // namespace noise
 
 }  // namespace city2ba

@@ -350,6 +350,32 @@ int c2b_add_incorrect_correspondences(c2b_ctx *ctx, const uint64_t *offsets, uin
 int c2b_add_incorrect_correspondences_resident(c2b_ctx *ctx, double mismatch_chance, uint64_t seed,
                                                c2b_mismatch_stats *out);
 
+/* ---- noise::join_landmarks (src/noise.rs:323-378) ---------------------------------------------------------------
+ * n = floor(join_percent * P) (0 when join_percent is negative or NaN) observations, min(n, O) of them, drawn over all
+ * O observations, are each re-pointed at one of the 10 nearest other landmarks of the landmark they see.  Points,
+ * offsets and (u, v) are not changed.  Deterministic in seed (DESIGN.md §4, "Joined landmarks"): one Philox4x32-10
+ * block per observation o (key seed, counter (o lo, o hi, 7, 0)); the selected observations are the min(n, O) smallest
+ * pairs (w0 | w1 << 32, o); the neighbour list is the m = min(11, P) smallest pairs (d2, k) over all points, d2 the
+ * squared distance to the landmark seen, rounded to nearest in the order (dx dx + dy dy) + dz dz; the observation
+ * takes list[1 + mulhi64(w2 | w3 << 32, m - 1)], the search is exact.  With at least one selection, P < 2 fails with a
+ * message ending in "No neighbors?!" and a point with a coordinate that is not finite fails naming the lowest such
+ * point: C2B_ERR_INVALID, nothing is changed then. */
+typedef struct {
+  uint64_t n_selected;               /* observations selected: min(n, O) */
+  uint64_t n_changed;                /* selections whose new point differs from the one they saw */
+  float ms_h2d, ms_compute, ms_d2h;  /* device time (CUDA events on the ctx stream); h2d/d2h 0 when resident;
+                                        ms_h2d includes the input check */
+} c2b_join_stats;
+/* in place on host arrays: pts holds P points (x, y, z), point_idx O = offsets[C] entries.  Rejects offsets[0] != 0,
+ * decreasing offsets and indices >= P with C2B_ERR_INVALID and leaves point_idx untouched.  C + P and O below
+ * 2^32 - 1.  Does not touch the ctx's resident problem.  out may be NULL. */
+int c2b_join_landmarks(c2b_ctx *ctx, const double *pts, uint64_t P, const uint64_t *offsets, uint64_t C,
+                       uint32_t *point_idx, double join_percent, uint64_t seed, c2b_join_stats *out);
+/* the same on the resident points and CSR, in HBM; afterwards c2b_download_obs, c2b_reprojection_error_resident,
+ * c2b_cull_problem_resident and c2b_write_bal_resident see the edited graph.  Refuses in the cases
+ * c2b_cull_problem_resident refuses. */
+int c2b_join_landmarks_resident(c2b_ctx *ctx, double join_percent, uint64_t seed, c2b_join_stats *out);
+
 /* ---- BAL files (BAProblem::write, src/baproblem.rs:709-764) ----------------------------------------------------
  * The file is encoded on the device and streamed to disk in chunks of at most bal_chunk_bytes: the D2H copy and
  * the host write of one chunk overlap the encoding of the next, and the device and pinned memory of the encoder

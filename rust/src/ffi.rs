@@ -55,6 +55,13 @@ pub struct c2b_mismatch_stats {
     pub ms_h2d: c_float, pub ms_compute: c_float, pub ms_d2h: c_float,
 }
 
+// noise::join_landmarks on the GPU (c2b_join_landmarks[_resident])
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct c2b_join_stats {
+    pub n_selected: u64, pub n_changed: u64,
+    pub ms_h2d: c_float, pub ms_compute: c_float, pub ms_d2h: c_float,
+}
+
 // BAL files on the GPU (c2b_write_bal / c2b_write_bal_resident)
 pub const C2B_BAL_TEXT: c_int = 0;
 pub const C2B_BAL_BINARY: c_int = 1;
@@ -167,6 +174,11 @@ extern "C" {
                                              out: *mut c2b_mismatch_stats) -> c_int;
     pub fn c2b_add_incorrect_correspondences_resident(ctx: *mut c2b_ctx, mismatch_chance: c_double, seed: u64,
                                                       out: *mut c2b_mismatch_stats) -> c_int;
+    pub fn c2b_join_landmarks(ctx: *mut c2b_ctx, pts: *const c_double, p: u64, offsets: *const u64, c: u64,
+                              point_idx: *mut u32, join_percent: c_double, seed: u64,
+                              out: *mut c2b_join_stats) -> c_int;
+    pub fn c2b_join_landmarks_resident(ctx: *mut c2b_ctx, join_percent: c_double, seed: u64,
+                                       out: *mut c2b_join_stats) -> c_int;
     // ---- BAL files: a Rust BAProblem::write would call c2b_write_bal with the format of its extension ----
     pub fn c2b_write_bal(ctx: *mut c2b_ctx, path: *const c_char, format: c_int, cams: *const c_double, c: u64,
                          pts: *const c_double, p: u64, offsets: *const u64, point_idx: *const u32,
